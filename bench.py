@@ -2,7 +2,7 @@
 """bench.py — benchmarks of the decode / training hot path on B200 (DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--prec f16|bf16|f32]
-                    [--workload decode_4096|decode_4096_strong|train_2048_mips|lut_65|video_1080p120]
+                    [--workload decode_4096|decode_4096_strong|train_2048_mips|lut_65|video_1080p120] [--dump-outputs DIR]
 
 Prints ONE JSON line.  The default workload is BASELINE.json configs[1]: full-frame decode of a 4096x4096 RGB texture on
 the tensor-core path, one frame per GPU per step ("weak": frames are independent).  `value` = decoded Gtexel/s over all
@@ -11,6 +11,10 @@ of the compressed grids + decoder, decode, D2H of the 8-bit frame inside the tim
 PCIe floor of the same copies.  `--impl reference` times the CPU port of the reference's algorithm (oracle/) on the host
 cores, one whole frame per step.  The other workloads are BASELINE configs 3 / 4 / 5 at their named shapes and the
 strong-scaling form of config 2 (one frame tiled over N GPUs); each prints its own line.
+
+`--steps K` is the number of timed steps of every workload and of each of its timed legs.  `--dump-outputs DIR` is
+accepted for decode_4096 only: after the timed steps it writes a fixed, seeded sample of the last step's frame to
+DIR/frame.npy.  With --gpus N > 1 that is rank 0's frame; every rank decodes its own seeded model.
 """
 import argparse
 import json
@@ -365,7 +369,7 @@ def bench_train(args, env, nic, ic, var2):
     for _ in range(4):
         coord = torch.randint(0, size - crop + 1, (nc, 2), generator=g)
         batches.append((coord.to(dev), ic.sample_crops(imgt, coord, crop)))
-    steps = max(args.steps, 20)
+    steps = args.steps
     for i in range(max(args.warmup, 3)):
         tr.step(*batches[i % 4], 0)
         tr.step_sampled(pyr)
@@ -441,7 +445,7 @@ def bench_gather(args, env, nic, ic, var2, fp):
         run()
     torch.cuda.synchronize()
     L.set_option(dev, L.OPT_TIME_KERNELS, 1)
-    for _ in range(5):
+    for _ in range(args.steps):
         run()
     torch.cuda.synchronize()
     kms, kn = L.kernel_time_ms(dev)
@@ -475,7 +479,7 @@ def bench_3d(args, env, nic, ic, var2):
             fn()
         torch.cuda.synchronize()
         L.set_option(dev, L.OPT_TIME_KERNELS, 1)
-        for _ in range(5):
+        for _ in range(args.steps):
             fn()
         torch.cuda.synchronize()
         kms, kn = L.kernel_time_ms(dev)
@@ -503,7 +507,7 @@ def run_decode_4096(args, env):
     texels = SIZE * SIZE
     tf_peak, hbm_peak, src = peaks()
 
-    def measure(prec):
+    def measure(prec, keep_frame=False):
         session = ic.DecodeSession(fp, dec, precision=prec)      # tables (re-packed weights) built once per model
         for _ in range(args.warmup):
             flush.zero_()
@@ -512,6 +516,7 @@ def run_decode_4096(args, env):
         l0 = nic.launch_count(dev)
         L.set_option(dev, L.OPT_TIME_KERNELS, 1)
         ms = timed_steps(env, lambda: session.decode(0, out_dtype=torch.uint8, out=out), args.steps, flush)
+        frame = out.cpu().numpy() if keep_frame else None        # the last timed step's frame, before other legs reuse `out`
         kms, kn = L.kernel_time_ms(dev)
         L.set_option(dev, L.OPT_TIME_KERNELS, 0)
         launches = nic.launch_count(dev) - l0
@@ -519,10 +524,10 @@ def run_decode_4096(args, env):
         ms_b = timed_steps(env, lambda: ic.decode(fp, dec, 0, precision=prec, out_dtype=torch.uint8, out=out), args.steps, flush)
         return {"ms_per_step": ms / args.steps, "kernel_ms": kms / max(kn, 1), "launches": launches,
                 "value": world * texels / (ms / args.steps * 1e-3) / 1e9,
-                "value_with_table_build": world * texels / (ms_b / args.steps * 1e-3) / 1e9}
+                "value_with_table_build": world * texels / (ms_b / args.steps * 1e-3) / 1e9, "frame": frame}
 
     sampler = ClockSampler(env.local) if rank == 0 else None
-    main = measure(args.prec)
+    main = measure(args.prec, keep_frame=bool(args.dump_outputs) and rank == 0)
     clocks = sampler.stop() if sampler else None
     other = "bf16" if args.prec == "f16" else "f16"
     alt = measure(other) if args.prec != "f32" else None
@@ -544,7 +549,7 @@ def run_decode_4096(args, env):
         e2e_step()
     pipe.finish()
     env.barrier()
-    k2 = max(3, args.steps)                  # the same K steps as `value`; pipeline fill and drain are inside the timed region
+    k2 = args.steps                          # the same K steps as `value`; pipeline fill and drain are inside the timed region
     # Three timed regions of K steps each, the MEDIAN reported and all three listed: the copies share the host's PCIe root
     # and memory with whatever else runs on the box, and a 20 ms region is short enough to be hit by one transient.
     e2e_runs = []
@@ -620,7 +625,21 @@ def run_decode_4096(args, env):
             line["psnr"] = psnr_vs_reference(out_host, keep)
             if "train" in line:
                 line["train"]["cpu_value"] = cpu_train_rate(threads)
+        if args.dump_outputs:
+            dump_frame_sample(args.dump_outputs, main["frame"])
         env.emit(line)
+
+
+DUMP_TEXELS = 1 << 22            # 4.2 M of the 16.8 M texels: 48 MB as float32
+
+
+def dump_frame_sample(out_dir, frame):
+    """Writes DIR/frame.npy: the uint8 RGB values of a fixed, seeded sample of the last timed step's 4096^2 frame, as
+    float32 [DUMP_TEXELS, 3], texels in raster order (row-major flat index).  The inputs are seeded too, so two builds run
+    with the same arguments can be compared value for value."""
+    idx = np.sort(np.random.default_rng(0).choice(SIZE * SIZE, DUMP_TEXELS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frame.npy"), frame.reshape(-1, 3)[idx].astype(np.float32))
 
 
 def psnr_vs_reference(ours_u8, ref_tiles):
@@ -712,7 +731,7 @@ def run_train_2048(args, env):
     dec = ic.ColorDecoder(73, 64, cout).to(dev)
     prec = args.train_prec or "bf16"                                   # config 3 names bf16
     tr = ic.FusedTrainer(fp, dec, num_epochs=1000000, fp_bits=8, seed=3, precision=prec, exchange=args.exchange)
-    steps = max(args.steps, 100)
+    steps = args.steps
     for _ in range(max(args.warmup, 20)):                              # touches most levels (peer buffers are mapped on first use)
         tr.step_sampled(pyr)
     env.barrier()
@@ -786,7 +805,7 @@ def run_lut_65(args, env):
 
     for _ in range(min(args.warmup, 2)):
         step()
-    steps = min(args.steps, 5)
+    steps = args.steps
     L.set_option(dev, L.OPT_TIME_KERNELS, 1)
     ms = timed_steps(env, step, steps) / steps
     kms, kn = L.kernel_time_ms(dev)
@@ -857,7 +876,7 @@ def run_video(args, env):
 
     for _ in range(args.warmup):
         step()
-    steps = min(args.steps, 10)
+    steps = args.steps
     L.set_option(dev, L.OPT_TIME_KERNELS, 1)
     ms = timed_steps(env, step, steps, flush) / steps
     kms, kn = L.kernel_time_ms(dev)
@@ -905,7 +924,13 @@ def main():
                     help="training workloads at N > 1: the data-parallel exchange (FusedTrainer)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the gather, 3-D and training side benchmarks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="decode_4096: after the timed steps, write a seeded sample of the last step's frame to DIR/frame.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "decode_4096"):
+        ap.error("--dump-outputs covers the decode_4096 workload of --impl ours")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

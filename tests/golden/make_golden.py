@@ -1,6 +1,6 @@
 """Generate `tests/golden/*.npz|json` by executing the UNMODIFIED reference on seeded inputs.
 
-Run in the build container only (needs `/root/reference`):  python tests/golden/make_golden.py
+Needs the reference project's `Projects/` directory:  NIC_REFERENCE_DIR=<it> python tests/golden/make_golden.py
 The fixtures hold reference OUTPUTS; inputs are regenerated from seeds by `tests/golden/inputs.py`
 (small inputs are stored as well, to make the fixtures self-describing).
 Large outputs are stored as (flat index, value) subsamples + float64 column sums + a sha256 of the bytes.

@@ -1,7 +1,8 @@
-"""Load the UNMODIFIED reference (`/root/reference/Projects/image_compression.py`) in-process.
+"""Load the UNMODIFIED reference (`$NIC_REFERENCE_DIR/image_compression.py`) in-process.
 
-Only used by `tests/golden/make_golden.py` in the build container; `/root/reference` does not exist on
-the GPU box, so nothing under `tests/` imports this at test time.  Recipe = SURVEY.md §8(c):
+NIC_REFERENCE_DIR names the `Projects/` directory of a checkout of the reference project, which is not part of this
+repository.  Used by `tests/golden/make_golden.py` to regenerate the fixtures; at test time only the tests that compare
+with the reference's source import it, and they skip when NIC_REFERENCE_DIR is unset.  Recipe = SURVEY.md §8(c):
 `runpy.run_path` with `NUM_EPOCHS=0`, no-op stubs for the two missing plotting/logging packages, and a
 scratch cwd that holds the directories the script writes into.
 """
@@ -11,7 +12,7 @@ import sys
 import tempfile
 import types
 
-REF = "/root/reference/Projects"
+REF = os.environ.get("NIC_REFERENCE_DIR", "")
 
 
 def _stub_modules():
@@ -45,6 +46,8 @@ def load_reference(*overrides, npy=None):
     """
     import numpy as np
 
+    if not REF or not os.path.exists(os.path.join(REF, "image_compression.py")):
+        raise FileNotFoundError("set NIC_REFERENCE_DIR to the reference project's Projects/ directory")
     os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
     sys.dont_write_bytecode = True
     _stub_modules()

@@ -176,8 +176,8 @@ def test_step_sampled_trains_and_is_reproducible():
 # ------------------------------------------------------------------------------------------------ host file helpers (f4)
 def test_host_file_helpers_formats(tmp_path):
     """save_result_to_csv / make_filename_by_seq / readClip / timelaps (utils.py:37-113): file formats as the reference
-    writes them — checked against the reference's own functions when /root/reference is present (this container), and
-    against the format spelled out here otherwise.  No device involved."""
+    writes them — checked against the format spelled out here, and against the reference's own functions as well when
+    NIC_REFERENCE_DIR names the reference's Projects/ directory.  No device involved."""
     import importlib.util
     import sys
     from neural_image_compression_v2_b200 import utils as U
@@ -195,8 +195,9 @@ def test_host_file_helpers_formats(tmp_path):
     (d / "run_0_000.csv").write_text("x")
     (d / "run_0_007.csv").write_text("x")
     assert U.make_filename_by_seq(str(d), "run_0.csv") == f"{d}/run_0_008.csv"
-    ref_utils = "/root/reference/Projects/utils.py"
-    if os.path.exists(ref_utils):
+    from ref_loader import REF
+    ref_utils = os.path.join(REF, "utils.py")
+    if REF and os.path.exists(ref_utils):
         sys.dont_write_bytecode = True
         spec = importlib.util.spec_from_file_location("ref_utils_host", ref_utils)
         R = importlib.util.module_from_spec(spec)

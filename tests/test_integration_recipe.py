@@ -1,5 +1,7 @@
-"""INTEGRATION.md section 1 against the REAL reference script (build container only: /root/reference does not exist on the
-GPU box, where tests/test_gpu_round2.py::test_integration_import_swap_recipe_runs_the_script_flow covers the run-time side).
+"""INTEGRATION.md section 1.  The documented block, exec'd on its own, binds every hot-path name to this package (runs
+everywhere).  The tests marked `needs_reference` check it against the REAL reference script, which is not part of this
+repository: they run when NIC_REFERENCE_DIR names the reference's Projects/ directory and skip otherwise
+(tests/test_gpu_round2.py::test_integration_import_swap_recipe_runs_the_script_flow covers the run-time side without it).
 
 The reference's image_compression.py is executed up to line 346 (imports, configuration, its function definitions — nothing
 that touches a device), the documented block is appended, and the resulting namespace is checked: every global name the
@@ -13,21 +15,44 @@ import sys
 
 import pytest
 
-REF = "/root/reference/Projects"
+from ref_loader import REF  # tests/golden: $NIC_REFERENCE_DIR
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = "neural_image_compression_v2_b200"
 
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "image_compression.py")),
-                                reason="the reference tree is only present in the build container")
+needs_reference = pytest.mark.skipif(not REF or not os.path.exists(os.path.join(REF, "image_compression.py")),
+                                     reason="needs the reference project's Projects/ directory in NIC_REFERENCE_DIR")
+
+HOT = ["ColorDecoder", "create_decoder_input_2d", "create_decoder_input_3d", "create_decoder_input_3d_v2",
+       "finally_decode_input_2d", "finally_decode_input_3d", "finally_decode_input_3d_v2", "create_pyramid", "create_pyramid_3d",
+       "create_pyramid_mip_levels", "fp_quantize_clamp", "fp_all_quantize", "fp_savable", "fp_load", "fp_freeze", "quantize4fp",
+       "save4fp", "load4fp", "quantize_to_bit", "calculate_psnr", "triangular_positional_encoding", "positional_encoding",
+       "bits2dtype_torch", "bits2dtype_np"]
+HOST_HELPERS = ("print_", "make_filename_by_seq", "safe_statistics", "quantize_from_bit_to_bit")
+
+
+def _recipe_block():
+    doc = open(os.path.join(ROOT, "INTEGRATION.md")).read()
+    sec1 = doc[doc.index("## 1."):doc.index("## 2.")]
+    return re.findall(r"```python\n(.*?)```", sec1, flags=re.S)[1]
+
+
+def test_recipe_block_binds_the_hot_path_names_and_nothing_else():
+    """The inserted block alone (the script's own globals absent, so var2 keeps its defaults): every hot-path name it binds
+    is this package's, and it binds none of the host-side helpers the script keeps from the reference's utils."""
+    ns = {"__name__": "recipe_block"}
+    exec(compile(_recipe_block(), "INTEGRATION.md(section 1 block)", "exec"), ns)
+    for name in HOT:
+        assert name in ns and ns[name].__module__.startswith(PKG), (name, getattr(ns.get(name), "__module__", None))
+    for name in HOST_HELPERS:
+        assert name not in ns, name
 
 
 def _namespace():
     import tempfile
     from ref_loader import _stub_modules                   # tensorboardX / matplotlib no-op stubs (tests/golden)
     _stub_modules()
-    doc = open(os.path.join(ROOT, "INTEGRATION.md")).read()
-    sec1 = doc[doc.index("## 1."):doc.index("## 2.")]
-    block = re.findall(r"```python\n(.*?)```", sec1, flags=re.S)[1]
+    block = _recipe_block()
     src = open(os.path.join(REF, "image_compression.py"), encoding="utf-8").read().split("\n")
     assert src[349].startswith("decoder = ColorDecoder()"), "the recipe's insertion point (line 350) moved"
     text = "\n".join(src[:346]) + "\n" + block
@@ -54,17 +79,13 @@ def _namespace():
     return ns, ref_mods, src
 
 
+@needs_reference
 def test_recipe_shadows_the_hot_path_and_every_script_global_resolves():
     ns, ref_mods, src = _namespace()
-    hot = ["ColorDecoder", "create_decoder_input_2d", "create_decoder_input_3d", "create_decoder_input_3d_v2",
-           "finally_decode_input_2d", "finally_decode_input_3d", "finally_decode_input_3d_v2", "create_pyramid", "create_pyramid_3d",
-           "create_pyramid_mip_levels", "fp_quantize_clamp", "fp_all_quantize", "fp_savable", "fp_load", "fp_freeze", "quantize4fp",
-           "save4fp", "load4fp", "quantize_to_bit", "calculate_psnr", "triangular_positional_encoding", "positional_encoding",
-           "bits2dtype_torch", "bits2dtype_np"]
-    for name in hot:
+    for name in HOT:
         assert ns[name].__module__.startswith(PKG), (name, ns[name].__module__)
     # host-side helpers stay the reference's own
-    for name in ("print_", "make_filename_by_seq", "safe_statistics", "quantize_from_bit_to_bit"):
+    for name in HOST_HELPERS:
         assert not ns[name].__module__.startswith(PKG)
     # globals used by the script's functions: defined by line 346 + the block, or assigned at module level further down
     tree = ast.parse("\n".join(src))
@@ -83,6 +104,7 @@ def test_recipe_shadows_the_hot_path_and_every_script_global_resolves():
         assert not missing, (fn.name, missing)
 
 
+@needs_reference
 def test_shadowed_functions_accept_the_reference_signatures():
     """Same parameter names in the same order as the reference's functions (ours may append optional ones)."""
     ns, ref_mods, src = _namespace()
