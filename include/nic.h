@@ -219,6 +219,38 @@ int nic_decode(NicHandle* h, const NicGeom* g, const float* g0, const float* g1,
 int nic_decode_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, const uint8_t* codes1, int bits,
                      const int64_t* origins, const NicMlp* m, void* out, int out_dtype, int precision, void* stream);
 
+/* ---- filtered sampling at continuous coordinates ------------------------------------------------------- */
+/* Bilinear (2-D) / trilinear (3-D) sampling of the decoded mip: what a renderer's texture read or a colour-LUT
+ * application does, without materialising the taps.  coords: [Q, D] fp32 normalised coordinates in axis order (x, y[, z]),
+ * x the first image axis (the slow axis of nic_decode's output).  The geometry describes the mip exactly as for a
+ * random-access nic_decode, with num_blocks = Q and block = 1; `origins` / origin0 are not used.  On each axis, with S the
+ * extent of the mip (every step one fp32 operation, so the result is reproducible bit for bit):
+ *   p  = align_corners ? u * (S - 1) : u * S - 0.5;      p = min(max(p, -2^24), 2^24)   (NaN -> -2^24)
+ *   i0 = floor(p), f = p - i0;  taps i0 and i0 + 1 with weights 1 - f and f;
+ *   NIC_ADDRESS_CLAMP: each tap clamped to [0, S - 1];  NIC_ADDRESS_WRAP: each tap reduced modulo S (fmod, + S if negative).
+ * The T = 2^D taps are ordered with x slowest; a tap's weight is the product of its per-axis weights (x first) and its value
+ * is nic_decode's output for that integer texel (fp32 sigmoid output, before any quantisation).  out [Q, cout] in out_dtype
+ * (NIC_DT_F32, or NIC_DT_U8 = floor(v*255+.5) of the blended value, quantised once) holds sum_k w_k * value_k, or with
+ * blend_prev set (1 - blend_weight) * prev + blend_weight * that sum (blending two mips: fractional LOD).
+ * precision NIC_PREC_F32: the taps are decoded by the reference-exact kernel and summed in tap order; F16 / BF16: one
+ * tensor-core pass, the T taps of a query are T adjacent rows of a tile and are summed in registers.  Q * T must stay below
+ * 2^31 - 128 (NIC_ERR_UNSUPPORTED).  An extent whose last texel would index outside the grids
+ * gives NIC_ERR_BOUNDS (the rule of a host-known origin, with origin 0 and block = extent). */
+enum { NIC_ADDRESS_CLAMP = 0, NIC_ADDRESS_WRAP = 1 };
+typedef struct NicSampler {
+  int32_t address;          /* NIC_ADDRESS_*                                                     */
+  int32_t align_corners;    /* 0: texel i centred at (i + .5)/S; 1: texel i at i/(S - 1)         */
+  int32_t extent[3];        /* texels of this mip along x, y, z (z ignored in 2-D)               */
+  float blend_weight;       /* used when blend_prev != NULL                                      */
+  const float* blend_prev;  /* optional [Q, cout] fp32: out = (1 - w) * prev + w * sample        */
+} NicSampler;
+int nic_sample(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const float* coords,
+               const NicSampler* s, const NicMlp* m, void* out, int out_dtype, int precision, void* stream);
+/* The same from the saved model's uint8 codes (as nic_decode_codes).  Tensor-core precisions only. */
+int nic_sample_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, const uint8_t* codes1, int bits,
+                     const float* coords, const NicSampler* s, const NicMlp* m, void* out, int out_dtype,
+                     int precision, void* stream);
+
 /* ---- fused training forward+backward (K3+K4) ----------------------------------------------------------- */
 /* One step of train_models up to loss.backward() (image_compression.py:239-265).
  *   targets [N, cout] fp32; noise: NULL (no noise), or [N, Cin] fp32 injected tensor (parity tests), or use

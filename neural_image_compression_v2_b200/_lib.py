@@ -37,6 +37,14 @@ class NicMlp(C.Structure):
                 ("w3", C.c_void_p), ("b3", C.c_void_p)]
 
 
+ADDRESS_CLAMP, ADDRESS_WRAP = 0, 1
+
+
+class NicSampler(C.Structure):
+    _fields_ = [("address", C.c_int32), ("align_corners", C.c_int32), ("extent", C.c_int32 * 3),
+                ("blend_weight", C.c_float), ("blend_prev", C.c_void_p)]
+
+
 class NicMlpGrad(C.Structure):
     _fields_ = [("w1", C.c_void_p), ("b1", C.c_void_p), ("w2", C.c_void_p), ("b2", C.c_void_p),
                 ("w3", C.c_void_p), ("b3", C.c_void_p)]
@@ -79,6 +87,9 @@ SYMBOLS = {
     "nic_mlp_backward": (_I, [_P, C.POINTER(NicMlp), _P, _L, _L, _P, _P, _P, _P, C.POINTER(NicMlpGrad), _P, _P]),
     "nic_decode": (_I, [_P, C.POINTER(NicGeom), _P, _P, _P, C.POINTER(NicMlp), _P, _I, _I, _P]),
     "nic_decode_codes": (_I, [_P, C.POINTER(NicGeom), _P, _P, _I, _P, C.POINTER(NicMlp), _P, _I, _I, _P]),
+    "nic_sample": (_I, [_P, C.POINTER(NicGeom), _P, _P, _P, C.POINTER(NicSampler), C.POINTER(NicMlp), _P, _I, _I, _P]),
+    "nic_sample_codes": (_I, [_P, C.POINTER(NicGeom), _P, _P, _I, _P, C.POINTER(NicSampler), C.POINTER(NicMlp), _P, _I,
+                              _I, _P]),
     "nic_train_step": (_I, [_P, C.POINTER(NicGeom), _P, _P, _P, C.POINTER(NicMlp), _P, _P, _I, C.c_uint64, C.c_uint64,
                             _L, C.POINTER(NicMlpGrad), _P, _P, _P, _P, _I, _P]),
     "nic_adam_step": (_I, [_P, C.POINTER(NicAdamTensor), _I, _F, _F, _F, _F, _I, _P]),

@@ -94,6 +94,7 @@ int nic_destroy(NicHandle* h) {
   if (h->xch_host_err) cudaFreeHost(h->xch_host_err);
   if (h->dbg_counters) cudaFree(h->dbg_counters);
   if (h->data_scratch) cudaFree(h->data_scratch);
+  if (h->sample_scratch) cudaFree(h->sample_scratch);
   if (h->adam_desc) cudaFree(h->adam_desc);
   for (int i = 0; i < 2 * NIC_MAX_TIMED; ++i)
     if (h->timed_ev[i]) cudaEventDestroy(h->timed_ev[i]);
@@ -411,6 +412,83 @@ int nic_decode_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, cons
                         (const long long*)origins, out, out_dtype, precision, st);
   h->src_code_bits = 0;
   return cuda_fail(h, rc, "nic_decode_codes");
+}
+
+// Geometry of a sampling call: the mip is validated like a host-known block (origin 0, block = extent), then described as
+// num_blocks one-texel queries.
+static int flatten_sampler(NicHandle* h, const NicGeom* g, const NicSampler* s, const float* coords, DevGeom* d,
+                           DevSampler* ds, const char* who) {
+  if (!g || !s) return fail(h, NIC_ERR_ARG, "%s: geometry or sampler is NULL", who);
+  if (s->address != NIC_ADDRESS_CLAMP && s->address != NIC_ADDRESS_WRAP) return fail(h, NIC_ERR_ARG, "%s: address mode %d", who, s->address);
+  if (g->num_blocks < 0) return fail(h, NIC_ERR_ARG, "%s: num_blocks %d", who, g->num_blocks);
+  if (g->num_blocks > 0 && !coords) return fail(h, NIC_ERR_ARG, "%s: coords is NULL", who);
+  const int dim = g->method == NIC_METHOD_2D ? 2 : 3;
+  NicGeom whole = *g;
+  whole.num_blocks = 1;
+  for (int a = 0; a < 3; ++a) {
+    if (a < dim && s->extent[a] < 1) return fail(h, NIC_ERR_ARG, "%s: extent %d on axis %d", who, s->extent[a], a);
+    if (a < dim && g->block[a] != 1) return fail(h, NIC_ERR_ARG, "%s: block must be 1 (one query per block)", who);
+    whole.block[a] = a < dim ? s->extent[a] : 1;
+    whole.origin0[a] = 0;
+  }
+  int rc = flatten_geom(h, &whole, false, d);
+  if (rc) return rc;
+  if (((long long)g->num_blocks << dim) >= (1ll << 31) - 128)
+    return fail(h, NIC_ERR_UNSUPPORTED, "%s: %d queries x %d taps reach 2^31 - 128 rows; split the batch", who, g->num_blocks, 1 << dim);
+  d->nblocks = g->num_blocks;
+  for (int a = 0; a < 3; ++a) d->B[a] = 1;
+  d->per_block = 1;
+  d->N = g->num_blocks;
+  memset(ds, 0, sizeof(*ds));
+  ds->coords = coords;
+  for (int a = 0; a < 3; ++a) ds->S[a] = a < dim ? s->extent[a] : 1;
+  ds->address = s->address;
+  ds->align_corners = s->align_corners != 0;
+  ds->blend_weight = s->blend_weight;
+  ds->prev = s->blend_prev;
+  return NIC_OK;
+}
+
+int nic_sample(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const float* coords,
+               const NicSampler* s, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+  NIC_ENTER(h);
+  DevGeom d;
+  DevSampler ds;
+  int rc = flatten_sampler(h, g, s, coords, &d, &ds, "nic_sample");
+  if (rc) return rc;
+  MlpDev md;
+  rc = flatten_mlp(h, m, &md, d.cin);
+  if (rc) return rc;
+  if (!g0 || !g1 || (!out && d.N > 0)) return fail(h, NIC_ERR_ARG, "nic_sample: NULL pointer");
+  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_sample: out_dtype %d", out_dtype);
+  if (precision == NIC_PREC_F32)
+    return cuda_fail(h, launch_sample_f32(h, d, ds, md, g0, g1, out, out_dtype, st), "nic_sample(f32)");
+  if (precision == NIC_PREC_F16 || precision == NIC_PREC_BF16)
+    return cuda_fail(h, launch_sample_tc(h, d, ds, md, g0, g1, out, out_dtype, precision, st), "nic_sample(tensor core)");
+  return fail(h, NIC_ERR_ARG, "nic_sample: precision %d", precision);
+}
+
+int nic_sample_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, const uint8_t* codes1, int bits,
+                     const float* coords, const NicSampler* s, const NicMlp* m, void* out, int out_dtype,
+                     int precision, void* stream) {
+  NIC_ENTER(h);
+  DevGeom d;
+  DevSampler ds;
+  int rc = flatten_sampler(h, g, s, coords, &d, &ds, "nic_sample_codes");
+  if (rc) return rc;
+  MlpDev md;
+  rc = flatten_mlp(h, m, &md, d.cin);
+  if (rc) return rc;
+  if (bits < 1 || bits > 8) return fail(h, NIC_ERR_ARG, "nic_sample_codes: bits %d (1..8)", bits);
+  if (!codes0 || !codes1 || (!out && d.N > 0)) return fail(h, NIC_ERR_ARG, "nic_sample_codes: NULL pointer");
+  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_sample_codes: out_dtype %d", out_dtype);
+  if (precision != NIC_PREC_F16 && precision != NIC_PREC_BF16)
+    return fail(h, NIC_ERR_UNSUPPORTED, "nic_sample_codes: tensor-core precisions only (f16 / bf16); unpack the codes for NIC_PREC_F32");
+  h->src_code_bits = bits;
+  rc = launch_sample_tc(h, d, ds, md, reinterpret_cast<const float*>(codes0), reinterpret_cast<const float*>(codes1), out,
+                        out_dtype, precision, st);
+  h->src_code_bits = 0;
+  return cuda_fail(h, rc, "nic_sample_codes");
 }
 
 int nic_train_step(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const int64_t* origins,

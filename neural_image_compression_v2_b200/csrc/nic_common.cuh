@@ -136,6 +136,50 @@ __device__ __forceinline__ Texel texel_of_fast(const DevGeom& g, unsigned n, con
 
 __device__ __forceinline__ int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
+// ------------------------------------------------------------------------------------------------ filtered sampling
+// What nic_sample / nic_sample_codes filter: the texel extent of the mip and how coordinates map onto it (nic.h NicSampler).
+struct DevSampler {
+  const float* coords;    // [Q, dim] normalised (x, y[, z])
+  int S[3];               // texels per axis (1 on unused axes)
+  int address;            // NIC_ADDRESS_*
+  int align_corners;
+  float blend_weight;     // out = (1 - t) * prev + t * sample when prev != NULL
+  const float* prev;      // [Q, cout] fp32 or NULL
+};
+
+// Tap `tap` (0 .. 2^dim - 1, x slowest) of the linear filter at normalised coordinates u[0..dim): writes the integer texel
+// of the mip to p[0..3) and returns the tap's weight.  Every step is one explicit fp32 operation (nic.h documents the rule),
+// so the oracle reproduces it bit for bit; after the clamp to +-2^24 the index arithmetic is exact (NaN -> -2^24).
+__device__ __forceinline__ float sample_tap(const DevSampler& s, int dim, const float* u, int tap, int* p) {
+  float w = 1.0f;
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    p[a] = 0;
+    if (a >= dim) continue;
+    const int S = s.S[a];
+    float x = s.align_corners ? __fmul_rn(u[a], (float)(S - 1)) : __fsub_rn(__fmul_rn(u[a], (float)S), 0.5f);
+    x = fminf(fmaxf(x, -16777216.0f), 16777216.0f);
+    const float i0 = floorf(x), f = __fsub_rn(x, i0);
+    const int hi = (tap >> (dim - 1 - a)) & 1;
+    int i = (int)i0 + hi;
+    if (s.address == NIC_ADDRESS_WRAP) {
+      i %= S;                 // = fmodf(i, S): exact, sign of the dividend
+      if (i < 0) i += S;
+    } else {
+      i = clampi(i, 0, S - 1);
+    }
+    p[a] = i;
+    w = __fmul_rn(w, hi ? f : __fsub_rn(1.0f, f));
+  }
+  return w;
+}
+
+// The last step of a sample: the optional blend with the previous mip's result, element `idx` of [Q, cout].
+__device__ __forceinline__ float sample_blend_prev(const DevSampler& s, long long idx, float v) {
+  if (!s.prev) return v;
+  return __fadd_rn(__fmul_rn(__fsub_rn(1.0f, s.blend_weight), __ldg(s.prev + idx)), __fmul_rn(s.blend_weight, v));
+}
+
 // Linear node index in a channel-major grid [C, (z,) y, x]; indices clamped for memory safety (the reference
 // raises IndexError instead; host-known origins are validated in nic_api.cu).
 __device__ __forceinline__ long long node_index(const int* nodes, int dim, int x, int y, int z) {

@@ -46,6 +46,8 @@ struct Handle {
   int step_metrics;          // NIC_OPT_STEP_METRICS: training steps also accumulate the 8-bit squared error in loss_sum[1]
   void* data_scratch;        // nic_data.cu: resample coefficient tables + 8-bit intermediate
   size_t data_scratch_bytes;
+  void* sample_scratch;      // nic_sample.cu: tap texels, tap weights and tap outputs of the fp32 sampling arm
+  size_t sample_scratch_bytes;
   int gelu_poly;             // NIC_OPT_GELU_POLY: -1 = tuned default, 0..8 = activation pairs (of 8) on the polynomial GELU
   struct PreparedKey {       // what the tables in tc_weights / tc_shadow were last built from
     const void *g0, *g1, *w1, *b1, *w2, *b2, *w3, *b3;
@@ -238,6 +240,11 @@ int launch_train_f32(Handle* h, const DevGeom& g, const MlpDev& m, const MlpGrad
                      float* dg1, float* loss_sum, float* out_save, cudaStream_t st);
 int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1,
                      const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st);
+// nic_sample / nic_sample_codes: g describes the mip with nblocks = queries (one texel each); smp the filter.
+int launch_sample_tc(Handle* h, const DevGeom& g, const DevSampler& smp, const MlpDev& m, const float* g0, const float* g1,
+                     void* out, int out_dtype, int precision, cudaStream_t st);
+int launch_sample_f32(Handle* h, const DevGeom& g, const DevSampler& smp, const MlpDev& m, const float* g0, const float* g1,
+                      void* out, int out_dtype, cudaStream_t st);
 int launch_train_tc(Handle* h, const DevGeom& g, const MlpDev& m, const MlpGradDev& gm, const float* g0, const float* g1,
                     const long long* origins, const float* targets, const float* noise, int noise_bits,
                     unsigned long long seed, unsigned long long step, float grad_scale, float* dg0, float* dg1,

@@ -578,16 +578,19 @@ __global__ void __launch_bounds__(WS_THREADS, 1) decode_tc2d_ws_kernel(DevGeom g
 //   layers : SS-form tcgen05.mma issued by the group's elected lane after a 128-thread named barrier (layer 1: KX/16
 //            MMAs; layers 2, 3: 4 MMAs + 1 bias MMA against a shared constant ones block), the epilogue overwrites the
 //            operand buffer with the next layer's activations;  the groups never meet at a CTA-wide barrier.
+// TAPS > 0 (nic_sample: 4 in 2-D, 8 in 3-D): row n is tap n % TAPS of query n / TAPS, its texel comes from the query's
+// coordinates (sample_tap); the TAPS rows of a query are adjacent lanes of one warp, which blend their weighted sigmoid
+// outputs with a shuffle butterfly before tap 0 stores the query.  TAPS = 0 is the plain decode.
 constexpr int GW_GROUP = 128;
 
 // NGT / LUTCAP: groups per CTA and capacity of the positional-encoding LUT.  The defaults (8 groups, or 5 for method 3's
 // 32 KB operand buffers, 256 LUT entries) always fit; with a 64-entry LUT (step >= 1/4: every full-resolution decode) a
 // SIXTH 32 KB group fits the 227 KB of shared memory for method 3 (225.8 KB), 20 % more tiles in flight.
 constexpr int gws_groups(int kx, int ngt) { return ngt ? ngt : (kx > 80 ? 5 : 8); }
-template <int METHOD, int FMT, typename OutT, int NPOLY, int NGT = 0, int LUTCAP = TC_LUT_MAX>
+template <int METHOD, int FMT, typename OutT, int NPOLY, int NGT = 0, int LUTCAP = TC_LUT_MAX, int TAPS = 0>
 __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GROUP, 1)
     decode_tc_gws_kernel(DevGeom g, ShadowGeom sg, const long long* __restrict__ origins, const uint4* __restrict__ wimg,
-                         int cout, int lut_n, OutT* __restrict__ out) {
+                         int cout, int lut_n, OutT* __restrict__ out, DevSampler smp) {
   using S = RowShape<METHOD>;
   using P = Pair<FMT>;
   constexpr int KX = S::KX, NG = gws_groups(KX, NGT), THREADS = NG * GW_GROUP;
@@ -665,9 +668,20 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
   for (unsigned tile = blockIdx.x + gridDim.x * slot; tile < ntiles; tile += gridDim.x * NG) {
     const unsigned n = tile * TC_ROWS + row;
     const bool live = n < (unsigned)g.N;
+    float tap_w = 0.f;                               // TAPS > 0: this row's filter weight (0 on dead rows)
     // ------------------------------------------------------------------------------------ gather -> operand buffer
     {
-      Texel t = texel_of_fast(g, live ? n : (unsigned)g.N - 1, origins);
+      Texel t;
+      if constexpr (TAPS > 0) {
+        const unsigned q = (live ? n : (unsigned)g.N - 1) / TAPS;
+        float u[3] = {0.f, 0.f, 0.f};
+#pragma unroll
+        for (int a = 0; a < S::DIM; ++a) u[a] = __ldg(smp.coords + (size_t)q * S::DIM + a);
+        const float w = sample_tap(smp, S::DIM, u, row % TAPS, t.p);
+        tap_w = live ? w : 0.f;
+      } else {
+        t = texel_of_fast(g, live ? n : (unsigned)g.N - 1, origins);
+      }
       AxisCoord ax[3];
 #pragma unroll
       for (int a = 0; a < 3; ++a) {
@@ -801,7 +815,28 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
     else tmem_ld4(tD, acc);
     tc_wait_ld();
     tc_fence_before();
-    if (live) {
+    if constexpr (TAPS > 0) {
+      // weighted taps, reduced over the TAPS lanes of the query in a fixed butterfly order (every lane takes part: the
+      // shuffles run before the live test); tap 0 applies the optional mip blend and stores, quantising once
+      float v[16];
+#pragma unroll
+      for (int c = 0; c < 16; ++c) v[c] = (c < cout) ? __fmul_rn(tap_w, sigmoid_tanh(__uint_as_float(acc[c]))) : 0.f;
+#pragma unroll
+      for (int msk = 1; msk < TAPS; msk <<= 1) {
+#pragma unroll
+        for (int c = 0; c < 4; ++c) v[c] = __fadd_rn(v[c], __shfl_xor_sync(0xffffffffu, v[c], msk));
+        if (cout > 4) {
+#pragma unroll
+          for (int c = 4; c < 16; ++c) v[c] = __fadd_rn(v[c], __shfl_xor_sync(0xffffffffu, v[c], msk));
+        }
+      }
+      if (live && row % TAPS == 0) {
+        const size_t o = (size_t)(n / TAPS) * cout;
+#pragma unroll
+        for (int c = 0; c < 16; ++c)
+          if (c < cout) store_out(out + o + c, sample_blend_prev(smp, (long long)(o + c), v[c]));
+      }
+    } else if (live) {
 #pragma unroll
       for (int c = 0; c < 4; ++c)
         if (c < cout) store_sigmoid(out + (size_t)n * cout + c, __uint_as_float(acc[c]));
@@ -1215,14 +1250,16 @@ static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const flo
   return (int)cudaGetLastError();
 }
 
-template <int METHOD, int FMT, typename OutT>
+// TAPS > 0: filtered sampling (smp set, g.N = queries * TAPS rows) always runs on the general kernel: the fast 2-D kernel
+// and the code-resident kernel have no per-row texel and no tap epilogue.
+template <int METHOD, int FMT, typename OutT, int TAPS = 0>
 static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1,
-                       const long long* origins, OutT* out, cudaStream_t st) {
+                       const long long* origins, OutT* out, cudaStream_t st, const DevSampler* smp = nullptr) {
   using S = RowShape<METHOD>;
-  if constexpr (METHOD == NIC_METHOD_2D) {
+  if constexpr (METHOD == NIC_METHOD_2D && TAPS == 0) {
     if (fast2d_eligible(g, origins) && !h->disable_fast2d) return launch_fast2d<FMT, OutT>(h, g, m, g0, g1, out, st);
   }
-  if constexpr (METHOD == NIC_METHOD_3D && FMT == 0) {       // small models given as codes, random-access queries
+  if constexpr (METHOD == NIC_METHOD_3D && FMT == 0 && TAPS == 0) {       // small models given as codes, random-access queries
     if (h->src_code_bits > 0) {
       const int crc = launch_codes_smem<METHOD, OutT>(h, g, m, reinterpret_cast<const uint8_t*>(g0),
                                                       reinterpret_cast<const uint8_t*>(g1), origins, out, st);
@@ -1271,35 +1308,40 @@ static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const float
   static_assert(GSMEM0 <= 227 * 1024 && (S::KX <= 80 || GSMEM6 <= 227 * 1024), "shared memory budget");
   // (not for random-access queries: they live on L1 hits, and the sixth group's 32 KB come out of the L1 — measured
   //  4.8 -> 4.2 Gquery/s on a 256^3 volume)
-  const bool six = S::KX > 80 && lut_n <= 64 && g.per_block > 1 && !(h->debug_flags & 128);
+  const bool six = TAPS == 0 && S::KX > 80 && lut_n <= 64 && g.per_block > 1 && !(h->debug_flags & 128);
   const int NG = six ? 6 : NG0, GSMEM = six ? GSMEM6 : GSMEM0;
-  void (*kern)(DevGeom, ShadowGeom, const long long*, const uint4*, int, int, OutT*) = nullptr;
-  if constexpr (S::KX > 80) {
+  void (*kern)(DevGeom, ShadowGeom, const long long*, const uint4*, int, int, OutT*, DevSampler) = nullptr;
+  if constexpr (S::KX > 80 && TAPS == 0) {
     if (six) kern = npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 6, 64> : decode_tc_gws_kernel<METHOD, FMT, OutT, 3, 6, 64>;
   }
-  if (!kern) kern = npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0> : decode_tc_gws_kernel<METHOD, FMT, OutT, 3>;
+  if (!kern)
+    kern = npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 0, TC_LUT_MAX, TAPS>
+                      : decode_tc_gws_kernel<METHOD, FMT, OutT, 3, 0, TC_LUT_MAX, TAPS>;
   if (npoly != 0 && npoly != 3) return NIC_ERR_UNSUPPORTED;      // (the NIC_GELU_SWEEP values exist for the fast 2-D kernel only)
   e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, GSMEM);
   if (e != cudaSuccess) return (int)e;
   long long groups = (ntiles + NG - 1) / NG;
   int grid = (int)(groups < h->sms ? groups : h->sms);
+  const DevSampler no_sampler = {};
   {
     KernelTimer timer(h, st);
-    kern<<<grid, NG * GW_GROUP, GSMEM, st>>>(g, sg, origins, (const uint4*)h->tc_weights, m.cout, lut_n, out);
+    kern<<<grid, NG * GW_GROUP, GSMEM, st>>>(g, sg, origins, (const uint4*)h->tc_weights, m.cout, lut_n, out,
+                                             smp ? *smp : no_sampler);
   }
   h->launches++;
   return (int)cudaGetLastError();
 }
 
-template <int METHOD>
+template <int METHOD, int TAPS = 0>
 static int launch_tc_m(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1,
-                       const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st) {
+                       const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st,
+                       const DevSampler* smp = nullptr) {
   if (precision == NIC_PREC_F16) {
-    if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 0, uint8_t>(h, g, m, g0, g1, origins, (uint8_t*)out, st);
-    return launch_tc_t<METHOD, 0, float>(h, g, m, g0, g1, origins, (float*)out, st);
+    if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 0, uint8_t, TAPS>(h, g, m, g0, g1, origins, (uint8_t*)out, st, smp);
+    return launch_tc_t<METHOD, 0, float, TAPS>(h, g, m, g0, g1, origins, (float*)out, st, smp);
   }
-  if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 1, uint8_t>(h, g, m, g0, g1, origins, (uint8_t*)out, st);
-  return launch_tc_t<METHOD, 1, float>(h, g, m, g0, g1, origins, (float*)out, st);
+  if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 1, uint8_t, TAPS>(h, g, m, g0, g1, origins, (uint8_t*)out, st, smp);
+  return launch_tc_t<METHOD, 1, float, TAPS>(h, g, m, g0, g1, origins, (float*)out, st, smp);
 }
 
 int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1,
@@ -1310,6 +1352,21 @@ int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const float* 
     case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D>(h, g, m, g0, g1, origins, out, out_dtype, precision, st);
     case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D>(h, g, m, g0, g1, origins, out, out_dtype, precision, st);
     case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2>(h, g, m, g0, g1, origins, out, out_dtype, precision, st);
+  }
+  return NIC_ERR_UNSUPPORTED;
+}
+
+int launch_sample_tc(Handle* h, const DevGeom& gq, const DevSampler& smp, const MlpDev& m, const float* g0, const float* g1,
+                     void* out, int out_dtype, int precision, cudaStream_t st) {
+  if (gq.nblocks == 0) return NIC_OK;
+  if (gq.C != 12 || gq.PE != 6 || m.hidden != 64 || m.cout > 16) return NIC_ERR_UNSUPPORTED;
+  DevGeom g = gq;                                   // one row per tap: queries x 2^dim rows
+  g.N = (long long)gq.nblocks << gq.dim;
+  if (g.N >= (1ll << 31) - TC_ROWS) return NIC_ERR_UNSUPPORTED;     // 32-bit row index in the kernel
+  switch (g.method) {
+    case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D, 4>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
+    case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D, 8>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
+    case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2, 8>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
   }
   return NIC_ERR_UNSUPPORTED;
 }

@@ -330,6 +330,112 @@ def decode_points_codes(codes, decoder, coords, num_bits, mip_level=0, precision
     return out
 
 
+# ------------------------------------------------------------------------------------------------ filtered sampling
+_ADDRESS = {"clamp": L.ADDRESS_CLAMP, "wrap": L.ADDRESS_WRAP}
+
+
+def _sample_coords(coords, dim):
+    if not torch.is_tensor(coords) or coords.dtype != torch.float32 or not coords.is_contiguous():
+        raise TypeError("coords must be a contiguous float32 tensor [Q, D] of normalised coordinates")
+    if coords.dim() != 2 or coords.shape[1] != dim:
+        raise ValueError(f"coords must be [Q, {dim}], got {tuple(coords.shape)}")
+    if not coords.is_cuda:
+        raise L.NicError(-3, "coords must be a CUDA tensor (no CPU fallback)")
+    if coords.shape[0] << dim >= 2 ** 31 - 128:
+        raise ValueError(f"at most (2^31 - 129) / {1 << dim} queries per call; split the batch")
+    return coords
+
+
+def _sample_passes(lod, size, table):
+    """[(mip, weight)] of a sample at `lod`: one pass, or two for a fractional lod between two mips of the table."""
+    if size is not None and float(lod) != math.floor(float(lod)):
+        raise ValueError("size may only be given with an integer lod")
+    lod = min(max(float(lod), 0.0), float(var2.MAX_MIP_LEVEL))
+    m = int(math.floor(lod))
+    t = lod - m
+    if t == 0.0 or m >= max(table):
+        return [(m, 1.0)]
+    return [(m, 1.0), (m + 1, t)]
+
+
+def _sample(launch, fp_like, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table):
+    """Common body of sample / sample_codes; launch(geom, grid0, grid1, sampler, mlp, out, out_dtype) calls the library."""
+    method = _method() if method is None else method
+    dim = 2 if method == L.METHOD_2D else 3
+    table = feature_pyramid_mip_levels() if level_table is None else level_table
+    if address not in _ADDRESS:
+        raise ValueError(f"address must be 'clamp' or 'wrap', got {address!r}")
+    if out_dtype not in (torch.float32, torch.uint8):
+        raise TypeError("out_dtype must be torch.float32 or torch.uint8")
+    passes = _sample_passes(lod, size, table)
+    coords = _sample_coords(coords, dim)
+    params = [p.detach().contiguous() for p in decoder.parameters_list()]
+    m = L.make_mlp(params)
+    q = coords.shape[0]
+    out = torch.empty((q, m.cout), dtype=out_dtype, device=coords.device)
+    prev = None
+    for i, (mip, t) in enumerate(passes):
+        fl = table[mip]
+        g0, g1 = fp_like[fl * 2], fp_like[fl * 2 + 1]
+        s = (var2.IMAGE_SIZE // pow(2, mip)) if size is None else size
+        extent = (s,) * dim if isinstance(s, int) else tuple(s)
+        geom = L.make_geom(method, g0, g1, 1, q, _step_log2(mip, fl), mip, var2.PE_CHANNELS, _pe_kind(method))
+        smp = L.NicSampler()
+        smp.address, smp.align_corners = _ADDRESS[address], int(bool(align_corners))
+        for a in range(3):
+            smp.extent[a] = int(extent[a]) if a < dim else 1
+        smp.blend_weight, smp.blend_prev = t, (prev.data_ptr() if prev is not None else None)
+        last = i == len(passes) - 1
+        dst = out if last else torch.empty((q, m.cout), dtype=torch.float32, device=coords.device)
+        launch(geom, g0, g1, smp, m, dst, out_dtype if last else torch.float32, coords)
+        prev = dst
+    return out
+
+
+def sample(fp, decoder, coords, lod=0, size=None, address="clamp", align_corners=False, precision=None,
+           out_dtype=torch.float32, method=None, level_table=None):
+    """Filtered sampling at continuous coordinates: bilinear (2-D) / trilinear (3-D) reads of the decoded mip, as a renderer
+    samples a texture or a colour LUT is applied, without materialising the taps (nic.h nic_sample has the exact rule).
+
+    coords: float32 `[Q, D]` CUDA tensor of normalised coordinates in axis order (x, y[, z]).  lod: mip level; a fractional
+    lod blends the two mips around it ((1 - t) * mip m + t * mip m + 1), clamped to [0, MAX_MIP_LEVEL].  size: texel extent
+    of the mip (int or per-axis tuple), default IMAGE_SIZE >> lod; integer lod only.  address: "clamp" or "wrap".
+    align_corners: texel i at i / (S - 1) instead of (i + .5) / S.  precision: "f32" | "f16" | "bf16" | "auto" (default
+    var2.DECODE_PRECISION).  Returns `[Q, Cout]` in out_dtype (torch.float32, or torch.uint8 = floor(v*255+.5))."""
+    pname = (precision or var2.DECODE_PRECISION).lower()
+
+    def launch(geom, g0, g1, smp, m, dst, dt, coords):
+        g0, g1 = _check_grid(g0.detach()), _check_grid(g1.detach())
+        h = L.handle(g0.device)
+        # "auto": the tensor-core kernels where they exist (C = 12, PE = 6, hidden 64), else the reference-exact kernel
+        for prec in (("f16", "f32") if pname == "auto" else (pname,)):
+            rc = L.load_library().nic_sample(h, C.byref(geom), L.ptr(g0), L.ptr(g1), L.ptr(coords), C.byref(smp), C.byref(m),
+                                             L.ptr(dst), L.DT_U8 if dt == torch.uint8 else L.DT_F32, L.PRECISIONS[prec],
+                                             L.stream_ptr(g0.device))
+            if not (rc == L.ERR_UNSUPPORTED and pname == "auto" and prec != "f32"):
+                break
+        L.check(h, rc)
+
+    return _sample(launch, fp, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table)
+
+
+def sample_codes(codes, decoder, coords, num_bits, lod=0, size=None, address="clamp", align_corners=False, precision="f16",
+                 out_dtype=torch.float32, method=None, level_table=None):
+    """`sample` straight from the saved model (`codes`: the uint8 list of fp_savable, one code per byte); the de-quantisation
+    of models.load4fp is fused into the grid read.  Tensor-core precisions only."""
+    def launch(geom, c0, c1, smp, m, dst, dt, coords):
+        for c in (c0, c1):
+            if not c.is_cuda or c.dtype != torch.uint8 or not c.is_contiguous():
+                raise TypeError("codes must be contiguous uint8 CUDA tensors")
+        h = L.handle(c0.device)
+        L.check(h, L.load_library().nic_sample_codes(h, C.byref(geom), L.ptr(c0), L.ptr(c1), num_bits, L.ptr(coords),
+                                                     C.byref(smp), C.byref(m), L.ptr(dst),
+                                                     L.DT_U8 if dt == torch.uint8 else L.DT_F32,
+                                                     L.PRECISIONS[precision.lower()], L.stream_ptr(c0.device)))
+
+    return _sample(launch, codes, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table)
+
+
 class DecodeSession:
     """A model that is decoded many times (regions, mips, repeated frames): the private tensor-core tables (16-bit
     channel-last shadow grids, per-node G1 rows, packed weight images) are built by the first `decode` and REUSED by the
@@ -352,6 +458,18 @@ class DecodeSession:
         finally:
             L.set_option(dev, L.OPT_REUSE_PREPARED, 0)
         self._fresh = True          # (a different mip level / path re-keys the tables inside the library and rebuilds)
+        return res
+
+    def sample(self, coords, lod=0, size=None, out_dtype=torch.uint8, **kw):
+        """`sample(...)` of this model, reusing the tensor-core tables like `decode` (the library rebuilds them when the mip or
+        the kernel they were built for differs)."""
+        dev = self.fp[0].device
+        L.set_option(dev, L.OPT_REUSE_PREPARED, int(self._fresh))
+        try:
+            res = sample(self.fp, self.decoder, coords, lod, size, precision=self.precision, out_dtype=out_dtype, **kw)
+        finally:
+            L.set_option(dev, L.OPT_REUSE_PREPARED, 0)
+        self._fresh = True
         return res
 
 
