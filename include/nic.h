@@ -251,6 +251,43 @@ int nic_sample_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, cons
                      const float* coords, const NicSampler* s, const NicMlp* m, void* out, int out_dtype,
                      int precision, void* stream);
 
+/* ---- per-query level of detail: trilinear mip filtering --------------------------------------------------- */
+/* Each query carries its own LOD, given directly or computed from screen-space derivatives, and is filtered across the
+ * two mips around it (2 x 4 taps in 2-D, 2 x 8 in 3-D).  For query q, with L = num_mips - 1 (every step one fp32 operation):
+ *   lambda = lod[q]                                                    (LOD given), or
+ *   lambda = 0.5 * log2f(max(|ddx[q] * E0|^2, |ddy[q] * E0|^2))        (derivatives of the normalised coordinates along the
+ *            screen's x and y; E0 = extent[0]; |v|^2 summed x first; the isotropic rule of the GL / Vulkan specifications)
+ *   lc = min(max(lambda, 0), L)                                        (fmaxf: NaN -> 0, -inf from zero derivatives -> 0)
+ *   m  = floor(lc),  t = lc - m                                        (lc = L gives t = 0)
+ *   out = (1 - t) * S_m + t * S_min(m+1, L)
+ * S_i is nic_sample's tap sum at mip i (its extent, the chain's address mode and align_corners) in fp32, before any
+ * quantisation, and the blend is the fp32 sequence of NicSampler's blend_prev; NIC_DT_U8 quantises the blended value once.
+ * So NIC_PREC_F32 equals, bit for bit, scalar nic_sample calls composed the same way (at t = 0 the result is S_m).
+ * F16 / BF16: one tensor-core pass, the 2 x 2^D taps of a query are adjacent rows of a tile; the row's mip is a decoder
+ * input (the reference's LOD column) instead of being folded into the bias, so a result may differ from a scalar-LOD
+ * tensor-core call at the same lambda by 16-bit rounding.
+ * Exactly one of `lod` ([Q] fp32) or the pair `ddx`, `ddy` ([Q, D] fp32 each) is given (NIC_ERR_ARG).  Every mip is
+ * validated as nic_sample validates one (NIC_ERR_BOUNDS, NIC_ERR_ARG); all mips share method, channels, PE channels and PE
+ * kind, geom[i].mip_level = i and geom[i].num_blocks = Q, and num_mips is in [1, NIC_MAX_MIPS] (NIC_ERR_ARG).
+ * Q * 2 * 2^D must stay below 2^31 - 128 (NIC_ERR_UNSUPPORTED).  With the triangular PE the tensor-core path needs every
+ * mip's step >= 1/4, as every mip of a model has (NIC_ERR_UNSUPPORTED otherwise). */
+#define NIC_MAX_MIPS 16
+typedef struct NicMipChain {
+  int32_t num_mips;                 /* mips 0 .. num_mips - 1 that a query may reach                                      */
+  int32_t address, align_corners;   /* as NicSampler                                                                      */
+  int32_t reserved;                 /* 0                                                                                  */
+  NicGeom geom[NIC_MAX_MIPS];       /* mip i exactly as nic_sample takes it: num_blocks = Q, block = 1, mip_level = i      */
+  const void* g0[NIC_MAX_MIPS];     /* mip i's two grids (fp32) or codes (uint8); mips of one pyramid level share them    */
+  const void* g1[NIC_MAX_MIPS];
+  int32_t extent[NIC_MAX_MIPS][3];  /* texels of mip i along x, y, z (z ignored in 2-D)                                   */
+} NicMipChain;
+int nic_sample_lod(NicHandle* h, const NicMipChain* c, const float* coords, const float* lod, const float* ddx,
+                   const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision, void* stream);
+/* The same from the saved model's uint8 codes (as nic_sample_codes).  Tensor-core precisions only. */
+int nic_sample_lod_codes(NicHandle* h, const NicMipChain* c, int bits, const float* coords, const float* lod,
+                         const float* ddx, const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision,
+                         void* stream);
+
 /* ---- fused training forward+backward (K3+K4) ----------------------------------------------------------- */
 /* One step of train_models up to loss.backward() (image_compression.py:239-265).
  *   targets [N, cout] fp32; noise: NULL (no noise), or [N, Cin] fp32 injected tensor (parity tests), or use

@@ -45,6 +45,15 @@ class NicSampler(C.Structure):
                 ("blend_weight", C.c_float), ("blend_prev", C.c_void_p)]
 
 
+MAX_MIPS = 16
+
+
+class NicMipChain(C.Structure):
+    _fields_ = [("num_mips", C.c_int32), ("address", C.c_int32), ("align_corners", C.c_int32), ("reserved", C.c_int32),
+                ("geom", NicGeom * MAX_MIPS), ("g0", C.c_void_p * MAX_MIPS), ("g1", C.c_void_p * MAX_MIPS),
+                ("extent", (C.c_int32 * 3) * MAX_MIPS)]
+
+
 class NicMlpGrad(C.Structure):
     _fields_ = [("w1", C.c_void_p), ("b1", C.c_void_p), ("w2", C.c_void_p), ("b2", C.c_void_p),
                 ("w3", C.c_void_p), ("b3", C.c_void_p)]
@@ -90,6 +99,8 @@ SYMBOLS = {
     "nic_sample": (_I, [_P, C.POINTER(NicGeom), _P, _P, _P, C.POINTER(NicSampler), C.POINTER(NicMlp), _P, _I, _I, _P]),
     "nic_sample_codes": (_I, [_P, C.POINTER(NicGeom), _P, _P, _I, _P, C.POINTER(NicSampler), C.POINTER(NicMlp), _P, _I,
                               _I, _P]),
+    "nic_sample_lod": (_I, [_P, C.POINTER(NicMipChain), _P, _P, _P, _P, C.POINTER(NicMlp), _P, _I, _I, _P]),
+    "nic_sample_lod_codes": (_I, [_P, C.POINTER(NicMipChain), _I, _P, _P, _P, _P, C.POINTER(NicMlp), _P, _I, _I, _P]),
     "nic_train_step": (_I, [_P, C.POINTER(NicGeom), _P, _P, _P, C.POINTER(NicMlp), _P, _P, _I, C.c_uint64, C.c_uint64,
                             _L, C.POINTER(NicMlpGrad), _P, _P, _P, _P, _I, _P]),
     "nic_adam_step": (_I, [_P, C.POINTER(NicAdamTensor), _I, _F, _F, _F, _F, _I, _P]),

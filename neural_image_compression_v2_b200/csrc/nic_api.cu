@@ -95,6 +95,7 @@ int nic_destroy(NicHandle* h) {
   if (h->dbg_counters) cudaFree(h->dbg_counters);
   if (h->data_scratch) cudaFree(h->data_scratch);
   if (h->sample_scratch) cudaFree(h->sample_scratch);
+  if (h->lod_chain) cudaFree(h->lod_chain);
   if (h->adam_desc) cudaFree(h->adam_desc);
   for (int i = 0; i < 2 * NIC_MAX_TIMED; ++i)
     if (h->timed_ev[i]) cudaEventDestroy(h->timed_ev[i]);
@@ -489,6 +490,97 @@ int nic_sample_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, cons
                         out_dtype, precision, st);
   h->src_code_bits = 0;
   return cuda_fail(h, rc, "nic_sample_codes");
+}
+
+// Geometry of a per-query-LOD call: every mip validated as flatten_sampler validates one, the chain's shared description,
+// and exactly one LOD source.
+static int flatten_chain(NicHandle* h, const NicMipChain* c, const float* coords, const float* lod, const float* ddx,
+                         const float* ddy, DevGeom* d, DevChain* dc, DevSampler* ds, const char* who) {
+  if (!c) return fail(h, NIC_ERR_ARG, "%s: chain is NULL", who);
+  if (c->num_mips < 1 || c->num_mips > NIC_MAX_MIPS) return fail(h, NIC_ERR_ARG, "%s: num_mips %d (1..%d)", who, c->num_mips, NIC_MAX_MIPS);
+  if (!((lod && !ddx && !ddy) || (!lod && ddx && ddy)))
+    return fail(h, NIC_ERR_ARG, "%s: give exactly one of lod or the pair ddx / ddy", who);
+  memset(dc, 0, sizeof(*dc));
+  for (int i = 0; i < c->num_mips; ++i) {
+    NicSampler s;
+    memset(&s, 0, sizeof(s));
+    s.address = c->address;
+    s.align_corners = c->align_corners;
+    for (int a = 0; a < 3; ++a) s.extent[a] = c->extent[i][a];
+    int rc = flatten_sampler(h, &c->geom[i], &s, coords, &d[i], ds, who);
+    if (rc) return rc;
+    if (c->geom[i].mip_level != i) return fail(h, NIC_ERR_ARG, "%s: geom[%d].mip_level is %d", who, i, c->geom[i].mip_level);
+    if (!c->g0[i] || !c->g1[i]) return fail(h, NIC_ERR_ARG, "%s: grids of mip %d are NULL", who, i);
+    if (d[i].method != d[0].method || d[i].C != d[0].C || d[i].PE != d[0].PE || d[i].pe_kind != d[0].pe_kind ||
+        d[i].nblocks != d[0].nblocks || memcmp(d[i].pe_div, d[0].pe_div, sizeof(d[0].pe_div)) != 0)
+      return fail(h, NIC_ERR_ARG, "%s: mip %d differs from mip 0 in method, channels, PE or query count", who, i);
+    DevMip& mp = dc->mip[i];
+    for (int a = 0; a < 3; ++a) { mp.n0[a] = d[i].n0[a]; mp.n1[a] = d[i].n1[a]; mp.S[a] = ds->S[a]; }
+    mp.step = d[i].step;
+    mp.interp = d[i].interp;
+    const int k = c->geom[i].step_log2 + 2;
+    mp.lut_shift = k < 0 ? 0 : (k > 6 ? 6 : k);
+  }
+  if (((long long)d[0].nblocks << (d[0].dim + 1)) >= (1ll << 31) - 128)
+    return fail(h, NIC_ERR_UNSUPPORTED, "%s: %d queries x %d taps reach 2^31 - 128 rows; split the batch", who, d[0].nblocks,
+                2 << d[0].dim);
+  ds->S[0] = ds->S[1] = ds->S[2] = 1;                // per mip: DevMip::S
+  dc->num_mips = c->num_mips;
+  dc->dim = d[0].dim;
+  dc->address = ds->address;
+  dc->align_corners = ds->align_corners;
+  dc->lod = lod;
+  dc->ddx = ddx;
+  dc->ddy = ddy;
+  for (int a = 0; a < 3; ++a) dc->E0[a] = a < d[0].dim ? (float)c->extent[0][a] : 1.0f;
+  return NIC_OK;
+}
+
+int nic_sample_lod(NicHandle* h, const NicMipChain* c, const float* coords, const float* lod, const float* ddx,
+                   const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+  NIC_ENTER(h);
+  DevGeom d[NIC_MAX_MIPS];
+  DevChain dc;
+  DevSampler ds;
+  int rc = flatten_chain(h, c, coords, lod, ddx, ddy, d, &dc, &ds, "nic_sample_lod");
+  if (rc) return rc;
+  MlpDev md;
+  rc = flatten_mlp(h, m, &md, d[0].cin);
+  if (rc) return rc;
+  if (!out && d[0].N > 0) return fail(h, NIC_ERR_ARG, "nic_sample_lod: out is NULL");
+  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_sample_lod: out_dtype %d", out_dtype);
+  const float* const* g0 = reinterpret_cast<const float* const*>(c->g0);
+  const float* const* g1 = reinterpret_cast<const float* const*>(c->g1);
+  if (precision == NIC_PREC_F32)
+    return cuda_fail(h, launch_sample_lod_f32(h, d, dc, ds, md, g0, g1, out, out_dtype, st), "nic_sample_lod(f32)");
+  if (precision == NIC_PREC_F16 || precision == NIC_PREC_BF16)
+    return cuda_fail(h, launch_sample_lod_tc(h, d, dc, ds, md, g0, g1, out, out_dtype, precision, st),
+                     "nic_sample_lod(tensor core)");
+  return fail(h, NIC_ERR_ARG, "nic_sample_lod: precision %d", precision);
+}
+
+int nic_sample_lod_codes(NicHandle* h, const NicMipChain* c, int bits, const float* coords, const float* lod,
+                         const float* ddx, const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision,
+                         void* stream) {
+  NIC_ENTER(h);
+  DevGeom d[NIC_MAX_MIPS];
+  DevChain dc;
+  DevSampler ds;
+  int rc = flatten_chain(h, c, coords, lod, ddx, ddy, d, &dc, &ds, "nic_sample_lod_codes");
+  if (rc) return rc;
+  MlpDev md;
+  rc = flatten_mlp(h, m, &md, d[0].cin);
+  if (rc) return rc;
+  if (bits < 1 || bits > 8) return fail(h, NIC_ERR_ARG, "nic_sample_lod_codes: bits %d (1..8)", bits);
+  if (!out && d[0].N > 0) return fail(h, NIC_ERR_ARG, "nic_sample_lod_codes: out is NULL");
+  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_sample_lod_codes: out_dtype %d", out_dtype);
+  if (precision != NIC_PREC_F16 && precision != NIC_PREC_BF16)
+    return fail(h, NIC_ERR_UNSUPPORTED, "nic_sample_lod_codes: tensor-core precisions only (f16 / bf16); unpack the codes for NIC_PREC_F32");
+  h->src_code_bits = bits;
+  rc = launch_sample_lod_tc(h, d, dc, ds, md, reinterpret_cast<const float* const*>(c->g0),
+                            reinterpret_cast<const float* const*>(c->g1), out, out_dtype, precision, st);
+  h->src_code_bits = 0;
+  return cuda_fail(h, rc, "nic_sample_lod_codes");
 }
 
 int nic_train_step(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const int64_t* origins,

@@ -180,6 +180,47 @@ __device__ __forceinline__ float sample_blend_prev(const DevSampler& s, long lon
   return __fadd_rn(__fmul_rn(__fsub_rn(1.0f, s.blend_weight), __ldg(s.prev + idx)), __fmul_rn(s.blend_weight, v));
 }
 
+// Per-query level of detail (nic.h NicMipChain): what varies from one mip of the chain to the next, and the LOD inputs.
+struct DevMip {
+  int n0[3], n1[3];       // nodes of the mip's two grids along x, y, z
+  int S[3];               // texels per axis (1 on unused axes)
+  float step;             // 2^step_log2
+  int interp;             // 0 at step 2 (fp_def.py:136)
+  int lut_shift;          // tensor-core PE: index (p << lut_shift) & 63 of the 64-entry LUT built at step 1/4
+  unsigned s0, s1;        // tensor-core path: offsets (in uint2) of the mip's shadow grids
+};
+struct DevChain {
+  int num_mips, dim, address, align_corners;
+  const float* lod;       // [Q], or NULL with ddx / ddy [Q, dim]
+  const float* ddx;
+  const float* ddy;
+  float E0[3];            // extent of mip 0 (derivatives are in normalised units)
+  DevMip mip[NIC_MAX_MIPS];
+};
+
+// lambda of query q clamped to [0, L] (nic.h nic_sample_lod; every step one fp32 operation).  fmaxf maps NaN and the -inf
+// of zero derivatives to 0.
+__device__ __forceinline__ float lod_clamped(const DevChain& c, long long q) {
+  float lam;
+  if (c.lod) {
+    lam = __ldg(c.lod + q);
+  } else {
+    float sx = 0.f, sy = 0.f;
+    for (int a = 0; a < c.dim; ++a) {
+      const float px = __fmul_rn(__ldg(c.ddx + q * c.dim + a), c.E0[a]), py = __fmul_rn(__ldg(c.ddy + q * c.dim + a), c.E0[a]);
+      sx = a == 0 ? __fmul_rn(px, px) : __fadd_rn(sx, __fmul_rn(px, px));
+      sy = a == 0 ? __fmul_rn(py, py) : __fadd_rn(sy, __fmul_rn(py, py));
+    }
+    lam = __fmul_rn(0.5f, log2f(fmaxf(sx, sy)));
+  }
+  return fminf(fmaxf(lam, 0.0f), (float)(c.num_mips - 1));
+}
+
+// out = (1 - t) * s_m + t * s_m1: the fp32 sequence of sample_blend_prev.
+__device__ __forceinline__ float lod_blend(float t, float s_m, float s_m1) {
+  return __fadd_rn(__fmul_rn(__fsub_rn(1.0f, t), s_m), __fmul_rn(t, s_m1));
+}
+
 // Linear node index in a channel-major grid [C, (z,) y, x]; indices clamped for memory safety (the reference
 // raises IndexError instead; host-known origins are validated in nic_api.cu).
 __device__ __forceinline__ long long node_index(const int* nodes, int dim, int x, int y, int z) {

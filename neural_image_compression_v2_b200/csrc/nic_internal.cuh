@@ -48,11 +48,17 @@ struct Handle {
   size_t data_scratch_bytes;
   void* sample_scratch;      // nic_sample.cu: tap texels, tap weights and tap outputs of the fp32 sampling arm
   size_t sample_scratch_bytes;
+  void* lod_chain;           // nic_sample_lod (tensor core): device copy of the call's DevChain
   int gelu_poly;             // NIC_OPT_GELU_POLY: -1 = tuned default, 0..8 = activation pairs (of 8) on the polynomial GELU
   struct PreparedKey {       // what the tables in tc_weights / tc_shadow were last built from
     const void *g0, *g1, *w1, *b1, *w2, *b2, *w3, *b3;
     int n0[3], n1[3], method, pe_kind, mip, fmt, fast, valid, code_bits, npoly;
     float step;
+    // nic_sample_lod: every mip of the chain (its grids, nodes and step); zero for the single-mip paths
+    int chain_mips;
+    const void* chain_g[2 * NIC_MAX_MIPS];
+    int chain_nodes[NIC_MAX_MIPS][6];
+    float chain_step[NIC_MAX_MIPS];
   } prepared;
   void* adam_desc;           // device copy of NicAdamTensor descriptors
   size_t adam_desc_bytes;
@@ -245,6 +251,12 @@ int launch_sample_tc(Handle* h, const DevGeom& g, const DevSampler& smp, const M
                      void* out, int out_dtype, int precision, cudaStream_t st);
 int launch_sample_f32(Handle* h, const DevGeom& g, const DevSampler& smp, const MlpDev& m, const float* g0, const float* g1,
                       void* out, int out_dtype, cudaStream_t st);
+// nic_sample_lod / nic_sample_lod_codes: g[i] describes mip i of the chain as launch_sample_* take it; c the chain.
+int launch_sample_lod_tc(Handle* h, const DevGeom* g, const DevChain& c, const DevSampler& smp, const MlpDev& m,
+                         const float* const* g0, const float* const* g1, void* out, int out_dtype, int precision,
+                         cudaStream_t st);
+int launch_sample_lod_f32(Handle* h, const DevGeom* g, const DevChain& c, const DevSampler& smp, const MlpDev& m,
+                          const float* const* g0, const float* const* g1, void* out, int out_dtype, cudaStream_t st);
 int launch_train_tc(Handle* h, const DevGeom& g, const MlpDev& m, const MlpGradDev& gm, const float* g0, const float* g1,
                     const long long* origins, const float* targets, const float* noise, int noise_bits,
                     unsigned long long seed, unsigned long long step, float grad_scale, float* dg0, float* dg1,

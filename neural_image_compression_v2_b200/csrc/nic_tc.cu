@@ -55,6 +55,18 @@ __global__ void pack_weights_kernel(MlpDev m, float lod, int KX, uint16_t* __res
   }
 }
 
+// nic_sample_lod (decode_tc_gws_kernel with TAPS = 2 * 2^D): the row carries the mip in column cin - 1 against
+// W1[:, cin - 1] and the constant 1 in column cin against b1 (the reference's own [... | pe | lod] layout), so W1' gets
+// those two columns instead of the folded bias.
+template <int FMT>
+__global__ void pack_lod_columns_kernel(MlpDev m, uint16_t* __restrict__ img) {
+  const int n = threadIdx.x;
+  if (n >= 64) return;
+  auto at = [&](int k) { return img + (k / 8) * 64 * 8 + n * 8 + (k % 8); };
+  *at(m.cin - 1) = to16<FMT>(m.w1[n * m.cin + m.cin - 1]);
+  *at(m.cin) = to16<FMT>(m.b1[n]);
+}
+
 // ------------------------------------------------------------------------------------------------ decoder-input row
 // Decoder-input row of one texel for C = 12, PE = 6 as packed 16-bit pairs (the layer-1 A operand):
 //   pairs [6j, 6j+6)         corner j of G0 (raw copy of the shadow node)
@@ -581,6 +593,12 @@ __global__ void __launch_bounds__(WS_THREADS, 1) decode_tc2d_ws_kernel(DevGeom g
 // TAPS > 0 (nic_sample: 4 in 2-D, 8 in 3-D): row n is tap n % TAPS of query n / TAPS, its texel comes from the query's
 // coordinates (sample_tap); the TAPS rows of a query are adjacent lanes of one warp, which blend their weighted sigmoid
 // outputs with a shuffle butterfly before tap 0 stores the query.  TAPS = 0 is the plain decode.
+// TAPS = 2 * 2^D (nic_sample_lod, 8 in 2-D, 16 in 3-D): every query carries its own LOD; its first 2^D rows are the taps at
+// mip m, the next 2^D the taps at mip min(m + 1, L).  Each lane computes its query's lambda and from it its row's mip; what
+// varies by mip (nodes, shadow-grid offsets, step, interpolation, extent) comes from the chain table, which `origins`
+// points at and the CTA copies to shared memory (lanes of a warp read different mips).  The mip is a decoder input
+// (column CIN - 1; the bias moves to column CIN), one PE LUT built at step 1/4 serves every mip, and the two halves of a
+// query blend after their butterflies.
 constexpr int GW_GROUP = 128;
 
 // NGT / LUTCAP: groups per CTA and capacity of the positional-encoding LUT.  The defaults (8 groups, or 5 for method 3's
@@ -598,7 +616,10 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
   constexpr int KG = 16 * 128;                       // bytes of one k-group (8 columns) of a 128-row K-major operand
   constexpr int OFF_LUT = W1_BYTES + W2_BYTES + W3_BYTES, OFF_ONE = OFF_LUT + LUTCAP * 16, OFF_ACT = OFF_ONE + 2 * KG;
   constexpr int ACT_BYTES = (KX / 8) * KG, OFF_BAR = OFF_ACT + NG * ACT_BYTES;
+  constexpr bool LODQ = TAPS == (2 << S::DIM);
+  constexpr int TQ = LODQ ? TAPS / 2 : TAPS;         // taps of one mip
   extern __shared__ __align__(128) uint8_t smem_raw[];
+  const DevChain* sChain = reinterpret_cast<const DevChain*>(smem_raw + OFF_BAR + 256);     // LODQ only
   uint8_t* sW1 = smem_raw;
   uint8_t* sW2 = sW1 + W1_BYTES;
   uint8_t* sW3 = sW2 + W2_BYTES;
@@ -618,7 +639,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
     uint4* dst = reinterpret_cast<uint4*>(smem_raw);
     for (int i = tid; i < OFF_LUT / 16; i += THREADS) dst[i] = __ldg(wimg + i);
     for (int i = tid; i < lut_n; i += THREADS) {
-      float u1 = __fmul_rn(__fmul_rn((float)i, g.step), 0.5f);
+      float u1 = __fmul_rn(__fmul_rn((float)i, LODQ ? 0.25f : g.step), 0.5f);
       uint4 e;
       auto v0 = P::pack(pe_triangular(u1, 0, 6), pe_triangular(u1, 1, 6));
       auto v1 = P::pack(pe_triangular(u1, 2, 6), pe_triangular(u1, 3, 6));
@@ -628,6 +649,11 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
       e.z = *reinterpret_cast<uint32_t*>(&v2);
       e.w = 0u;
       sLut[i] = e;
+    }
+    if constexpr (LODQ) {
+      const uint32_t* src = reinterpret_cast<const uint32_t*>(origins);
+      uint32_t* cdst = reinterpret_cast<uint32_t*>(smem_raw + OFF_BAR + 256);
+      for (int i = tid; i < (int)(sizeof(DevChain) / 4); i += THREADS) cdst[i] = __ldg(src + i);
     }
     if (slot == 0) {
       auto one = P::pack(1.0f, 0.0f);
@@ -669,6 +695,9 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
     const unsigned n = tile * TC_ROWS + row;
     const bool live = n < (unsigned)g.N;
     float tap_w = 0.f;                               // TAPS > 0: this row's filter weight (0 on dead rows)
+    float lod_t = 0.f;                               // LODQ: the query's weight of mip m + 1
+    int row_mip = 0;                                 // LODQ: this row's mip and its entry of the chain table
+    const DevMip* mp = nullptr;
     // ------------------------------------------------------------------------------------ gather -> operand buffer
     {
       Texel t;
@@ -677,23 +706,40 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
         float u[3] = {0.f, 0.f, 0.f};
 #pragma unroll
         for (int a = 0; a < S::DIM; ++a) u[a] = __ldg(smp.coords + (size_t)q * S::DIM + a);
-        const float w = sample_tap(smp, S::DIM, u, row % TAPS, t.p);
-        tap_w = live ? w : 0.f;
+        if constexpr (LODQ) {
+          const float lc = lod_clamped(*sChain, q);
+          const int m = (int)floorf(lc);
+          lod_t = __fsub_rn(lc, (float)m);
+          row_mip = min(m + (row % TAPS >= TQ), sChain->num_mips - 1);
+          mp = &sChain->mip[row_mip];
+          DevSampler sm = smp;
+#pragma unroll
+          for (int a = 0; a < 3; ++a) sm.S[a] = mp->S[a];
+          const float w = sample_tap(sm, S::DIM, u, row % TQ, t.p);
+          tap_w = live ? w : 0.f;
+        } else {
+          const float w = sample_tap(smp, S::DIM, u, row % TAPS, t.p);
+          tap_w = live ? w : 0.f;
+        }
       } else {
         t = texel_of_fast(g, live ? n : (unsigned)g.N - 1, origins);
       }
+      const int* n0 = LODQ ? mp->n0 : g.n0;
+      const int* n1 = LODQ ? mp->n1 : g.n1;
+      const uint2* s0 = LODQ ? sg.s0 + mp->s0 : sg.s0;
+      const uint2* s1 = LODQ ? sg.s1 + mp->s1 : sg.s1;
       AxisCoord ax[3];
 #pragma unroll
       for (int a = 0; a < 3; ++a) {
-        ax[a] = axis_coord(t.p[a], g.step);
-        ax[a].i0 = clampi(ax[a].i0, 0, g.n0[a] - 2 < 0 ? 0 : g.n0[a] - 2);
-        ax[a].i1 = clampi(ax[a].i1, 0, g.n1[a] - 2 < 0 ? 0 : g.n1[a] - 2);
+        ax[a] = axis_coord(t.p[a], LODQ ? mp->step : g.step);
+        ax[a].i0 = clampi(ax[a].i0, 0, n0[a] - 2 < 0 ? 0 : n0[a] - 2);
+        ax[a].i1 = clampi(ax[a].i1, 0, n1[a] - 2 < 0 ? 0 : n1[a] - 2);
       }
 #pragma unroll
       for (int j = 0; j < S::NC0; ++j) {             // G0 corners: raw copies
         const int8_t* d = S::DIM == 2 ? kCorner2D[j] : (METHOD == NIC_METHOD_3D ? kCorner3D[j] : kCorner3Dv2[j]);
         const int dz = S::DIM == 3 ? d[0] : 0;
-        const uint2* node = sg.s0 + 3 * node_lin(g.n0, S::DIM, ax[0].i0 + d[2], ax[1].i0 + d[1], ax[2].i0 + dz);
+        const uint2* node = s0 + 3 * node_lin(n0, S::DIM, ax[0].i0 + d[2], ax[1].i0 + d[1], ax[2].i0 + dz);
 #pragma unroll
         for (int q = 0; q < 3; ++q) *piece(12 * j + 4 * q) = __ldg(node + q);
       }
@@ -702,9 +748,12 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
       for (int j = 0; j < S::NC1; ++j) {
         const int8_t* d = S::DIM == 2 ? kCorner2D[j] : kCorner3D[j];
         const int dz = S::DIM == 3 ? d[0] : 0;
-        const uint2* node = sg.s1 + 3 * node_lin(g.n1, S::DIM, ax[0].i1 + d[2], ax[1].i1 + d[1], ax[2].i1 + dz);
+        const uint2* node = s1 + 3 * node_lin(n1, S::DIM, ax[0].i1 + d[2], ax[1].i1 + d[1], ax[2].i1 + dz);
         float f[3];
         g1_factors(g, j, ax, f);
+        if constexpr (LODQ) {
+          if (!mp->interp) f[0] = f[1] = f[2] = 1.0f;
+        }
         float w = f[0] * f[1];
         if (S::DIM == 3) w *= f[2];
         typename P::T2 w2 = P::cst(w);
@@ -728,7 +777,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
 #pragma unroll
       for (int a = 0; a < S::DIM; ++a) {
         if (g.pe_kind == NIC_PE_TRIANGULAR) {
-          uint4 e = sLut[t.p[a] & lut_mask];
+          uint4 e = sLut[LODQ ? ((t.p[a] << mp->lut_shift) & 63) : (t.p[a] & lut_mask)];
           tail[3 * a] = e.x;
           tail[3 * a + 1] = e.y;
           tail[3 * a + 2] = e.z;
@@ -742,7 +791,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
         }
       }
       {
-        auto one = P::pack(1.0f, 0.0f);
+        auto one = P::pack(LODQ ? (float)row_mip : 1.0f, LODQ ? 1.0f : 0.0f);     // LODQ: [... | pe | mip | 1]
         tail[(S::CIN - 1 - T0) / 2] = *reinterpret_cast<uint32_t*>(&one);
       }
 #pragma unroll
@@ -822,7 +871,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
 #pragma unroll
       for (int c = 0; c < 16; ++c) v[c] = (c < cout) ? __fmul_rn(tap_w, sigmoid_tanh(__uint_as_float(acc[c]))) : 0.f;
 #pragma unroll
-      for (int msk = 1; msk < TAPS; msk <<= 1) {
+      for (int msk = 1; msk < TQ; msk <<= 1) {
 #pragma unroll
         for (int c = 0; c < 4; ++c) v[c] = __fadd_rn(v[c], __shfl_xor_sync(0xffffffffu, v[c], msk));
         if (cout > 4) {
@@ -830,11 +879,19 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
           for (int c = 4; c < 16; ++c) v[c] = __fadd_rn(v[c], __shfl_xor_sync(0xffffffffu, v[c], msk));
         }
       }
+      if constexpr (LODQ) {                           // tap 0 holds S_m, tap TQ S_m1: tap 0 blends (1 - t) * S_m + t * S_m1
+#pragma unroll
+        for (int c = 0; c < 4; ++c) v[c] = lod_blend(lod_t, v[c], __shfl_xor_sync(0xffffffffu, v[c], TQ));
+        if (cout > 4) {
+#pragma unroll
+          for (int c = 4; c < 16; ++c) v[c] = lod_blend(lod_t, v[c], __shfl_xor_sync(0xffffffffu, v[c], TQ));
+        }
+      }
       if (live && row % TAPS == 0) {
         const size_t o = (size_t)(n / TAPS) * cout;
 #pragma unroll
         for (int c = 0; c < 16; ++c)
-          if (c < cout) store_out(out + o + c, sample_blend_prev(smp, (long long)(o + c), v[c]));
+          if (c < cout) store_out(out + o + c, LODQ ? v[c] : sample_blend_prev(smp, (long long)(o + c), v[c]));
       }
     } else if (live) {
 #pragma unroll
@@ -1367,6 +1424,127 @@ int launch_sample_tc(Handle* h, const DevGeom& gq, const DevSampler& smp, const 
     case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D, 4>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
     case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D, 8>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
     case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2, 8>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
+  }
+  return NIC_ERR_UNSUPPORTED;
+}
+
+// Per-query LOD: the shadow grids of every pyramid level the chain reaches (built once, keyed by the whole chain), the
+// W1 image with the mip column, the chain table in device memory, one pass of the general kernel with 2 * 2^D rows a query.
+template <int METHOD, int FMT, typename OutT>
+static int launch_lod_t(Handle* h, const DevGeom* gm, DevChain c, const DevSampler& smp, const MlpDev& m,
+                        const float* const* g0, const float* const* g1, OutT* out, cudaStream_t st) {
+  using S = RowShape<METHOD>;
+  constexpr int TAPS = 2 << S::DIM;
+  int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
+  if (rc) return rc;
+  size_t off[NIC_MAX_MIPS][2];
+  int first[NIC_MAX_MIPS];                           // the first mip of the chain with the same grids (one shadow each)
+  size_t total = 0;
+  for (int i = 0; i < c.num_mips; ++i) {
+    first[i] = i;
+    for (int j = 0; j < i && first[i] == i; ++j)
+      if (g0[j] == g0[i] && g1[j] == g1[i] && !memcmp(gm[j].n0, gm[i].n0, sizeof(gm[i].n0)) &&
+          !memcmp(gm[j].n1, gm[i].n1, sizeof(gm[i].n1)))
+        first[i] = j;
+    if (first[i] != i) {
+      off[i][0] = off[first[i]][0];
+      off[i][1] = off[first[i]][1];
+      continue;
+    }
+    off[i][0] = total;
+    total += ((size_t)plane_size_host(gm[i].n0, gm[i].dim) * gm[i].C * 2 + 255) & ~(size_t)255;
+    off[i][1] = total;
+    total += ((size_t)plane_size_host(gm[i].n1, gm[i].dim) * gm[i].C * 2 + 255) & ~(size_t)255;
+  }
+  if (total / 8 >= (1ull << 32)) return NIC_ERR_UNSUPPORTED;            // 32-bit shadow offsets in the chain table
+  rc = ensure_scratch(&h->tc_shadow, &h->tc_shadow_bytes, total);
+  if (rc) return rc;
+  uint8_t* shadow = (uint8_t*)h->tc_shadow;
+  for (int i = 0; i < c.num_mips; ++i) {
+    c.mip[i].s0 = (unsigned)(off[i][0] / 8);
+    c.mip[i].s1 = (unsigned)(off[i][1] / 8);
+  }
+  cudaError_t e = cudaSuccess;
+  const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : (FMT == 0 ? WS_NPOLY_F16 : WS_NPOLY_BF16);
+  if (npoly != 0 && npoly != 3) return NIC_ERR_UNSUPPORTED;
+  Handle::PreparedKey key = make_key(gm[0], m, g0[0], g1[0], FMT, 3, h->src_code_bits, npoly);
+  key.chain_mips = c.num_mips;
+  for (int i = 0; i < c.num_mips; ++i) {
+    key.chain_g[2 * i] = g0[i];
+    key.chain_g[2 * i + 1] = g1[i];
+    for (int a = 0; a < 3; ++a) { key.chain_nodes[i][a] = gm[i].n0[a]; key.chain_nodes[i][3 + a] = gm[i].n1[a]; }
+    key.chain_step[i] = gm[i].step;
+  }
+  if (!prepared_matches(h, key)) {
+    h->prepared.valid = 0;
+    for (int i = 0; i < c.num_mips; ++i) {
+      if (first[i] != i) continue;
+      e = (cudaError_t)launch_relayout<FMT>(h, gm[i], g0[i], gm[i].n0, (uint16_t*)(shadow + off[i][0]), st);
+      if (e != cudaSuccess) return (int)e;
+      e = (cudaError_t)launch_relayout<FMT>(h, gm[i], g1[i], gm[i].n1, (uint16_t*)(shadow + off[i][1]), st);
+      if (e != cudaSuccess) return (int)e;
+    }
+    pack_weights_kernel<FMT><<<16, 256, 0, st>>>(m, 0.0f, S::KX, (uint16_t*)h->tc_weights, npoly);
+    pack_lod_columns_kernel<FMT><<<1, 64, 0, st>>>(m, (uint16_t*)h->tc_weights);
+    h->launches += 2;
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return (int)e;
+    memcpy(&h->prepared, &key, sizeof(key));
+  }
+  if (!h->lod_chain && cudaMalloc(&h->lod_chain, sizeof(DevChain)) != cudaSuccess) {
+    h->lod_chain = nullptr;
+    return NIC_ERR_SCRATCH;
+  }
+  e = cudaMemcpyAsync(h->lod_chain, &c, sizeof(DevChain), cudaMemcpyHostToDevice, st);
+  if (e != cudaSuccess) return (int)e;
+  DevGeom g = gm[0];                                  // method, PE, coordinates; the rest is per row from the chain
+  g.N = (long long)g.nblocks * TAPS;
+  g.interp = 1;                                       // (g1_factors computes the weights; rows of step-2 mips drop them)
+  const long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS;
+  ShadowGeom sg = {(const uint2*)shadow, (const uint2*)shadow};
+  constexpr int IMG = b_image_bytes(64, S::KX) + b_image_bytes(64, TC_K2) + b_image_bytes(16, TC_K2);
+  constexpr int NG = gws_groups(S::KX, 0);
+  constexpr int GSMEM = IMG + TC_LUT_MAX * 16 + 2 * 2048 + NG * (S::KX / 8) * 2048 + 256 + ((sizeof(DevChain) + 15) & ~15);
+  static_assert(GSMEM <= 227 * 1024, "shared memory budget");
+  void (*kern)(DevGeom, ShadowGeom, const long long*, const uint4*, int, int, OutT*, DevSampler) =
+      npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 0, TC_LUT_MAX, TAPS>
+                 : decode_tc_gws_kernel<METHOD, FMT, OutT, 3, 0, TC_LUT_MAX, TAPS>;
+  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, GSMEM);
+  if (e != cudaSuccess) return (int)e;
+  const long long groups = (ntiles + NG - 1) / NG;
+  const int grid = (int)(groups < h->sms ? groups : h->sms);
+  {
+    KernelTimer timer(h, st);
+    kern<<<grid, NG * GW_GROUP, GSMEM, st>>>(g, sg, (const long long*)h->lod_chain, (const uint4*)h->tc_weights, m.cout, 64,
+                                             out, smp);
+  }
+  h->launches++;
+  return (int)cudaGetLastError();
+}
+
+template <int METHOD>
+static int launch_lod_m(Handle* h, const DevGeom* gm, const DevChain& c, const DevSampler& smp, const MlpDev& m,
+                        const float* const* g0, const float* const* g1, void* out, int out_dtype, int precision,
+                        cudaStream_t st) {
+  if (precision == NIC_PREC_F16) {
+    if (out_dtype == NIC_DT_U8) return launch_lod_t<METHOD, 0, uint8_t>(h, gm, c, smp, m, g0, g1, (uint8_t*)out, st);
+    return launch_lod_t<METHOD, 0, float>(h, gm, c, smp, m, g0, g1, (float*)out, st);
+  }
+  if (out_dtype == NIC_DT_U8) return launch_lod_t<METHOD, 1, uint8_t>(h, gm, c, smp, m, g0, g1, (uint8_t*)out, st);
+  return launch_lod_t<METHOD, 1, float>(h, gm, c, smp, m, g0, g1, (float*)out, st);
+}
+
+int launch_sample_lod_tc(Handle* h, const DevGeom* gm, const DevChain& c, const DevSampler& smp, const MlpDev& m,
+                         const float* const* g0, const float* const* g1, void* out, int out_dtype, int precision,
+                         cudaStream_t st) {
+  if (gm[0].nblocks == 0) return NIC_OK;
+  if (gm[0].C != 12 || gm[0].PE != 6 || m.hidden != 64 || m.cout > 16) return NIC_ERR_UNSUPPORTED;
+  for (int i = 0; i < c.num_mips; ++i)               // one 64-entry LUT at step 1/4 serves the triangular PE of every mip
+    if (gm[0].pe_kind == NIC_PE_TRIANGULAR && gm[i].step < 0.25f) return NIC_ERR_UNSUPPORTED;
+  switch (gm[0].method) {
+    case NIC_METHOD_2D: return launch_lod_m<NIC_METHOD_2D>(h, gm, c, smp, m, g0, g1, out, out_dtype, precision, st);
+    case NIC_METHOD_3D: return launch_lod_m<NIC_METHOD_3D>(h, gm, c, smp, m, g0, g1, out, out_dtype, precision, st);
+    case NIC_METHOD_3D_V2: return launch_lod_m<NIC_METHOD_3D_V2>(h, gm, c, smp, m, g0, g1, out, out_dtype, precision, st);
   }
   return NIC_ERR_UNSUPPORTED;
 }

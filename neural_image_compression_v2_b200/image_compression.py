@@ -358,8 +358,62 @@ def _sample_passes(lod, size, table):
     return [(m, 1.0), (m + 1, t)]
 
 
-def _sample(launch, fp_like, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table):
-    """Common body of sample / sample_codes; launch(geom, grid0, grid1, sampler, mlp, out, out_dtype) calls the library."""
+def _lod_args(lod, grad, size):
+    """Is this a per-query LOD call (lod a tensor, or grad given)?  Checks what needs no tensor."""
+    if grad is None and not torch.is_tensor(lod):
+        return False
+    if grad is not None and lod is not None:
+        raise ValueError("give lod or grad, not both")
+    if size is not None:
+        raise ValueError("size may not be given with a per-query lod or grad (each mip has its own extent)")
+    return True
+
+
+def _lod_inputs(lod, grad, coords, dim):
+    """(lod, ddx, ddy) of a per-query LOD call (lod a tensor [Q], or grad = (ddx, ddy) tensors [Q, D])."""
+    q = coords.shape[0] if torch.is_tensor(coords) and coords.dim() == 2 else None      # (coords are checked next)
+    named = [("lod", lod, (q,))] if grad is None else []
+    if grad is not None:
+        if not isinstance(grad, (tuple, list)) or len(grad) != 2:
+            raise TypeError("grad must be a pair (ddx, ddy) of float32 tensors [Q, D]")
+        named = [("ddx", grad[0], (q, dim)), ("ddy", grad[1], (q, dim))]
+    for name, t, shape in named:
+        if not torch.is_tensor(t) or t.dtype != torch.float32 or not t.is_contiguous():
+            raise TypeError(f"{name} must be a contiguous float32 tensor {list(shape)}")
+        if q is not None and tuple(t.shape) != shape:
+            raise ValueError(f"{name} must be {list(shape)}, got {tuple(t.shape)}")
+    for name, t, _ in named:
+        if not t.is_cuda:
+            raise L.NicError(-3, f"{name} must be a CUDA tensor (no CPU fallback)")
+        if q is not None and coords.is_cuda and t.device != coords.device:
+            raise ValueError(f"{name} is on {t.device}, coords on {coords.device}")
+    return (lod, None, None) if grad is None else (None, grad[0], grad[1])
+
+
+def _mip_chain(fp_like, q, address, align_corners, method, table):
+    """NicMipChain of mips 0 .. min(MAX_MIP_LEVEL, max(table)), each at its default extent IMAGE_SIZE >> mip."""
+    dim = 2 if method == L.METHOD_2D else 3
+    last = min(var2.MAX_MIP_LEVEL, max(table))
+    if last + 1 > L.MAX_MIPS:
+        raise ValueError(f"a per-query lod reaches at most {L.MAX_MIPS} mips; the table has {last + 1}")
+    c = L.NicMipChain()
+    c.num_mips, c.address, c.align_corners = last + 1, _ADDRESS[address], int(bool(align_corners))
+    grids = []
+    for mip in range(last + 1):
+        fl = table[mip]
+        g0, g1 = fp_like[fl * 2], fp_like[fl * 2 + 1]
+        grids += [g0, g1]
+        c.geom[mip] = L.make_geom(method, g0, g1, 1, q, _step_log2(mip, fl), mip, var2.PE_CHANNELS, _pe_kind(method))
+        c.g0[mip], c.g1[mip] = L.ptr(g0), L.ptr(g1)
+        for a in range(3):
+            c.extent[mip][a] = var2.IMAGE_SIZE // pow(2, mip) if a < dim else 1
+    return c, grids
+
+
+def _sample(launch, launch_lod, fp_like, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table,
+            grad=None):
+    """Common body of sample / sample_codes; launch(geom, grid0, grid1, sampler, mlp, out, out_dtype) calls the library for
+    one mip, launch_lod(chain, grids, mlp, out, out_dtype, coords, lod, ddx, ddy) for a per-query lod."""
     method = _method() if method is None else method
     dim = 2 if method == L.METHOD_2D else 3
     table = feature_pyramid_mip_levels() if level_table is None else level_table
@@ -367,12 +421,19 @@ def _sample(launch, fp_like, decoder, coords, lod, size, address, align_corners,
         raise ValueError(f"address must be 'clamp' or 'wrap', got {address!r}")
     if out_dtype not in (torch.float32, torch.uint8):
         raise TypeError("out_dtype must be torch.float32 or torch.uint8")
-    passes = _sample_passes(lod, size, table)
+    per_query = _lod_args(lod, grad, size)
+    passes = None if per_query else _sample_passes(0 if lod is None else lod, size, table)
+    lod_inputs = _lod_inputs(lod, grad, coords, dim) if per_query else None
     coords = _sample_coords(coords, dim)
     params = [p.detach().contiguous() for p in decoder.parameters_list()]
     m = L.make_mlp(params)
     q = coords.shape[0]
     out = torch.empty((q, m.cout), dtype=out_dtype, device=coords.device)
+    if per_query:
+        if q > 0:
+            chain, grids = _mip_chain(fp_like, q, address, align_corners, method, table)
+            launch_lod(chain, grids, m, out, out_dtype, coords, *lod_inputs)
+        return out
     prev = None
     for i, (mip, t) in enumerate(passes):
         fl = table[mip]
@@ -392,8 +453,8 @@ def _sample(launch, fp_like, decoder, coords, lod, size, address, align_corners,
     return out
 
 
-def sample(fp, decoder, coords, lod=0, size=None, address="clamp", align_corners=False, precision=None,
-           out_dtype=torch.float32, method=None, level_table=None):
+def sample(fp, decoder, coords, lod=None, size=None, address="clamp", align_corners=False, precision=None,
+           out_dtype=torch.float32, method=None, level_table=None, grad=None):
     """Filtered sampling at continuous coordinates: bilinear (2-D) / trilinear (3-D) reads of the decoded mip, as a renderer
     samples a texture or a colour LUT is applied, without materialising the taps (nic.h nic_sample has the exact rule).
 
@@ -401,7 +462,12 @@ def sample(fp, decoder, coords, lod=0, size=None, address="clamp", align_corners
     lod blends the two mips around it ((1 - t) * mip m + t * mip m + 1), clamped to [0, MAX_MIP_LEVEL].  size: texel extent
     of the mip (int or per-axis tuple), default IMAGE_SIZE >> lod; integer lod only.  address: "clamp" or "wrap".
     align_corners: texel i at i / (S - 1) instead of (i + .5) / S.  precision: "f32" | "f16" | "bf16" | "auto" (default
-    var2.DECODE_PRECISION).  Returns `[Q, Cout]` in out_dtype (torch.float32, or torch.uint8 = floor(v*255+.5))."""
+    var2.DECODE_PRECISION).  Returns `[Q, Cout]` in out_dtype (torch.float32, or torch.uint8 = floor(v*255+.5)).
+
+    Per-query level of detail (nic.h nic_sample_lod has the exact rule): lod a float32 CUDA tensor `[Q]`, or
+    grad=(ddx, ddy), float32 CUDA tensors `[Q, D]` holding the derivatives of the normalised coordinates along the screen's
+    x and y (lambda = log2 of the longer one in texels of mip 0).  Each query blends the two mips around its clamped lambda,
+    over mips 0 .. min(MAX_MIP_LEVEL, max(level_table)) at their default extents (no `size`), in one pass."""
     pname = (precision or var2.DECODE_PRECISION).lower()
 
     def launch(geom, g0, g1, smp, m, dst, dt, coords):
@@ -416,24 +482,49 @@ def sample(fp, decoder, coords, lod=0, size=None, address="clamp", align_corners
                 break
         L.check(h, rc)
 
-    return _sample(launch, fp, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table)
+    def launch_lod(chain, grids, m, dst, dt, coords, lod, ddx, ddy):
+        for g in grids:
+            _check_grid(g.detach())
+        h = L.handle(coords.device)
+        for prec in (("f16", "f32") if pname == "auto" else (pname,)):
+            rc = L.load_library().nic_sample_lod(h, C.byref(chain), L.ptr(coords), L.ptr(lod), L.ptr(ddx), L.ptr(ddy),
+                                                 C.byref(m), L.ptr(dst), L.DT_U8 if dt == torch.uint8 else L.DT_F32,
+                                                 L.PRECISIONS[prec], L.stream_ptr(coords.device))
+            if not (rc == L.ERR_UNSUPPORTED and pname == "auto" and prec != "f32"):
+                break
+        L.check(h, rc)
+
+    return _sample(launch, launch_lod, fp, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table,
+                   grad)
 
 
-def sample_codes(codes, decoder, coords, num_bits, lod=0, size=None, address="clamp", align_corners=False, precision="f16",
-                 out_dtype=torch.float32, method=None, level_table=None):
+def sample_codes(codes, decoder, coords, num_bits, lod=None, size=None, address="clamp", align_corners=False,
+                 precision="f16", out_dtype=torch.float32, method=None, level_table=None, grad=None):
     """`sample` straight from the saved model (`codes`: the uint8 list of fp_savable, one code per byte); the de-quantisation
     of models.load4fp is fused into the grid read.  Tensor-core precisions only."""
-    def launch(geom, c0, c1, smp, m, dst, dt, coords):
-        for c in (c0, c1):
+    def check_codes(cs):
+        for c in cs:
             if not c.is_cuda or c.dtype != torch.uint8 or not c.is_contiguous():
                 raise TypeError("codes must be contiguous uint8 CUDA tensors")
+
+    def launch_lod(chain, grids, m, dst, dt, coords, lod, ddx, ddy):
+        check_codes(grids)
+        h = L.handle(coords.device)
+        L.check(h, L.load_library().nic_sample_lod_codes(h, C.byref(chain), num_bits, L.ptr(coords), L.ptr(lod), L.ptr(ddx),
+                                                         L.ptr(ddy), C.byref(m), L.ptr(dst),
+                                                         L.DT_U8 if dt == torch.uint8 else L.DT_F32,
+                                                         L.PRECISIONS[precision.lower()], L.stream_ptr(coords.device)))
+
+    def launch(geom, c0, c1, smp, m, dst, dt, coords):
+        check_codes((c0, c1))
         h = L.handle(c0.device)
         L.check(h, L.load_library().nic_sample_codes(h, C.byref(geom), L.ptr(c0), L.ptr(c1), num_bits, L.ptr(coords),
                                                      C.byref(smp), C.byref(m), L.ptr(dst),
                                                      L.DT_U8 if dt == torch.uint8 else L.DT_F32,
                                                      L.PRECISIONS[precision.lower()], L.stream_ptr(c0.device)))
 
-    return _sample(launch, codes, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table)
+    return _sample(launch, launch_lod, codes, decoder, coords, lod, size, address, align_corners, out_dtype, method,
+                   level_table, grad)
 
 
 class DecodeSession:
@@ -460,9 +551,9 @@ class DecodeSession:
         self._fresh = True          # (a different mip level / path re-keys the tables inside the library and rebuilds)
         return res
 
-    def sample(self, coords, lod=0, size=None, out_dtype=torch.uint8, **kw):
+    def sample(self, coords, lod=None, size=None, out_dtype=torch.uint8, **kw):
         """`sample(...)` of this model, reusing the tensor-core tables like `decode` (the library rebuilds them when the mip or
-        the kernel they were built for differs)."""
+        the kernel they were built for differs).  A per-query lod or grad= reuses the tables of the whole mip chain."""
         dev = self.fp[0].device
         L.set_option(dev, L.OPT_REUSE_PREPARED, int(self._fresh))
         try:
