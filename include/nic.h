@@ -288,6 +288,41 @@ int nic_sample_lod_codes(NicHandle* h, const NicMipChain* c, int bits, const flo
                          const float* ddx, const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision,
                          void* stream);
 
+/* ---- applying a baked 3-D colour LUT to images ------------------------------------------------------------ */
+/* A colour LUT is decoded once (nic_decode / nic_decode_codes of the whole 3-D mip, fp32 out), packed into a table of 4-channel
+ * texels by nic_lut_pack (the bake), and then applied to every pixel of an image by nic_lut_apply, a pure gather: no decoder
+ * runs per pixel.  Channel k of a pixel indexes LUT axis k: R -> x (the first, slowest axis of the decoded [Sx, Sy, Sz, C]),
+ * G -> y, B -> z, which is nic_sample's coordinate order.  For each pixel (every step one fp32 operation):
+ *   u  = NIC_DT_U8 input: __fdiv_rn((float)v, 255.f); NIC_DT_F32 input: the value as given;
+ *   on each axis nic_sample's rule with align_corners = 1 and NIC_ADDRESS_CLAMP: p = u * (S - 1), clamped to +-2^24 (NaN ->
+ *   -2^24), i0 = floor(p), f = p - i0; the low tap i0 and the high tap i0 + 1, each clamped to [0, S - 1];
+ *   NIC_INTERP_TRILINEAR: the 8 taps, weights and order of nic_sample (x slowest; weight = product of the per-axis weights,
+ *     x first), summed as acc = 0, acc = acc + w_k * v_k for k = 0..7 (each product and sum rounded): fp32 apply of a table
+ *     baked at NIC_PREC_F32 equals nic_sample at NIC_PREC_F32 bit for bit;
+ *   NIC_INTERP_TETRAHEDRAL: the axes ordered by descending f, ties broken x before y before z (a stable sort): a1, a2, a3.
+ *     Corners v0 = c(lo), v1 = c(lo + e_a1), v2 = c(lo + e_a1 + e_a2), v3 = c(hi) (each step moves one axis from its low tap to
+ *     its high tap); weights w0 = 1 - f_a1, w1 = f_a1 - f_a2, w2 = f_a2 - f_a3, w3 = f_a3; acc = 0, acc = acc + w_k * v_k for
+ *     k = 0..3.  It reads 4 texels instead of 8 and reproduces the table exactly on the neutral axis of a cubic table;
+ *   out: NIC_DT_F32 the fp32 result; NIC_DT_U8 floor(v * 255 + .5) of it, clamped to [0, 255] (quantised once).
+ * Errors: NIC_ERR_ARG for a NULL pointer with pixels > 0, a bad dtype, cout, interp or reserved field, an extent < 1, pixels < 0
+ * or src / dst overlapping (no in-place apply); NIC_ERR_UNSUPPORTED for Sx * Sy * Sz >= 2^31.  pixels == 0 launches nothing. */
+enum { NIC_INTERP_TRILINEAR = 0, NIC_INTERP_TETRAHEDRAL = 1 };
+typedef struct NicLut {
+  const void* table;     /* [Sx][Sy][Sz][4] of table_dtype, x slowest (nic_decode's texel order); channels >= cout are 0 */
+  int32_t table_dtype;   /* NIC_DT_F32 (the exact arm) or NIC_DT_F16                                               */
+  int32_t cout;          /* 1..4                                                                                   */
+  int32_t extent[3];     /* Sx, Sy, Sz >= 1, Sx*Sy*Sz < 2^31                                                       */
+  int32_t reserved;      /* 0                                                                                      */
+} NicLut;
+/* dense [Sx, Sy, Sz, cout] fp32 (what nic_decode / nic_decode_codes write for a 3-D block) -> the table layout above
+ * (NIC_DT_F16: __float2half_rn of each value; channels cout..3 written as 0). */
+int nic_lut_pack(NicHandle* h, const float* dense, const int32_t extent[3], int cout, void* table, int table_dtype,
+                 void* stream);
+/* src [pixels, 3] (NIC_DT_U8 or NIC_DT_F32) -> dst [pixels, cout] (NIC_DT_U8 or NIC_DT_F32); dst must not overlap src.
+ * Any element alignment of src and dst is accepted (a view that starts 3 bytes into a buffer works). */
+int nic_lut_apply(NicHandle* h, const NicLut* lut, const void* src, int src_dtype, int64_t pixels, void* dst,
+                  int dst_dtype, int interp, void* stream);
+
 /* ---- fused training forward+backward (K3+K4) ----------------------------------------------------------- */
 /* One step of train_models up to loss.backward() (image_compression.py:239-265).
  *   targets [N, cout] fp32; noise: NULL (no noise), or [N, Cin] fp32 injected tensor (parity tests), or use

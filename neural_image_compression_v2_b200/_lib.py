@@ -54,6 +54,14 @@ class NicMipChain(C.Structure):
                 ("extent", (C.c_int32 * 3) * MAX_MIPS)]
 
 
+INTERP_TRILINEAR, INTERP_TETRAHEDRAL = 0, 1
+
+
+class NicLut(C.Structure):
+    _fields_ = [("table", C.c_void_p), ("table_dtype", C.c_int32), ("cout", C.c_int32), ("extent", C.c_int32 * 3),
+                ("reserved", C.c_int32)]
+
+
 class NicMlpGrad(C.Structure):
     _fields_ = [("w1", C.c_void_p), ("b1", C.c_void_p), ("w2", C.c_void_p), ("b2", C.c_void_p),
                 ("w3", C.c_void_p), ("b3", C.c_void_p)]
@@ -101,6 +109,8 @@ SYMBOLS = {
                               _I, _P]),
     "nic_sample_lod": (_I, [_P, C.POINTER(NicMipChain), _P, _P, _P, _P, C.POINTER(NicMlp), _P, _I, _I, _P]),
     "nic_sample_lod_codes": (_I, [_P, C.POINTER(NicMipChain), _I, _P, _P, _P, _P, C.POINTER(NicMlp), _P, _I, _I, _P]),
+    "nic_lut_pack": (_I, [_P, _P, C.POINTER(C.c_int32), _I, _P, _I, _P]),
+    "nic_lut_apply": (_I, [_P, C.POINTER(NicLut), _P, _I, _L, _P, _I, _I, _P]),
     "nic_train_step": (_I, [_P, C.POINTER(NicGeom), _P, _P, _P, C.POINTER(NicMlp), _P, _P, _I, C.c_uint64, C.c_uint64,
                             _L, C.POINTER(NicMlpGrad), _P, _P, _P, _P, _I, _P]),
     "nic_adam_step": (_I, [_P, C.POINTER(NicAdamTensor), _I, _F, _F, _F, _F, _I, _P]),

@@ -14,7 +14,7 @@ LIB = os.path.join(HERE, "libnic.so")
 # (source, extra defines, object name)
 UNITS = [("nic_api.cu", [], "nic_api.o"), ("nic_f32.cu", [], "nic_f32.o"), ("nic_optim.cu", [], "nic_optim.o"),
          ("nic_tc.cu", [], "nic_tc.o"), ("nic_gather.cu", [], "nic_gather.o"), ("nic_train_tc.cu", [], "nic_train_tc.o"),
-         ("nic_data.cu", [], "nic_data.o"), ("nic_sample.cu", [], "nic_sample.o"),
+         ("nic_data.cu", [], "nic_data.o"), ("nic_sample.cu", [], "nic_sample.o"), ("nic_lut.cu", [], "nic_lut.o"),
          ("nic_f32_mlp.cu", ["-DNIC_H=64", "-DNIC_PART=0"], "nic_f32_fwd64.o"),
          ("nic_f32_mlp.cu", ["-DNIC_H=64", "-DNIC_PART=1"], "nic_f32_bwd64.o"),
          ("nic_f32_mlp.cu", ["-DNIC_H=32", "-DNIC_PART=0"], "nic_f32_fwd32.o"),

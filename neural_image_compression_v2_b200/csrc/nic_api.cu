@@ -583,6 +583,51 @@ int nic_sample_lod_codes(NicHandle* h, const NicMipChain* c, int bits, const flo
   return cuda_fail(h, rc, "nic_sample_lod_codes");
 }
 
+// Texels of a LUT extent: NIC_ERR_ARG for an extent < 1, NIC_ERR_UNSUPPORTED from 2^31 texels on (int texel indices).
+static int lut_texels(NicHandle* h, const int32_t* extent, long long* texels, const char* who) {
+  if (!extent) return fail(h, NIC_ERR_ARG, "%s: extent is NULL", who);
+  for (int a = 0; a < 3; ++a)
+    if (extent[a] < 1) return fail(h, NIC_ERR_ARG, "%s: extent %d on axis %d", who, extent[a], a);
+  *texels = (long long)extent[0] * extent[1] * extent[2];
+  if (*texels >= (1ll << 31)) return fail(h, NIC_ERR_UNSUPPORTED, "%s: %lld texels reach 2^31", who, *texels);
+  return NIC_OK;
+}
+
+int nic_lut_pack(NicHandle* h, const float* dense, const int32_t extent[3], int cout, void* table, int table_dtype,
+                 void* stream) {
+  NIC_ENTER(h);
+  if (!dense || !table) return fail(h, NIC_ERR_ARG, "nic_lut_pack: NULL pointer");
+  if (cout < 1 || cout > 4) return fail(h, NIC_ERR_ARG, "nic_lut_pack: cout %d (1..4)", cout);
+  if (table_dtype != NIC_DT_F32 && table_dtype != NIC_DT_F16) return fail(h, NIC_ERR_ARG, "nic_lut_pack: table_dtype %d", table_dtype);
+  long long texels = 0;
+  int rc = lut_texels(h, extent, &texels, "nic_lut_pack");
+  if (rc) return rc;
+  return cuda_fail(h, launch_lut_pack(h, dense, texels, cout, table, table_dtype, st), "nic_lut_pack");
+}
+
+int nic_lut_apply(NicHandle* h, const NicLut* lut, const void* src, int src_dtype, int64_t pixels, void* dst,
+                  int dst_dtype, int interp, void* stream) {
+  NIC_ENTER(h);
+  if (!lut) return fail(h, NIC_ERR_ARG, "nic_lut_apply: lut is NULL");
+  if (pixels < 0) return fail(h, NIC_ERR_ARG, "nic_lut_apply: pixels %lld", (long long)pixels);
+  if (pixels > 0 && (!lut->table || !src || !dst)) return fail(h, NIC_ERR_ARG, "nic_lut_apply: NULL pointer");
+  if (lut->table_dtype != NIC_DT_F32 && lut->table_dtype != NIC_DT_F16)
+    return fail(h, NIC_ERR_ARG, "nic_lut_apply: table_dtype %d", lut->table_dtype);
+  if (lut->cout < 1 || lut->cout > 4) return fail(h, NIC_ERR_ARG, "nic_lut_apply: cout %d (1..4)", lut->cout);
+  if (lut->reserved != 0) return fail(h, NIC_ERR_ARG, "nic_lut_apply: reserved is %d (must be 0)", lut->reserved);
+  if (src_dtype != NIC_DT_U8 && src_dtype != NIC_DT_F32) return fail(h, NIC_ERR_ARG, "nic_lut_apply: src_dtype %d", src_dtype);
+  if (dst_dtype != NIC_DT_U8 && dst_dtype != NIC_DT_F32) return fail(h, NIC_ERR_ARG, "nic_lut_apply: dst_dtype %d", dst_dtype);
+  if (interp != NIC_INTERP_TRILINEAR && interp != NIC_INTERP_TETRAHEDRAL) return fail(h, NIC_ERR_ARG, "nic_lut_apply: interp %d", interp);
+  long long texels = 0;
+  int rc = lut_texels(h, lut->extent, &texels, "nic_lut_apply");
+  if (rc) return rc;
+  if (pixels == 0) return NIC_OK;
+  const uintptr_t s0 = (uintptr_t)src, s1 = s0 + (uintptr_t)pixels * 3 * (src_dtype == NIC_DT_U8 ? 1 : 4);
+  const uintptr_t d0 = (uintptr_t)dst, d1 = d0 + (uintptr_t)pixels * lut->cout * (dst_dtype == NIC_DT_U8 ? 1 : 4);
+  if (s0 < d1 && d0 < s1) return fail(h, NIC_ERR_ARG, "nic_lut_apply: src and dst overlap (no in-place apply)");
+  return cuda_fail(h, launch_lut_apply(h, *lut, src, src_dtype, pixels, dst, dst_dtype, interp, st), "nic_lut_apply");
+}
+
 int nic_train_step(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const int64_t* origins,
                    const NicMlp* m, const float* targets, const float* noise, int noise_bits, uint64_t seed,
                    uint64_t step, int64_t global_n, const NicMlpGrad* gm, float* dg0, float* dg1, float* loss_sum,

@@ -174,6 +174,47 @@ __device__ __forceinline__ float sample_tap(const DevSampler& s, int dim, const 
   return w;
 }
 
+// Tetrahedral interpolation of an S[0] x S[1] x S[2] table at normalised coordinates u[0..3) (nic.h nic_lut_apply), on
+// sample_tap's axis rule with align_corners and clamp addressing: writes the texels of the 4 corners to p[k][0..3) and their
+// weights to w[k], k = 0..3 in summation order.  The axes are ordered by descending fraction with a fixed compare-exchange
+// network (swaps only on a strictly larger fraction, so ties keep x before y before z), which compiles to selects.
+__device__ __forceinline__ void tetra_corners(const int* S, const float* u, int (*p)[3], float* w) {
+  float f[3];
+  int lo[3], hi[3];
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    float x = __fmul_rn(u[a], (float)(S[a] - 1));
+    x = fminf(fmaxf(x, -16777216.0f), 16777216.0f);
+    const float i0 = floorf(x);
+    f[a] = __fsub_rn(x, i0);
+    lo[a] = clampi((int)i0, 0, S[a] - 1);
+    hi[a] = clampi((int)i0 + 1, 0, S[a] - 1);
+  }
+  float f1 = f[0], f2 = f[1], f3 = f[2];
+  int m1 = 1, m2 = 2, m3 = 4;                       // the axis of each rank as a bit: x = 1, y = 2, z = 4
+  auto cx = [](float& fa, int& ma, float& fb, int& mb) {
+    const bool sw = fb > fa;
+    const float tf = sw ? fb : fa;
+    const int tm = sw ? mb : ma;
+    fb = sw ? fa : fb;
+    mb = sw ? ma : mb;
+    fa = tf;
+    ma = tm;
+  };
+  cx(f1, m1, f2, m2);
+  cx(f2, m2, f3, m3);
+  cx(f1, m1, f2, m2);
+  const int mask[4] = {0, m1, m1 | m2, 7};
+#pragma unroll
+  for (int k = 0; k < 4; ++k)
+#pragma unroll
+    for (int a = 0; a < 3; ++a) p[k][a] = (mask[k] >> a) & 1 ? hi[a] : lo[a];
+  w[0] = __fsub_rn(1.0f, f1);
+  w[1] = __fsub_rn(f1, f2);
+  w[2] = __fsub_rn(f2, f3);
+  w[3] = f3;
+}
+
 // The last step of a sample: the optional blend with the previous mip's result, element `idx` of [Q, cout].
 __device__ __forceinline__ float sample_blend_prev(const DevSampler& s, long long idx, float v) {
   if (!s.prev) return v;

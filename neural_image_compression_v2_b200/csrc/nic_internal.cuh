@@ -257,6 +257,10 @@ int launch_sample_lod_tc(Handle* h, const DevGeom* g, const DevChain& c, const D
                          cudaStream_t st);
 int launch_sample_lod_f32(Handle* h, const DevGeom* g, const DevChain& c, const DevSampler& smp, const MlpDev& m,
                           const float* const* g0, const float* const* g1, void* out, int out_dtype, cudaStream_t st);
+// nic_lut_pack / nic_lut_apply (nic_lut.cu): arguments validated by nic_api.cu.
+int launch_lut_pack(Handle* h, const float* dense, long long texels, int cout, void* table, int table_dtype, cudaStream_t st);
+int launch_lut_apply(Handle* h, const NicLut& lut, const void* src, int src_dtype, long long pixels, void* dst, int dst_dtype,
+                     int interp, cudaStream_t st);
 int launch_train_tc(Handle* h, const DevGeom& g, const MlpDev& m, const MlpGradDev& gm, const float* g0, const float* g1,
                     const long long* origins, const float* targets, const float* noise, int noise_bits,
                     unsigned long long seed, unsigned long long step, float grad_scale, float* dg0, float* dg1,

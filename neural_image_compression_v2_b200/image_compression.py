@@ -527,6 +527,102 @@ def sample_codes(codes, decoder, coords, num_bits, lod=None, size=None, address=
                    level_table, grad)
 
 
+# ------------------------------------------------------------------------------------------------ baked colour LUTs
+_INTERP = {"trilinear": L.INTERP_TRILINEAR, "tetrahedral": L.INTERP_TETRAHEDRAL}
+_TABLE_DT = {torch.float32: L.DT_F32, torch.float16: L.DT_F16}
+
+
+class BakedLut:
+    """A 3-D colour LUT decoded once and packed for application to images (nic.h nic_lut_apply has the exact rule): `apply`
+    is a pure gather per pixel, no decoder runs.  `table` is the `[Sx, Sy, Sz, 4]` float32 or float16 CUDA tensor (x slowest,
+    channels from `cout` on are 0), `extent` is (Sx, Sy, Sz) and `cout` the number of output channels (1..4).  Build one with
+    `bake_lut`, `bake_lut_codes` or `BakedLut.from_table`."""
+
+    def __init__(self, table, extent, cout):
+        self.table, self.extent, self.cout = table, tuple(int(e) for e in extent), int(cout)
+
+    @classmethod
+    def from_table(cls, dense, table_dtype=torch.float32):
+        """A plain LUT: `dense` is a contiguous float32 CUDA tensor `[Sx, Sy, Sz, C]`, C in 1..4 (what `decode` writes for a
+        3-D block), packed as float32 (exact) or float16 (`__float2half_rn` of each value)."""
+        if not torch.is_tensor(dense) or dense.dtype != torch.float32 or not dense.is_contiguous():
+            raise TypeError("dense must be a contiguous float32 tensor [Sx, Sy, Sz, C]")
+        if dense.dim() != 4 or not 1 <= dense.shape[3] <= 4 or dense.numel() == 0:
+            raise ValueError(f"dense must be [Sx, Sy, Sz, C] with every extent >= 1 and C in 1..4, got {tuple(dense.shape)}")
+        if table_dtype not in _TABLE_DT:
+            raise TypeError("table_dtype must be torch.float32 or torch.float16")
+        if not dense.is_cuda:
+            raise L.NicError(-3, "dense must be a CUDA tensor (no CPU fallback)")
+        extent, cout = tuple(dense.shape[:3]), int(dense.shape[3])
+        table = torch.empty(extent + (4,), dtype=table_dtype, device=dense.device)
+        h = L.handle(dense.device)
+        L.check(h, L.load_library().nic_lut_pack(h, L.ptr(dense), (C.c_int32 * 3)(*extent), cout, L.ptr(table),
+                                                 _TABLE_DT[table_dtype], L.stream_ptr(dense.device)))
+        return cls(table, extent, cout)
+
+    def apply(self, image, interpolation="trilinear", out_dtype=torch.uint8, out=None):
+        """Applies the LUT to every pixel of `image`, a contiguous uint8 or float32 CUDA tensor `[..., 3]` (`[H, W, 3]`,
+        `[F, H, W, 3]`, `[N, 3]`): R, G, B index the x, y, z axes; uint8 values are read as v / 255, floats as given
+        (align_corners, clamped at the edges).  interpolation: "trilinear" (8 texels) or "tetrahedral" (4 texels, exact on
+        the neutral axis).  Returns `[..., cout]` in out_dtype (torch.uint8 = floor(v*255+.5), or torch.float32), written
+        into `out` when given (a contiguous tensor of that shape and dtype that does not overlap `image`)."""
+        if interpolation not in _INTERP:
+            raise ValueError(f"interpolation must be 'trilinear' or 'tetrahedral', got {interpolation!r}")
+        if out_dtype not in (torch.float32, torch.uint8):
+            raise TypeError("out_dtype must be torch.float32 or torch.uint8")
+        if not torch.is_tensor(image) or image.dtype not in (torch.uint8, torch.float32) or not image.is_contiguous():
+            raise TypeError("image must be a contiguous uint8 or float32 tensor [..., 3]")
+        if image.dim() < 1 or image.shape[-1] != 3:
+            raise ValueError(f"image must be [..., 3] (R, G, B last), got {tuple(image.shape)}")
+        if not image.is_cuda:
+            raise L.NicError(-3, "image must be a CUDA tensor (no CPU fallback)")
+        if image.device != self.table.device:
+            raise ValueError(f"image is on {image.device}, the LUT on {self.table.device}")
+        shape = tuple(image.shape[:-1]) + (self.cout,)
+        if out is None:
+            out = torch.empty(shape, dtype=out_dtype, device=image.device)
+        elif (not torch.is_tensor(out) or tuple(out.shape) != shape or out.dtype != out_dtype or not out.is_contiguous()
+              or out.device != image.device):
+            raise ValueError(f"out must be a contiguous {out_dtype} tensor of shape {shape} on {image.device}")
+        pixels = image.numel() // 3
+        s0, d0 = image.data_ptr(), out.data_ptr()
+        if pixels > 0 and s0 < d0 + out.numel() * out.element_size() and d0 < s0 + image.numel() * image.element_size():
+            raise ValueError("out overlaps image (the LUT is not applied in place)")
+        lut = L.NicLut()
+        lut.table, lut.table_dtype, lut.cout = self.table.data_ptr(), _TABLE_DT[self.table.dtype], self.cout
+        for a in range(3):
+            lut.extent[a] = self.extent[a]
+        h = L.handle(image.device)
+        L.check(h, L.load_library().nic_lut_apply(h, C.byref(lut), L.ptr(image), L.DT_U8 if image.dtype == torch.uint8 else L.DT_F32,
+                                                  pixels, L.ptr(out), L.DT_U8 if out_dtype == torch.uint8 else L.DT_F32,
+                                                  _INTERP[interpolation], L.stream_ptr(image.device)))
+        return out
+
+
+def _lut_method(method):
+    method = _method() if method is None else method
+    if method == L.METHOD_2D:
+        raise ValueError("a 2-D model is a texture (read it with sample); a colour LUT needs a 3-D model (method 3 or 4)")
+    return method
+
+
+def bake_lut(fp, decoder, mip_level=0, size=None, precision=None, method=None, level_table=None):
+    """Bakes a 3-D model into a `BakedLut`: one dense `decode` of the whole mip with float32 output (size and defaults as
+    `decode`; a 65^3 LUT passes size=65), packed as a float32 table when precision is "f32" (default
+    var2.DECODE_PRECISION) and as float16 for the tensor-core precisions."""
+    method = _lut_method(method)
+    pname = (precision or var2.DECODE_PRECISION).lower()
+    dense = decode(fp, decoder, mip_level, size, None, pname, torch.float32, None, method, level_table)
+    return BakedLut.from_table(dense, torch.float32 if L.PRECISIONS.get(pname) == L.PREC_F32 else torch.float16)
+
+
+def bake_lut_codes(codes, decoder, num_bits, mip_level=0, size=None, precision="f16", method=None, level_table=None):
+    """`bake_lut` straight from the saved model (`codes`: the uint8 list of fp_savable): one dense `decode_codes`."""
+    method = _lut_method(method)
+    dense = decode_codes(codes, decoder, num_bits, mip_level, size, None, precision, torch.float32, None, method, level_table)
+    return BakedLut.from_table(dense, torch.float32 if L.PRECISIONS.get(precision.lower()) == L.PREC_F32 else torch.float16)
+
+
 class DecodeSession:
     """A model that is decoded many times (regions, mips, repeated frames): the private tensor-core tables (16-bit
     channel-last shadow grids, per-node G1 rows, packed weight images) are built by the first `decode` and REUSED by the
