@@ -667,7 +667,15 @@ class HostDecodePipeline:
       caller stream : decode-from-codes in row bands (the tables are built by the first band and reused by the others);
       copy stream   : D2H of each 8-bit band while the next band decodes (the device frame is double-buffered too).
     With `wait=False` the H2D of frame i + 1 and the D2H of frame i overlap the decode of frame i (PCIe is full
-    duplex); call `finish()` before reading the last host buffer."""
+    duplex).  `decode_frame` never blocks the host on the device, with either `wait`, so the host buffers of a frame stay
+    in use after it returns:
+      * `codes` and `host_params` are read by the frame's upload, which may still be pending (it waits for the decode
+        of frame i - 2 to release its device buffer).  Overwrite them, e.g. with the next frame's model, only after
+        `self.uploaded.synchronize()` (the upload event of the latest frame) or a later host synchronisation of the
+        caller's stream.
+      * `host_out` is written by the frame's downloads.  Read it only after synchronising the caller's stream: with
+        `wait=True` that stream already waits for the downloads, with `wait=False` call `finish()` first.  A later frame
+        may write the same `host_out` at once (the downloads are ordered on one stream)."""
 
     def __init__(self, size, device, precision="f16", bands=4, bits=8):
         self.size, self.device, self.precision, self.bits = size, torch.device(device), precision, bits
@@ -679,6 +687,7 @@ class HostDecodePipeline:
         self.out = None
         self.d2h_done = [None, None]
         self.dec_done = [None, None]
+        self.uploaded = None
         self.frame = 0
         self._last = None
 
@@ -712,6 +721,7 @@ class HostDecodePipeline:
                     p.copy_(hp, non_blocking=True)
             uploaded = torch.cuda.Event()
             uploaded.record(self.up_stream)
+        self.uploaded = uploaded
         main.wait_event(uploaded)
         if self.d2h_done[k] is not None:
             main.wait_event(self.d2h_done[k])        # the frame that used this device buffer two frames ago has left
