@@ -374,45 +374,50 @@ int nic_mlp_backward(NicHandle* h, const NicMlp* m, const float* x, int64_t ldx,
   return cuda_fail(h, launch_mlp_backward_f32(h, md, gd, x, ldx, n, z1, z2, out, dout, dx, st), "nic_mlp_backward");
 }
 
-int nic_decode(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const int64_t* origins,
-               const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+// Each decode / sampling entry point and its *_codes twin share one body.  `codes` says which of the two was called: the
+// grids are float32 (bits is 0) or uint8 codes of width bits.  It is a flag of its own because a codes call with bits 0
+// must be refused, not read as floats.
+// check_call: the checks a call makes once its geometry and MLP are flattened, in this order: the code width of a codes
+// call (1..8), the NULL pointers, out_dtype, the precision.  Codes are read by the tensor-core kernels only.
+static int check_call(NicHandle* h, bool codes, int bits, bool null_ptr, const char* null_msg, int out_dtype, int precision,
+                      const char* who) {
+  if (codes && (bits < 1 || bits > 8)) return fail(h, NIC_ERR_ARG, "%s: bits %d (1..8)", who, bits);
+  if (null_ptr) return fail(h, NIC_ERR_ARG, "%s: %s", who, null_msg);
+  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "%s: out_dtype %d", who, out_dtype);
+  if (codes && precision != NIC_PREC_F16 && precision != NIC_PREC_BF16)
+    return fail(h, NIC_ERR_UNSUPPORTED, "%s: tensor-core precisions only (f16 / bf16); unpack the codes for NIC_PREC_F32", who);
+  if (precision != NIC_PREC_F32 && precision != NIC_PREC_F16 && precision != NIC_PREC_BF16)
+    return fail(h, NIC_ERR_ARG, "%s: precision %d", who, precision);
+  return NIC_OK;
+}
+
+static int decode_impl(NicHandle* h, const NicGeom* g, const void* g0, const void* g1, bool codes, int bits,
+                       const int64_t* origins, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
   NIC_ENTER(h);
+  const char* who = codes ? "nic_decode_codes" : "nic_decode";
   DevGeom d;
   int rc = flatten_geom(h, g, origins != nullptr, &d);
   if (rc) return rc;
   MlpDev md;
   rc = flatten_mlp(h, m, &md, d.cin);
   if (rc) return rc;
-  if (!g0 || !g1 || (!out && d.N > 0)) return fail(h, NIC_ERR_ARG, "nic_decode: NULL pointer");
-  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_decode: out_dtype %d", out_dtype);
+  rc = check_call(h, codes, bits, !g0 || !g1 || (!out && d.N > 0), "NULL pointer", out_dtype, precision, who);
+  if (rc) return rc;
   if (precision == NIC_PREC_F32)
-    return cuda_fail(h, launch_mlp_forward_f32(h, &d, md, g0, g1, (const long long*)origins, nullptr, 0, d.N, out, out_dtype,
-                                               nullptr, nullptr, st), "nic_decode(f32)");
-  if (precision == NIC_PREC_F16 || precision == NIC_PREC_BF16)
-    return cuda_fail(h, launch_decode_tc(h, d, md, g0, g1, (const long long*)origins, out, out_dtype, precision, st),
-                     "nic_decode(tensor core)");
-  return fail(h, NIC_ERR_ARG, "nic_decode: precision %d", precision);
+    return cuda_fail(h, launch_mlp_forward_f32(h, &d, md, (const float*)g0, (const float*)g1, (const long long*)origins, nullptr,
+                                               0, d.N, out, out_dtype, nullptr, nullptr, st), "nic_decode(f32)");
+  return cuda_fail(h, launch_decode_tc(h, d, md, g0, g1, bits, (const long long*)origins, out, out_dtype, precision, st),
+                   codes ? who : "nic_decode(tensor core)");
+}
+
+int nic_decode(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const int64_t* origins,
+               const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+  return decode_impl(h, g, g0, g1, false, 0, origins, m, out, out_dtype, precision, stream);
 }
 
 int nic_decode_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, const uint8_t* codes1, int bits,
                      const int64_t* origins, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
-  NIC_ENTER(h);
-  DevGeom d;
-  int rc = flatten_geom(h, g, origins != nullptr, &d);
-  if (rc) return rc;
-  MlpDev md;
-  rc = flatten_mlp(h, m, &md, d.cin);
-  if (rc) return rc;
-  if (bits < 1 || bits > 8) return fail(h, NIC_ERR_ARG, "nic_decode_codes: bits %d (1..8)", bits);
-  if (!codes0 || !codes1 || (!out && d.N > 0)) return fail(h, NIC_ERR_ARG, "nic_decode_codes: NULL pointer");
-  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_decode_codes: out_dtype %d", out_dtype);
-  if (precision != NIC_PREC_F16 && precision != NIC_PREC_BF16)
-    return fail(h, NIC_ERR_UNSUPPORTED, "nic_decode_codes: tensor-core precisions only (f16 / bf16); unpack the codes for NIC_PREC_F32");
-  h->src_code_bits = bits;
-  rc = launch_decode_tc(h, d, md, reinterpret_cast<const float*>(codes0), reinterpret_cast<const float*>(codes1),
-                        (const long long*)origins, out, out_dtype, precision, st);
-  h->src_code_bits = 0;
-  return cuda_fail(h, rc, "nic_decode_codes");
+  return decode_impl(h, g, codes0, codes1, true, bits, origins, m, out, out_dtype, precision, stream);
 }
 
 // Geometry of a sampling call: the mip is validated like a host-known block (origin 0, block = extent), then described as
@@ -450,46 +455,36 @@ static int flatten_sampler(NicHandle* h, const NicGeom* g, const NicSampler* s, 
   return NIC_OK;
 }
 
-int nic_sample(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const float* coords,
-               const NicSampler* s, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+static int sample_impl(NicHandle* h, const NicGeom* g, const void* g0, const void* g1, bool codes, int bits,
+                       const float* coords, const NicSampler* s, const NicMlp* m, void* out, int out_dtype, int precision,
+                       void* stream) {
   NIC_ENTER(h);
+  const char* who = codes ? "nic_sample_codes" : "nic_sample";
   DevGeom d;
   DevSampler ds;
-  int rc = flatten_sampler(h, g, s, coords, &d, &ds, "nic_sample");
+  int rc = flatten_sampler(h, g, s, coords, &d, &ds, who);
   if (rc) return rc;
   MlpDev md;
   rc = flatten_mlp(h, m, &md, d.cin);
   if (rc) return rc;
-  if (!g0 || !g1 || (!out && d.N > 0)) return fail(h, NIC_ERR_ARG, "nic_sample: NULL pointer");
-  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_sample: out_dtype %d", out_dtype);
+  rc = check_call(h, codes, bits, !g0 || !g1 || (!out && d.N > 0), "NULL pointer", out_dtype, precision, who);
+  if (rc) return rc;
   if (precision == NIC_PREC_F32)
-    return cuda_fail(h, launch_sample_f32(h, d, ds, md, g0, g1, out, out_dtype, st), "nic_sample(f32)");
-  if (precision == NIC_PREC_F16 || precision == NIC_PREC_BF16)
-    return cuda_fail(h, launch_sample_tc(h, d, ds, md, g0, g1, out, out_dtype, precision, st), "nic_sample(tensor core)");
-  return fail(h, NIC_ERR_ARG, "nic_sample: precision %d", precision);
+    return cuda_fail(h, launch_sample_f32(h, d, ds, md, (const float*)g0, (const float*)g1, out, out_dtype, st),
+                     "nic_sample(f32)");
+  return cuda_fail(h, launch_sample_tc(h, d, ds, md, g0, g1, bits, out, out_dtype, precision, st),
+                   codes ? who : "nic_sample(tensor core)");
+}
+
+int nic_sample(NicHandle* h, const NicGeom* g, const float* g0, const float* g1, const float* coords,
+               const NicSampler* s, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+  return sample_impl(h, g, g0, g1, false, 0, coords, s, m, out, out_dtype, precision, stream);
 }
 
 int nic_sample_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, const uint8_t* codes1, int bits,
                      const float* coords, const NicSampler* s, const NicMlp* m, void* out, int out_dtype,
                      int precision, void* stream) {
-  NIC_ENTER(h);
-  DevGeom d;
-  DevSampler ds;
-  int rc = flatten_sampler(h, g, s, coords, &d, &ds, "nic_sample_codes");
-  if (rc) return rc;
-  MlpDev md;
-  rc = flatten_mlp(h, m, &md, d.cin);
-  if (rc) return rc;
-  if (bits < 1 || bits > 8) return fail(h, NIC_ERR_ARG, "nic_sample_codes: bits %d (1..8)", bits);
-  if (!codes0 || !codes1 || (!out && d.N > 0)) return fail(h, NIC_ERR_ARG, "nic_sample_codes: NULL pointer");
-  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_sample_codes: out_dtype %d", out_dtype);
-  if (precision != NIC_PREC_F16 && precision != NIC_PREC_BF16)
-    return fail(h, NIC_ERR_UNSUPPORTED, "nic_sample_codes: tensor-core precisions only (f16 / bf16); unpack the codes for NIC_PREC_F32");
-  h->src_code_bits = bits;
-  rc = launch_sample_tc(h, d, ds, md, reinterpret_cast<const float*>(codes0), reinterpret_cast<const float*>(codes1), out,
-                        out_dtype, precision, st);
-  h->src_code_bits = 0;
-  return cuda_fail(h, rc, "nic_sample_codes");
+  return sample_impl(h, g, codes0, codes1, true, bits, coords, s, m, out, out_dtype, precision, stream);
 }
 
 // Geometry of a per-query-LOD call: every mip validated as flatten_sampler validates one, the chain's shared description,
@@ -536,51 +531,38 @@ static int flatten_chain(NicHandle* h, const NicMipChain* c, const float* coords
   return NIC_OK;
 }
 
-int nic_sample_lod(NicHandle* h, const NicMipChain* c, const float* coords, const float* lod, const float* ddx,
-                   const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+static int sample_lod_impl(NicHandle* h, const NicMipChain* c, bool codes, int bits, const float* coords, const float* lod,
+                           const float* ddx, const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision,
+                           void* stream) {
   NIC_ENTER(h);
+  const char* who = codes ? "nic_sample_lod_codes" : "nic_sample_lod";
   DevGeom d[NIC_MAX_MIPS];
   DevChain dc;
   DevSampler ds;
-  int rc = flatten_chain(h, c, coords, lod, ddx, ddy, d, &dc, &ds, "nic_sample_lod");
+  int rc = flatten_chain(h, c, coords, lod, ddx, ddy, d, &dc, &ds, who);
   if (rc) return rc;
   MlpDev md;
   rc = flatten_mlp(h, m, &md, d[0].cin);
   if (rc) return rc;
-  if (!out && d[0].N > 0) return fail(h, NIC_ERR_ARG, "nic_sample_lod: out is NULL");
-  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_sample_lod: out_dtype %d", out_dtype);
-  const float* const* g0 = reinterpret_cast<const float* const*>(c->g0);
-  const float* const* g1 = reinterpret_cast<const float* const*>(c->g1);
+  rc = check_call(h, codes, bits, !out && d[0].N > 0, "out is NULL", out_dtype, precision, who);
+  if (rc) return rc;
   if (precision == NIC_PREC_F32)
-    return cuda_fail(h, launch_sample_lod_f32(h, d, dc, ds, md, g0, g1, out, out_dtype, st), "nic_sample_lod(f32)");
-  if (precision == NIC_PREC_F16 || precision == NIC_PREC_BF16)
-    return cuda_fail(h, launch_sample_lod_tc(h, d, dc, ds, md, g0, g1, out, out_dtype, precision, st),
-                     "nic_sample_lod(tensor core)");
-  return fail(h, NIC_ERR_ARG, "nic_sample_lod: precision %d", precision);
+    return cuda_fail(h, launch_sample_lod_f32(h, d, dc, ds, md, reinterpret_cast<const float* const*>(c->g0),
+                                              reinterpret_cast<const float* const*>(c->g1), out, out_dtype, st),
+                     "nic_sample_lod(f32)");
+  return cuda_fail(h, launch_sample_lod_tc(h, d, dc, ds, md, c->g0, c->g1, bits, out, out_dtype, precision, st),
+                   codes ? who : "nic_sample_lod(tensor core)");
+}
+
+int nic_sample_lod(NicHandle* h, const NicMipChain* c, const float* coords, const float* lod, const float* ddx,
+                   const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+  return sample_lod_impl(h, c, false, 0, coords, lod, ddx, ddy, m, out, out_dtype, precision, stream);
 }
 
 int nic_sample_lod_codes(NicHandle* h, const NicMipChain* c, int bits, const float* coords, const float* lod,
                          const float* ddx, const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision,
                          void* stream) {
-  NIC_ENTER(h);
-  DevGeom d[NIC_MAX_MIPS];
-  DevChain dc;
-  DevSampler ds;
-  int rc = flatten_chain(h, c, coords, lod, ddx, ddy, d, &dc, &ds, "nic_sample_lod_codes");
-  if (rc) return rc;
-  MlpDev md;
-  rc = flatten_mlp(h, m, &md, d[0].cin);
-  if (rc) return rc;
-  if (bits < 1 || bits > 8) return fail(h, NIC_ERR_ARG, "nic_sample_lod_codes: bits %d (1..8)", bits);
-  if (!out && d[0].N > 0) return fail(h, NIC_ERR_ARG, "nic_sample_lod_codes: out is NULL");
-  if (out_dtype != NIC_DT_F32 && out_dtype != NIC_DT_U8) return fail(h, NIC_ERR_ARG, "nic_sample_lod_codes: out_dtype %d", out_dtype);
-  if (precision != NIC_PREC_F16 && precision != NIC_PREC_BF16)
-    return fail(h, NIC_ERR_UNSUPPORTED, "nic_sample_lod_codes: tensor-core precisions only (f16 / bf16); unpack the codes for NIC_PREC_F32");
-  h->src_code_bits = bits;
-  rc = launch_sample_lod_tc(h, d, dc, ds, md, reinterpret_cast<const float* const*>(c->g0),
-                            reinterpret_cast<const float* const*>(c->g1), out, out_dtype, precision, st);
-  h->src_code_bits = 0;
-  return cuda_fail(h, rc, "nic_sample_lod_codes");
+  return sample_lod_impl(h, c, true, bits, coords, lod, ddx, ddy, m, out, out_dtype, precision, stream);
 }
 
 // Texels of a LUT extent: NIC_ERR_ARG for an extent < 1, NIC_ERR_UNSUPPORTED from 2^31 texels on (int texel indices).

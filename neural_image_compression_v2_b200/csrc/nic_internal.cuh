@@ -38,7 +38,6 @@ struct Handle {
   void* tc_partials;         // per-CTA MLP-gradient partial sums of the tensor-core training step
   size_t tc_partials_bytes;
   int disable_fast2d;        // testing knob: force the general tensor-core kernel
-  int src_code_bits;         // > 0 while a nic_decode_codes call is in flight: grid pointers are uint8 codes of that width
   int reuse_prepared;        // NIC_OPT_REUSE_PREPARED
   int debug_flags;           // knock-out experiments (option 100), never set in production
   unsigned long long* dbg_counters;   // 16 device counters (nic_debug_counters), allocated on first use
@@ -244,17 +243,18 @@ int launch_train_f32(Handle* h, const DevGeom& g, const MlpDev& m, const MlpGrad
                      const float* g1, const long long* origins, const float* targets, const float* noise,
                      int noise_bits, unsigned long long seed, unsigned long long step, float grad_scale, float* dg0,
                      float* dg1, float* loss_sum, float* out_save, cudaStream_t st);
-int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1,
+// The tensor-core launchers read the grids as float32 (code_bits = 0) or as uint8 codes of width code_bits (1..8).
+int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
                      const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st);
 // nic_sample / nic_sample_codes: g describes the mip with nblocks = queries (one texel each); smp the filter.
-int launch_sample_tc(Handle* h, const DevGeom& g, const DevSampler& smp, const MlpDev& m, const float* g0, const float* g1,
-                     void* out, int out_dtype, int precision, cudaStream_t st);
+int launch_sample_tc(Handle* h, const DevGeom& g, const DevSampler& smp, const MlpDev& m, const void* g0, const void* g1,
+                     int code_bits, void* out, int out_dtype, int precision, cudaStream_t st);
 int launch_sample_f32(Handle* h, const DevGeom& g, const DevSampler& smp, const MlpDev& m, const float* g0, const float* g1,
                       void* out, int out_dtype, cudaStream_t st);
 // nic_sample_lod / nic_sample_lod_codes: g[i] describes mip i of the chain as launch_sample_* take it; c the chain.
 int launch_sample_lod_tc(Handle* h, const DevGeom* g, const DevChain& c, const DevSampler& smp, const MlpDev& m,
-                         const float* const* g0, const float* const* g1, void* out, int out_dtype, int precision,
-                         cudaStream_t st);
+                         const void* const* g0, const void* const* g1, int code_bits, void* out, int out_dtype,
+                         int precision, cudaStream_t st);
 int launch_sample_lod_f32(Handle* h, const DevGeom* g, const DevChain& c, const DevSampler& smp, const MlpDev& m,
                           const float* const* g0, const float* const* g1, void* out, int out_dtype, cudaStream_t st);
 // nic_lut_pack / nic_lut_apply (nic_lut.cu): arguments validated by nic_api.cu.

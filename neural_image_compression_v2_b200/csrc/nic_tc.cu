@@ -1170,8 +1170,8 @@ __global__ void __launch_bounds__(CQ_NG * GW_GROUP, 1)
 
 // ------------------------------------------------------------------------------------------------ launcher
 // NIC_OPT_REUSE_PREPARED: do the private tables already describe these inputs?
-static Handle::PreparedKey make_key(const DevGeom& g, const MlpDev& m, const float* g0, const float* g1, int fmt, int fast,
-                                    int code_bits = 0, int npoly = 0) {
+static Handle::PreparedKey make_key(const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int fmt, int fast,
+                                    int code_bits, int npoly) {
   Handle::PreparedKey k;
   memset(&k, 0, sizeof(k));
   k.g0 = g0; k.g1 = g1; k.w1 = m.w1; k.b1 = m.b1; k.w2 = m.w2; k.b2 = m.b2; k.w3 = m.w3; k.b3 = m.b3;
@@ -1195,18 +1195,17 @@ static bool fast2d_eligible(const DevGeom& g, const long long* origins) {
 // Random-access queries (1-texel blocks) on a model given as uint8 codes whose two grids fit shared memory next to three
 // operand buffers: the code-resident kernel.  Returns -1000 when the call does not qualify (the caller falls through).
 template <int METHOD, typename OutT>
-static int launch_codes_smem(Handle* h, const DevGeom& g, const MlpDev& m, const uint8_t* c0, const uint8_t* c1,
+static int launch_codes_smem(Handle* h, const DevGeom& g, const MlpDev& m, const void* c0, const void* c1, int bits,
                              const long long* origins, OutT* out, cudaStream_t st) {
   using S = RowShape<METHOD>;
   const long long nodes0 = plane_size_host(g.n0, g.dim), nodes1 = plane_size_host(g.n1, g.dim);
   const long long bytes0 = (nodes0 * 12 + 15) & ~15ll, bytes1 = (nodes1 * 12 + 15) & ~15ll;
   const long long smem = cq_fixed_smem<METHOD>() + bytes0 + bytes1;
-  const int bits = h->src_code_bits;
   if (!origins || g.per_block != 1 || bits < 1 || bits > 8 || smem > 227 * 1024 || h->disable_fast2d) return -1000;
   int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
   if (rc) return rc;
   const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : WS_NPOLY_F16;
-  const Handle::PreparedKey key = make_key(g, m, (const float*)c0, (const float*)c1, 0, 2, bits, npoly);
+  const Handle::PreparedKey key = make_key(g, m, c0, c1, 0, 2, bits, npoly);
   if (!prepared_matches(h, key)) {
     h->prepared.valid = 0;
     pack_weights_kernel<0><<<16, 256, 0, st>>>(m, g.lod, S::KX, (uint16_t*)h->tc_weights, npoly, 12 * (S::NC0 + 1),
@@ -1235,16 +1234,16 @@ static int launch_codes_smem(Handle* h, const DevGeom& g, const MlpDev& m, const
   const int grid = (int)(groups < h->sms ? groups : h->sms);
   {
     KernelTimer timer(h, st);
-    kern<<<grid, CQ_NG * GW_GROUP, (size_t)smem, st>>>(g, c0, c1, (1 << (bits - 1)) - 1, (int)bytes0, origins,
-                                                        (const uint4*)h->tc_weights, m.cout, lut_n, out);
+    kern<<<grid, CQ_NG * GW_GROUP, (size_t)smem, st>>>(g, (const uint8_t*)c0, (const uint8_t*)c1, (1 << (bits - 1)) - 1,
+                                                        (int)bytes0, origins, (const uint4*)h->tc_weights, m.cout, lut_n, out);
   }
   h->launches++;
   return (int)cudaGetLastError();
 }
 
 template <int FMT, typename OutT>
-static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1, OutT* out,
-                         cudaStream_t st) {
+static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
+                         OutT* out, cudaStream_t st) {
   int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
   if (rc) return rc;
   const long long nodes0 = plane_size_host(g.n0, 2), nodes1 = plane_size_host(g.n1, 2);
@@ -1257,14 +1256,15 @@ static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const flo
   // how many of every 8 activation pairs take the polynomial (FMA-pipe) GELU instead of MUFU.TANH: tuned per format so
   // that the XU and FMA pipes finish together (profiles/r02*); NIC_OPT_GELU_POLY overrides it for A/B runs
   const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : (FMT == 0 ? WS_NPOLY_F16 : WS_NPOLY_BF16);
-  const Handle::PreparedKey key = make_key(g, m, g0, g1, FMT, 1, h->src_code_bits, npoly);
+  const Handle::PreparedKey key = make_key(g, m, g0, g1, FMT, 1, code_bits, npoly);
   if (!prepared_matches(h, key)) {
     h->prepared.valid = 0;
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, g.n0, s0, st);
+    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, code_bits, g.n0, s0, st);
     if (e != cudaSuccess) return (int)e;
     const long long tiles_r = (long long)((g.n1[0] + G1R_TX - 1) / G1R_TX) * ((g.n1[1] + G1R_TY - 1) / G1R_TY);
     const long long cap_r = 2ll * h->sms;
-    g1_rows_kernel<FMT><<<(int)(tiles_r < cap_r ? tiles_r : cap_r), 256, 0, st>>>(m, g1, g.n1[0], g.n1[1], R, h->src_code_bits);
+    g1_rows_kernel<FMT><<<(int)(tiles_r < cap_r ? tiles_r : cap_r), 256, 0, st>>>(m, (const float*)g1, g.n1[0], g.n1[1], R,
+                                                                                 code_bits);
     h->launches++;
     pack_fast_kernel<FMT><<<32, 256, 0, st>>>(m, g.lod, g.step, (uint16_t*)h->tc_weights, npoly);
     h->launches++;
@@ -1310,16 +1310,15 @@ static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const flo
 // TAPS > 0: filtered sampling (smp set, g.N = queries * TAPS rows) always runs on the general kernel: the fast 2-D kernel
 // and the code-resident kernel have no per-row texel and no tap epilogue.
 template <int METHOD, int FMT, typename OutT, int TAPS = 0>
-static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1,
+static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
                        const long long* origins, OutT* out, cudaStream_t st, const DevSampler* smp = nullptr) {
   using S = RowShape<METHOD>;
   if constexpr (METHOD == NIC_METHOD_2D && TAPS == 0) {
-    if (fast2d_eligible(g, origins) && !h->disable_fast2d) return launch_fast2d<FMT, OutT>(h, g, m, g0, g1, out, st);
+    if (fast2d_eligible(g, origins) && !h->disable_fast2d) return launch_fast2d<FMT, OutT>(h, g, m, g0, g1, code_bits, out, st);
   }
   if constexpr (METHOD == NIC_METHOD_3D && FMT == 0 && TAPS == 0) {       // small models given as codes, random-access queries
-    if (h->src_code_bits > 0) {
-      const int crc = launch_codes_smem<METHOD, OutT>(h, g, m, reinterpret_cast<const uint8_t*>(g0),
-                                                      reinterpret_cast<const uint8_t*>(g1), origins, out, st);
+    if (code_bits > 0) {
+      const int crc = launch_codes_smem<METHOD, OutT>(h, g, m, g0, g1, code_bits, origins, out, st);
       if (crc != -1000) return crc;
     }
   }
@@ -1335,12 +1334,12 @@ static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const float
   uint16_t* s1 = (uint16_t*)((uint8_t*)h->tc_shadow + b0);
   cudaError_t e = cudaSuccess;
   const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : (FMT == 0 ? WS_NPOLY_F16 : WS_NPOLY_BF16);
-  const Handle::PreparedKey key = make_key(g, m, g0, g1, FMT, 0, h->src_code_bits, npoly);
+  const Handle::PreparedKey key = make_key(g, m, g0, g1, FMT, 0, code_bits, npoly);
   if (!prepared_matches(h, key)) {
     h->prepared.valid = 0;
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, g.n0, s0, st);
+    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, code_bits, g.n0, s0, st);
     if (e != cudaSuccess) return (int)e;
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g1, g.n1, s1, st);
+    e = (cudaError_t)launch_relayout<FMT>(h, g, g1, code_bits, g.n1, s1, st);
     if (e != cudaSuccess) return (int)e;
     pack_weights_kernel<FMT><<<16, 256, 0, st>>>(m, g.lod, S::KX, (uint16_t*)h->tc_weights, npoly);
     h->launches++;
@@ -1390,40 +1389,40 @@ static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const float
 }
 
 template <int METHOD, int TAPS = 0>
-static int launch_tc_m(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1,
+static int launch_tc_m(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
                        const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st,
                        const DevSampler* smp = nullptr) {
   if (precision == NIC_PREC_F16) {
-    if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 0, uint8_t, TAPS>(h, g, m, g0, g1, origins, (uint8_t*)out, st, smp);
-    return launch_tc_t<METHOD, 0, float, TAPS>(h, g, m, g0, g1, origins, (float*)out, st, smp);
+    if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 0, uint8_t, TAPS>(h, g, m, g0, g1, code_bits, origins, (uint8_t*)out, st, smp);
+    return launch_tc_t<METHOD, 0, float, TAPS>(h, g, m, g0, g1, code_bits, origins, (float*)out, st, smp);
   }
-  if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 1, uint8_t, TAPS>(h, g, m, g0, g1, origins, (uint8_t*)out, st, smp);
-  return launch_tc_t<METHOD, 1, float, TAPS>(h, g, m, g0, g1, origins, (float*)out, st, smp);
+  if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 1, uint8_t, TAPS>(h, g, m, g0, g1, code_bits, origins, (uint8_t*)out, st, smp);
+  return launch_tc_t<METHOD, 1, float, TAPS>(h, g, m, g0, g1, code_bits, origins, (float*)out, st, smp);
 }
 
-int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const float* g0, const float* g1,
+int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
                      const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st) {
   if (g.N == 0) return NIC_OK;
   if (g.C != 12 || g.PE != 6 || m.hidden != 64 || m.cout > 16) return NIC_ERR_UNSUPPORTED;
   switch (g.method) {
-    case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D>(h, g, m, g0, g1, origins, out, out_dtype, precision, st);
-    case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D>(h, g, m, g0, g1, origins, out, out_dtype, precision, st);
-    case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2>(h, g, m, g0, g1, origins, out, out_dtype, precision, st);
+    case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D>(h, g, m, g0, g1, code_bits, origins, out, out_dtype, precision, st);
+    case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D>(h, g, m, g0, g1, code_bits, origins, out, out_dtype, precision, st);
+    case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2>(h, g, m, g0, g1, code_bits, origins, out, out_dtype, precision, st);
   }
   return NIC_ERR_UNSUPPORTED;
 }
 
-int launch_sample_tc(Handle* h, const DevGeom& gq, const DevSampler& smp, const MlpDev& m, const float* g0, const float* g1,
-                     void* out, int out_dtype, int precision, cudaStream_t st) {
+int launch_sample_tc(Handle* h, const DevGeom& gq, const DevSampler& smp, const MlpDev& m, const void* g0, const void* g1,
+                     int code_bits, void* out, int out_dtype, int precision, cudaStream_t st) {
   if (gq.nblocks == 0) return NIC_OK;
   if (gq.C != 12 || gq.PE != 6 || m.hidden != 64 || m.cout > 16) return NIC_ERR_UNSUPPORTED;
   DevGeom g = gq;                                   // one row per tap: queries x 2^dim rows
   g.N = (long long)gq.nblocks << gq.dim;
   if (g.N >= (1ll << 31) - TC_ROWS) return NIC_ERR_UNSUPPORTED;     // 32-bit row index in the kernel
   switch (g.method) {
-    case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D, 4>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
-    case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D, 8>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
-    case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2, 8>(h, g, m, g0, g1, nullptr, out, out_dtype, precision, st, &smp);
+    case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D, 4>(h, g, m, g0, g1, code_bits, nullptr, out, out_dtype, precision, st, &smp);
+    case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D, 8>(h, g, m, g0, g1, code_bits, nullptr, out, out_dtype, precision, st, &smp);
+    case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2, 8>(h, g, m, g0, g1, code_bits, nullptr, out, out_dtype, precision, st, &smp);
   }
   return NIC_ERR_UNSUPPORTED;
 }
@@ -1432,7 +1431,7 @@ int launch_sample_tc(Handle* h, const DevGeom& gq, const DevSampler& smp, const 
 // W1 image with the mip column, the chain table in device memory, one pass of the general kernel with 2 * 2^D rows a query.
 template <int METHOD, int FMT, typename OutT>
 static int launch_lod_t(Handle* h, const DevGeom* gm, DevChain c, const DevSampler& smp, const MlpDev& m,
-                        const float* const* g0, const float* const* g1, OutT* out, cudaStream_t st) {
+                        const void* const* g0, const void* const* g1, int code_bits, OutT* out, cudaStream_t st) {
   using S = RowShape<METHOD>;
   constexpr int TAPS = 2 << S::DIM;
   int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
@@ -1467,7 +1466,7 @@ static int launch_lod_t(Handle* h, const DevGeom* gm, DevChain c, const DevSampl
   cudaError_t e = cudaSuccess;
   const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : (FMT == 0 ? WS_NPOLY_F16 : WS_NPOLY_BF16);
   if (npoly != 0 && npoly != 3) return NIC_ERR_UNSUPPORTED;
-  Handle::PreparedKey key = make_key(gm[0], m, g0[0], g1[0], FMT, 3, h->src_code_bits, npoly);
+  Handle::PreparedKey key = make_key(gm[0], m, g0[0], g1[0], FMT, 3, code_bits, npoly);
   key.chain_mips = c.num_mips;
   for (int i = 0; i < c.num_mips; ++i) {
     key.chain_g[2 * i] = g0[i];
@@ -1479,9 +1478,9 @@ static int launch_lod_t(Handle* h, const DevGeom* gm, DevChain c, const DevSampl
     h->prepared.valid = 0;
     for (int i = 0; i < c.num_mips; ++i) {
       if (first[i] != i) continue;
-      e = (cudaError_t)launch_relayout<FMT>(h, gm[i], g0[i], gm[i].n0, (uint16_t*)(shadow + off[i][0]), st);
+      e = (cudaError_t)launch_relayout<FMT>(h, gm[i], g0[i], code_bits, gm[i].n0, (uint16_t*)(shadow + off[i][0]), st);
       if (e != cudaSuccess) return (int)e;
-      e = (cudaError_t)launch_relayout<FMT>(h, gm[i], g1[i], gm[i].n1, (uint16_t*)(shadow + off[i][1]), st);
+      e = (cudaError_t)launch_relayout<FMT>(h, gm[i], g1[i], code_bits, gm[i].n1, (uint16_t*)(shadow + off[i][1]), st);
       if (e != cudaSuccess) return (int)e;
     }
     pack_weights_kernel<FMT><<<16, 256, 0, st>>>(m, 0.0f, S::KX, (uint16_t*)h->tc_weights, npoly);
@@ -1524,27 +1523,27 @@ static int launch_lod_t(Handle* h, const DevGeom* gm, DevChain c, const DevSampl
 
 template <int METHOD>
 static int launch_lod_m(Handle* h, const DevGeom* gm, const DevChain& c, const DevSampler& smp, const MlpDev& m,
-                        const float* const* g0, const float* const* g1, void* out, int out_dtype, int precision,
-                        cudaStream_t st) {
+                        const void* const* g0, const void* const* g1, int code_bits, void* out, int out_dtype,
+                        int precision, cudaStream_t st) {
   if (precision == NIC_PREC_F16) {
-    if (out_dtype == NIC_DT_U8) return launch_lod_t<METHOD, 0, uint8_t>(h, gm, c, smp, m, g0, g1, (uint8_t*)out, st);
-    return launch_lod_t<METHOD, 0, float>(h, gm, c, smp, m, g0, g1, (float*)out, st);
+    if (out_dtype == NIC_DT_U8) return launch_lod_t<METHOD, 0, uint8_t>(h, gm, c, smp, m, g0, g1, code_bits, (uint8_t*)out, st);
+    return launch_lod_t<METHOD, 0, float>(h, gm, c, smp, m, g0, g1, code_bits, (float*)out, st);
   }
-  if (out_dtype == NIC_DT_U8) return launch_lod_t<METHOD, 1, uint8_t>(h, gm, c, smp, m, g0, g1, (uint8_t*)out, st);
-  return launch_lod_t<METHOD, 1, float>(h, gm, c, smp, m, g0, g1, (float*)out, st);
+  if (out_dtype == NIC_DT_U8) return launch_lod_t<METHOD, 1, uint8_t>(h, gm, c, smp, m, g0, g1, code_bits, (uint8_t*)out, st);
+  return launch_lod_t<METHOD, 1, float>(h, gm, c, smp, m, g0, g1, code_bits, (float*)out, st);
 }
 
 int launch_sample_lod_tc(Handle* h, const DevGeom* gm, const DevChain& c, const DevSampler& smp, const MlpDev& m,
-                         const float* const* g0, const float* const* g1, void* out, int out_dtype, int precision,
-                         cudaStream_t st) {
+                         const void* const* g0, const void* const* g1, int code_bits, void* out, int out_dtype,
+                         int precision, cudaStream_t st) {
   if (gm[0].nblocks == 0) return NIC_OK;
   if (gm[0].C != 12 || gm[0].PE != 6 || m.hidden != 64 || m.cout > 16) return NIC_ERR_UNSUPPORTED;
   for (int i = 0; i < c.num_mips; ++i)               // one 64-entry LUT at step 1/4 serves the triangular PE of every mip
     if (gm[0].pe_kind == NIC_PE_TRIANGULAR && gm[i].step < 0.25f) return NIC_ERR_UNSUPPORTED;
   switch (gm[0].method) {
-    case NIC_METHOD_2D: return launch_lod_m<NIC_METHOD_2D>(h, gm, c, smp, m, g0, g1, out, out_dtype, precision, st);
-    case NIC_METHOD_3D: return launch_lod_m<NIC_METHOD_3D>(h, gm, c, smp, m, g0, g1, out, out_dtype, precision, st);
-    case NIC_METHOD_3D_V2: return launch_lod_m<NIC_METHOD_3D_V2>(h, gm, c, smp, m, g0, g1, out, out_dtype, precision, st);
+    case NIC_METHOD_2D: return launch_lod_m<NIC_METHOD_2D>(h, gm, c, smp, m, g0, g1, code_bits, out, out_dtype, precision, st);
+    case NIC_METHOD_3D: return launch_lod_m<NIC_METHOD_3D>(h, gm, c, smp, m, g0, g1, code_bits, out, out_dtype, precision, st);
+    case NIC_METHOD_3D_V2: return launch_lod_m<NIC_METHOD_3D_V2>(h, gm, c, smp, m, g0, g1, code_bits, out, out_dtype, precision, st);
   }
   return NIC_ERR_UNSUPPORTED;
 }

@@ -354,7 +354,8 @@ static inline int ensure_scratch(void** ptr, size_t* have, size_t need) {
 }
 
 template <int FMT>
-static inline int launch_relayout(Handle* h, const DevGeom& g, const float* src, const int* nodes, uint16_t* dst, cudaStream_t st) {
+static inline int launch_relayout(Handle* h, const DevGeom& g, const void* src, int code_bits, const int* nodes, uint16_t* dst,
+                                  cudaStream_t st) {
   const int dim = g.dim;
   const int nx = nodes[0], nf = dim == 2 ? nodes[1] : nodes[2], no = dim == 2 ? 1 : nodes[1];
   const long long sf = dim == 2 ? nx : (long long)nodes[1] * nx, so = dim == 2 ? 0 : nx;
@@ -368,9 +369,9 @@ static inline int launch_relayout(Handle* h, const DevGeom& g, const float* src,
       cudaError_t e = cudaFuncSetAttribute(relayout_kernel<FMT, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (e != cudaSuccess) return (int)e;
     }
-    relayout_kernel<FMT, 32><<<grid, 256, smem, st>>>(src, dst, g.C, nx, nf, no, sf, so, plane, h->src_code_bits);
+    relayout_kernel<FMT, 32><<<grid, 256, smem, st>>>((const float*)src, dst, g.C, nx, nf, no, sf, so, plane, code_bits);
   } else {
-    relayout_kernel<FMT, 8><<<grid, 256, smem, st>>>(src, dst, g.C, nx, nf, no, sf, so, plane, h->src_code_bits);
+    relayout_kernel<FMT, 8><<<grid, 256, smem, st>>>((const float*)src, dst, g.C, nx, nf, no, sf, so, plane, code_bits);
   }
   h->launches++;
   return (int)cudaGetLastError();

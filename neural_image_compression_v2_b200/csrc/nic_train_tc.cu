@@ -1430,9 +1430,9 @@ static int launch_train_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const
   sa.t1 = small ? nodes1 * g.C : 0;
   if (sa.t0 >= (1ll << 32) || sa.t1 >= (1ll << 32)) return NIC_ERR_UNSUPPORTED;        // 32-bit index math in the side kernels
   if (!small) {
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, g.n0, s0, st);
+    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, 0, g.n0, s0, st);
     if (e != cudaSuccess) return (int)e;
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g1, g.n1, s1, st);
+    e = (cudaError_t)launch_relayout<FMT>(h, g, g1, 0, g.n1, s1, st);
     if (e != cudaSuccess) return (int)e;
   }
   {

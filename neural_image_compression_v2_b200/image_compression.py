@@ -202,102 +202,95 @@ def finally_decode_input_3d_v2(fp, image_size, mip_level, x=0, y=0, z=0):
 
 
 # ------------------------------------------------------------------------------------------------ fused decode
+def _check_codes(codes):
+    for c in codes:
+        if not c.is_cuda or c.dtype != torch.uint8 or not c.is_contiguous():
+            raise TypeError("codes must be contiguous uint8 CUDA tensors")
+    return codes
+
+
+def _check_grids(grids, bits):
+    """The grids a call reads: float32 grids (bits None) or uint8 codes (the list fp_savable returns)."""
+    return [_check_grid(g.detach()) for g in grids] if bits is None else _check_codes(grids)
+
+
+def _launch(h, fn, fn_codes, bits, pname, head, tail, stream):
+    """fn(h, *head, *tail, precision, stream) on float32 grids (bits None), fn_codes(h, *head, bits, *tail, precision,
+    stream) on codes (the library checks bits); raises on failure.  "auto" (float32 grids only): the tensor-core kernels
+    where they exist (C = 12, PE = 6, hidden 64), else the reference-exact CUDA-core kernel."""
+    if bits is not None:
+        rc = fn_codes(h, *head, bits, *tail, L.PRECISIONS[pname], stream)
+    else:
+        for prec in (("f16", "f32") if pname == "auto" else (pname,)):
+            rc = fn(h, *head, *tail, L.PRECISIONS[prec], stream)
+            if not (rc == L.ERR_UNSUPPORTED and pname == "auto" and prec != "f32"):
+                break
+    L.check(h, rc)
+
+
+def _decode(fp_like, bits, decoder, mip_level, size, origin, coords, precision, out_dtype, out, method, level_table):
+    """Common body of decode / decode_points (bits None: float32 grids) and decode_codes / decode_points_codes (uint8 codes of
+    width bits).  coords None: one block of `size` texels at `origin`; else Q one-texel blocks at coords [Q, D]."""
+    method = _method() if method is None else method
+    dim = 2 if method == L.METHOD_2D else 3
+    table = feature_pyramid_mip_levels() if level_table is None else level_table
+    fl = table[mip_level]
+    g0, g1 = _check_grids((fp_like[fl * 2], fp_like[fl * 2 + 1]), bits)
+    if coords is None:
+        if size is None:
+            size = var2.IMAGE_SIZE // pow(2, mip_level)
+        block = (size,) * dim if isinstance(size, int) else tuple(size)
+        blocks, shape = 1, block
+    else:
+        coords = L.origins_tensor(coords, g0.device, dim)
+        blocks = coords.shape[0]
+        if blocks >= 2 ** 31 - 128:
+            raise ValueError("at most 2^31 - 129 queries per call; split the batch")
+        block, shape = 1, (blocks,)
+    params = [p.detach().contiguous() for p in decoder.parameters_list()]
+    m = L.make_mlp(params)
+    geom = L.make_geom(method, g0, g1, block, blocks, _step_log2(mip_level, fl), mip_level, var2.PE_CHANNELS, _pe_kind(method),
+                       origin0=origin)
+    if out_dtype not in (torch.float32, torch.uint8):
+        raise TypeError("out_dtype must be torch.float32 or torch.uint8")
+    shape += (m.cout,)
+    if out is None:
+        out = torch.empty(shape, dtype=out_dtype, device=g0.device)
+    elif tuple(out.shape) != shape or out.dtype != out_dtype or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous {out_dtype} tensor of shape {shape}")
+    lib = L.load_library()
+    _launch(L.handle(g0.device), lib.nic_decode, lib.nic_decode_codes, bits, (precision or var2.DECODE_PRECISION).lower(),
+            (C.byref(geom), L.ptr(g0), L.ptr(g1)),
+            (L.ptr(coords), C.byref(m), L.ptr(out), L.DT_U8 if out_dtype == torch.uint8 else L.DT_F32), L.stream_ptr(g0.device))
+    return out
+
+
 def decode(fp, decoder, mip_level=0, size=None, origin=None, precision=None, out_dtype=torch.float32, out=None,
            method=None, level_table=None):
     """Fused gather + MLP for one block: the body of decode_image's single-shot branch
     (image_compression.py:313-327) without materialising X.
 
     size: texels per axis (int) or per-axis tuple (x, y[, z]); default IMAGE_SIZE >> mip_level.
-    origin: block origin in texels of this mip level.  precision: "f32" | "f16" | "bf16" (default
+    origin: block origin in texels of this mip level.  precision: "f32" | "f16" | "bf16" | "auto" (default
     var2.DECODE_PRECISION).  out_dtype: torch.float32 or torch.uint8 (floor(v*255+.5)).
     Returns [Sx, Sy(, Sz), Cout]."""
-    method = _method() if method is None else method
-    dim = 2 if method == L.METHOD_2D else 3
-    table = feature_pyramid_mip_levels() if level_table is None else level_table
-    fl = table[mip_level]
-    g0, g1 = _check_grid(fp[fl * 2].detach()), _check_grid(fp[fl * 2 + 1].detach())
-    if size is None:
-        size = var2.IMAGE_SIZE // pow(2, mip_level)
-    block = (size,) * dim if isinstance(size, int) else tuple(size)
-    params = [p.detach().contiguous() for p in decoder.parameters_list()]
-    m = L.make_mlp(params)
-    geom = L.make_geom(method, g0, g1, block, 1, _step_log2(mip_level, fl), mip_level, var2.PE_CHANNELS,
-                       _pe_kind(method), origin0=origin)
-    pname = (precision or var2.DECODE_PRECISION).lower()
-    if out_dtype not in (torch.float32, torch.uint8):
-        raise TypeError("out_dtype must be torch.float32 or torch.uint8")
-    shape = block + (m.cout,)
-    if out is None:
-        out = torch.empty(shape, dtype=out_dtype, device=g0.device)
-    elif tuple(out.shape) != shape or out.dtype != out_dtype or not out.is_contiguous():
-        raise ValueError(f"out must be a contiguous {out_dtype} tensor of shape {shape}")
-    h = L.handle(g0.device)
-    # "auto": the tensor-core kernels where they exist (C = 12, PE = 6, hidden 64), else the reference-exact CUDA-core kernel
-    for prec in (("f16", "f32") if pname == "auto" else (pname,)):
-        rc = L.load_library().nic_decode(h, C.byref(geom), L.ptr(g0), L.ptr(g1), None, C.byref(m), L.ptr(out),
-                                         L.DT_U8 if out_dtype == torch.uint8 else L.DT_F32, L.PRECISIONS[prec],
-                                         L.stream_ptr(g0.device))
-        if not (rc == L.ERR_UNSUPPORTED and pname == "auto" and prec != "f32"):
-            break
-    L.check(h, rc)
-    return out
+    return _decode(fp, None, decoder, mip_level, size, origin, None, precision, out_dtype, out, method, level_table)
 
 
 def decode_codes(codes, decoder, num_bits, mip_level=0, size=None, origin=None, precision="f16", out_dtype=torch.uint8,
                  out=None, method=None, level_table=None):
     """`decode` straight from the saved model: `codes` is the list fp_savable / torch.load returns (uint8, one code per
     byte).  The de-quantisation of models.load4fp is fused into the grid read (no float32 grids are materialised)."""
-    method = _method() if method is None else method
-    dim = 2 if method == L.METHOD_2D else 3
-    table = feature_pyramid_mip_levels() if level_table is None else level_table
-    fl = table[mip_level]
-    c0, c1 = codes[fl * 2], codes[fl * 2 + 1]
-    for c in (c0, c1):
-        if not c.is_cuda or c.dtype != torch.uint8 or not c.is_contiguous():
-            raise TypeError("codes must be contiguous uint8 CUDA tensors")
-    if size is None:
-        size = var2.IMAGE_SIZE // pow(2, mip_level)
-    block = (size,) * dim if isinstance(size, int) else tuple(size)
-    params = [p.detach().contiguous() for p in decoder.parameters_list()]
-    m = L.make_mlp(params)
-    geom = L.make_geom(method, c0, c1, block, 1, _step_log2(mip_level, fl), mip_level, var2.PE_CHANNELS, _pe_kind(method),
-                       origin0=origin)
-    shape = block + (m.cout,)
-    if out is None:
-        out = torch.empty(shape, dtype=out_dtype, device=c0.device)
-    elif tuple(out.shape) != shape or out.dtype != out_dtype or not out.is_contiguous():
-        raise ValueError(f"out must be a contiguous {out_dtype} tensor of shape {shape}")
-    h = L.handle(c0.device)
-    L.check(h, L.load_library().nic_decode_codes(h, C.byref(geom), L.ptr(c0), L.ptr(c1), num_bits, None, C.byref(m), L.ptr(out),
-                                                 L.DT_U8 if out_dtype == torch.uint8 else L.DT_F32,
-                                                 L.PRECISIONS[precision.lower()], L.stream_ptr(c0.device)))
-    return out
+    return _decode(codes, num_bits, decoder, mip_level, size, origin, None, precision, out_dtype, out, method, level_table)
 
 
 def decode_points(fp, decoder, coords, mip_level=0, precision=None, out_dtype=torch.float32, method=None,
                   level_table=None):
     """Random-access decode: coords `[Q, D]` integer texel coordinates of mip `mip_level` -> `[Q, Cout]`.
     Each query is a 1-texel block whose origin is the query (the `coord` mechanism of create_decoder_input_*,
-    image_compression.py:71-167, with sample_number = 1); used for LUT look-ups (BASELINE config 4)."""
-    method = _method() if method is None else method
-    dim = 2 if method == L.METHOD_2D else 3
-    table = feature_pyramid_mip_levels() if level_table is None else level_table
-    fl = table[mip_level]
-    g0, g1 = _check_grid(fp[fl * 2].detach()), _check_grid(fp[fl * 2 + 1].detach())
-    coords = L.origins_tensor(coords, g0.device, dim)
-    params = [p.detach().contiguous() for p in decoder.parameters_list()]
-    m = L.make_mlp(params)
-    q = coords.shape[0]
-    if q >= 2 ** 31 - 128:
-        raise ValueError("at most 2^31 - 129 queries per call; split the batch")
-    geom = L.make_geom(method, g0, g1, 1, q, _step_log2(mip_level, fl), mip_level, var2.PE_CHANNELS, _pe_kind(method))
-    prec = L.PRECISIONS[(precision or var2.DECODE_PRECISION).lower()]
-    out = torch.empty((q, m.cout), dtype=out_dtype, device=g0.device)
-    h = L.handle(g0.device)
-    L.check(h, L.load_library().nic_decode(h, C.byref(geom), L.ptr(g0), L.ptr(g1), L.ptr(coords), C.byref(m), L.ptr(out),
-                                           L.DT_U8 if out_dtype == torch.uint8 else L.DT_F32, prec,
-                                           L.stream_ptr(g0.device)))
-    return out
+    image_compression.py:71-167, with sample_number = 1); used for LUT look-ups (BASELINE config 4).
+    precision: "f32" | "f16" | "bf16" | "auto" (default var2.DECODE_PRECISION), as for `decode`."""
+    return _decode(fp, None, decoder, mip_level, None, None, coords, precision, out_dtype, None, method, level_table)
 
 
 def decode_points_codes(codes, decoder, coords, num_bits, mip_level=0, precision="f16", out_dtype=torch.uint8, method=None,
@@ -307,27 +300,7 @@ def decode_points_codes(codes, decoder, coords, num_bits, mip_level=0, precision
     operand buffers (a 65^3 LUT: 18^3 + 10^3 nodes = 82 KB of codes) and the precision is f16, the queries run on the
     code-resident kernel (decode_codes_smem_kernel: corner reads are shared-memory loads, models.load4fp is folded into the
     first layer); otherwise on the general tensor-core kernel with the de-quantisation fused into the grid read."""
-    method = _method() if method is None else method
-    dim = 2 if method == L.METHOD_2D else 3
-    table = feature_pyramid_mip_levels() if level_table is None else level_table
-    fl = table[mip_level]
-    c0, c1 = codes[fl * 2], codes[fl * 2 + 1]
-    for c in (c0, c1):
-        if not c.is_cuda or c.dtype != torch.uint8 or not c.is_contiguous():
-            raise TypeError("codes must be contiguous uint8 CUDA tensors")
-    coords = L.origins_tensor(coords, c0.device, dim)
-    params = [p.detach().contiguous() for p in decoder.parameters_list()]
-    m = L.make_mlp(params)
-    q = coords.shape[0]
-    if q >= 2 ** 31 - 128:
-        raise ValueError("at most 2^31 - 129 queries per call; split the batch")
-    geom = L.make_geom(method, c0, c1, 1, q, _step_log2(mip_level, fl), mip_level, var2.PE_CHANNELS, _pe_kind(method))
-    out = torch.empty((q, m.cout), dtype=out_dtype, device=c0.device)
-    h = L.handle(c0.device)
-    L.check(h, L.load_library().nic_decode_codes(h, C.byref(geom), L.ptr(c0), L.ptr(c1), num_bits, L.ptr(coords), C.byref(m),
-                                                 L.ptr(out), L.DT_U8 if out_dtype == torch.uint8 else L.DT_F32,
-                                                 L.PRECISIONS[precision.lower()], L.stream_ptr(c0.device)))
-    return out
+    return _decode(codes, num_bits, decoder, mip_level, None, None, coords, precision, out_dtype, None, method, level_table)
 
 
 # ------------------------------------------------------------------------------------------------ filtered sampling
@@ -410,10 +383,8 @@ def _mip_chain(fp_like, q, address, align_corners, method, table):
     return c, grids
 
 
-def _sample(launch, launch_lod, fp_like, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table,
-            grad=None):
-    """Common body of sample / sample_codes; launch(geom, grid0, grid1, sampler, mlp, out, out_dtype) calls the library for
-    one mip, launch_lod(chain, grids, mlp, out, out_dtype, coords, lod, ddx, ddy) for a per-query lod."""
+def _sample(fp_like, bits, decoder, coords, lod, size, address, align_corners, precision, out_dtype, method, level_table, grad):
+    """Common body of sample (bits None: float32 grids) and sample_codes (uint8 codes of width bits)."""
     method = _method() if method is None else method
     dim = 2 if method == L.METHOD_2D else 3
     table = feature_pyramid_mip_levels() if level_table is None else level_table
@@ -429,10 +400,15 @@ def _sample(launch, launch_lod, fp_like, decoder, coords, lod, size, address, al
     m = L.make_mlp(params)
     q = coords.shape[0]
     out = torch.empty((q, m.cout), dtype=out_dtype, device=coords.device)
+    pname = (precision or var2.DECODE_PRECISION).lower()
+    lib = L.load_library()
     if per_query:
         if q > 0:
             chain, grids = _mip_chain(fp_like, q, address, align_corners, method, table)
-            launch_lod(chain, grids, m, out, out_dtype, coords, *lod_inputs)
+            _check_grids(grids, bits)
+            _launch(L.handle(coords.device), lib.nic_sample_lod, lib.nic_sample_lod_codes, bits, pname, (C.byref(chain),),
+                    (L.ptr(coords), *[L.ptr(t) for t in lod_inputs], C.byref(m), L.ptr(out),
+                     L.DT_U8 if out_dtype == torch.uint8 else L.DT_F32), L.stream_ptr(coords.device))
         return out
     prev = None
     for i, (mip, t) in enumerate(passes):
@@ -448,7 +424,10 @@ def _sample(launch, launch_lod, fp_like, decoder, coords, lod, size, address, al
         smp.blend_weight, smp.blend_prev = t, (prev.data_ptr() if prev is not None else None)
         last = i == len(passes) - 1
         dst = out if last else torch.empty((q, m.cout), dtype=torch.float32, device=coords.device)
-        launch(geom, g0, g1, smp, m, dst, out_dtype if last else torch.float32, coords)
+        g0, g1 = _check_grids((g0, g1), bits)
+        _launch(L.handle(g0.device), lib.nic_sample, lib.nic_sample_codes, bits, pname, (C.byref(geom), L.ptr(g0), L.ptr(g1)),
+                (L.ptr(coords), C.byref(smp), C.byref(m), L.ptr(dst), L.DT_U8 if last and out_dtype == torch.uint8 else L.DT_F32),
+                L.stream_ptr(g0.device))
         prev = dst
     return out
 
@@ -468,62 +447,14 @@ def sample(fp, decoder, coords, lod=None, size=None, address="clamp", align_corn
     grad=(ddx, ddy), float32 CUDA tensors `[Q, D]` holding the derivatives of the normalised coordinates along the screen's
     x and y (lambda = log2 of the longer one in texels of mip 0).  Each query blends the two mips around its clamped lambda,
     over mips 0 .. min(MAX_MIP_LEVEL, max(level_table)) at their default extents (no `size`), in one pass."""
-    pname = (precision or var2.DECODE_PRECISION).lower()
-
-    def launch(geom, g0, g1, smp, m, dst, dt, coords):
-        g0, g1 = _check_grid(g0.detach()), _check_grid(g1.detach())
-        h = L.handle(g0.device)
-        # "auto": the tensor-core kernels where they exist (C = 12, PE = 6, hidden 64), else the reference-exact kernel
-        for prec in (("f16", "f32") if pname == "auto" else (pname,)):
-            rc = L.load_library().nic_sample(h, C.byref(geom), L.ptr(g0), L.ptr(g1), L.ptr(coords), C.byref(smp), C.byref(m),
-                                             L.ptr(dst), L.DT_U8 if dt == torch.uint8 else L.DT_F32, L.PRECISIONS[prec],
-                                             L.stream_ptr(g0.device))
-            if not (rc == L.ERR_UNSUPPORTED and pname == "auto" and prec != "f32"):
-                break
-        L.check(h, rc)
-
-    def launch_lod(chain, grids, m, dst, dt, coords, lod, ddx, ddy):
-        for g in grids:
-            _check_grid(g.detach())
-        h = L.handle(coords.device)
-        for prec in (("f16", "f32") if pname == "auto" else (pname,)):
-            rc = L.load_library().nic_sample_lod(h, C.byref(chain), L.ptr(coords), L.ptr(lod), L.ptr(ddx), L.ptr(ddy),
-                                                 C.byref(m), L.ptr(dst), L.DT_U8 if dt == torch.uint8 else L.DT_F32,
-                                                 L.PRECISIONS[prec], L.stream_ptr(coords.device))
-            if not (rc == L.ERR_UNSUPPORTED and pname == "auto" and prec != "f32"):
-                break
-        L.check(h, rc)
-
-    return _sample(launch, launch_lod, fp, decoder, coords, lod, size, address, align_corners, out_dtype, method, level_table,
-                   grad)
+    return _sample(fp, None, decoder, coords, lod, size, address, align_corners, precision, out_dtype, method, level_table, grad)
 
 
 def sample_codes(codes, decoder, coords, num_bits, lod=None, size=None, address="clamp", align_corners=False,
                  precision="f16", out_dtype=torch.float32, method=None, level_table=None, grad=None):
     """`sample` straight from the saved model (`codes`: the uint8 list of fp_savable, one code per byte); the de-quantisation
     of models.load4fp is fused into the grid read.  Tensor-core precisions only."""
-    def check_codes(cs):
-        for c in cs:
-            if not c.is_cuda or c.dtype != torch.uint8 or not c.is_contiguous():
-                raise TypeError("codes must be contiguous uint8 CUDA tensors")
-
-    def launch_lod(chain, grids, m, dst, dt, coords, lod, ddx, ddy):
-        check_codes(grids)
-        h = L.handle(coords.device)
-        L.check(h, L.load_library().nic_sample_lod_codes(h, C.byref(chain), num_bits, L.ptr(coords), L.ptr(lod), L.ptr(ddx),
-                                                         L.ptr(ddy), C.byref(m), L.ptr(dst),
-                                                         L.DT_U8 if dt == torch.uint8 else L.DT_F32,
-                                                         L.PRECISIONS[precision.lower()], L.stream_ptr(coords.device)))
-
-    def launch(geom, c0, c1, smp, m, dst, dt, coords):
-        check_codes((c0, c1))
-        h = L.handle(c0.device)
-        L.check(h, L.load_library().nic_sample_codes(h, C.byref(geom), L.ptr(c0), L.ptr(c1), num_bits, L.ptr(coords),
-                                                     C.byref(smp), C.byref(m), L.ptr(dst),
-                                                     L.DT_U8 if dt == torch.uint8 else L.DT_F32,
-                                                     L.PRECISIONS[precision.lower()], L.stream_ptr(c0.device)))
-
-    return _sample(launch, launch_lod, codes, decoder, coords, lod, size, address, align_corners, out_dtype, method,
+    return _sample(codes, num_bits, decoder, coords, lod, size, address, align_corners, precision, out_dtype, method,
                    level_table, grad)
 
 

@@ -184,7 +184,7 @@ def test_f32_sample_equals_oracle(kind, address, align_corners):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("precision", ["f32", "f16"])
+@pytest.mark.parametrize("precision", ["f32", "f16", "auto"])
 def test_sample_at_texel_centres_is_decode_points(precision):
     """f = 0 on every axis: the sample is the texel's decode, bit for bit (pins the tap, PE and LOD mapping)."""
     ic = nic().image_compression

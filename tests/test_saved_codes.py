@@ -320,14 +320,20 @@ def test_sample_and_bake_from_codes_at_odd_widths(bits):
 
 @pytest.mark.gpu
 def test_decode_codes_refusals():
-    """A float32-precision decode from codes is NIC_ERR_UNSUPPORTED; code widths 0 and 9 are NIC_ERR_ARG."""
+    """A float32-precision decode or sample from codes is NIC_ERR_UNSUPPORTED; code widths 0 and 9 are NIC_ERR_ARG.
+    sample_codes at an integer lod, at a fractional lod (two passes) and with a per-query lod tensor."""
     n = nic()
-    ic = n.image_compression
-    configure(IMAGE_SIZE=64)
-    codes = _codes(np.random.default_rng(860), [(12, s, s) for s in I.pyramid_sizes(64, True)], 8)
+    ic, fpd = n.image_compression, n.fp_def
+    configure(IMAGE_SIZE=64, TF_NO_MIP=False, MAX_MIP_LEVEL=6)
+    codes = _codes(np.random.default_rng(860), [(12, s, s) for s in I.pyramid_sizes(64, False)], 8)
     dec = make_decoder(I.make_mlp(73, seed=861))
-    for call in (lambda **kw: ic.decode_codes(codes, dec, level_table={0: 0}, **kw),
-                 lambda **kw: ic.decode_points_codes(codes, dec, torch.tensor([[3, 5]]), level_table={0: 0}, **kw)):
+    table = fpd.create_pyramid_mip_levels(64, 16)
+    c = T(_query_coords(np.random.default_rng(862), 64, 2))
+    lam = T(np.linspace(-1, 7, 64, dtype=F32))
+    calls = [lambda **kw: ic.decode_codes(codes, dec, level_table=table, **kw),
+             lambda **kw: ic.decode_points_codes(codes, dec, torch.tensor([[3, 5]]), level_table=table, **kw)]
+    calls += [lambda lod=lod, **kw: ic.sample_codes(codes, dec, c, lod=lod, level_table=table, **kw) for lod in (0, 1.25, lam)]
+    for call in calls:
         with pytest.raises(n.NicError) as e:
             call(num_bits=8, precision="f32")
         assert e.value.status == ERR_UNSUPPORTED
