@@ -100,9 +100,11 @@ int64_t nic_launch_count(const NicHandle* h);
 /* Tuning / testing knobs.  NIC_OPT_DISABLE_FAST2D = 1 forces the general tensor-core decode kernel even when the
  * geometry qualifies for the aligned full-resolution 2-D fast path (both must give the same image). */
 /* NIC_OPT_REUSE_PREPARED = 1: the caller asserts that grids and decoder weights have not changed since the previous
- * tensor-core nic_decode on this handle; if that call prepared its private tables (shadow grids, per-node G1 rows,
- * packed weights) for the same pointers, node counts, step, mip level and precision, they are reused instead of being
- * rebuilt (decoding one frame as several row bands).  Off by default: every call rebuilds from the caller's tensors. */
+ * tensor-core call on this handle (nic_decode, nic_decode_codes, nic_sample, nic_sample_codes, nic_sample_lod,
+ * nic_sample_lod_codes); if that call prepared its private tables (shadow grids, per-node G1 rows, packed weights) for the
+ * same kernel, pointers, node counts, steps, mip level, code width and precision, they are reused instead of being
+ * rebuilt (decoding one frame as several row bands).  A training step on the handle discards them.  Off by default: every
+ * call rebuilds from the caller's tensors. */
 /* NIC_OPT_DEBUG_KNOCKOUT: profiling only (tools/run_decode.py, tools/run_train.py) — decode: bit 0 skips the output
  * stores, bit 1 replaces GELU by a plain pack, bit 2 issues one MMA per layer; training: bit 4 skips the grid-gradient
  * atomics, bits 5 / 6 make nic_adam_step_exchange skip the flag wait / read only its own buffer (timing experiments in

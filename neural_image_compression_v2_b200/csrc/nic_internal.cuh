@@ -49,15 +49,15 @@ struct Handle {
   size_t sample_scratch_bytes;
   void* lod_chain;           // nic_sample_lod (tensor core): device copy of the call's DevChain
   int gelu_poly;             // NIC_OPT_GELU_POLY: -1 = tuned default, 0..8 = activation pairs (of 8) on the polynomial GELU
-  struct PreparedKey {       // what the tables in tc_weights / tc_shadow were last built from
-    const void *g0, *g1, *w1, *b1, *w2, *b2, *w3, *b3;
-    int n0[3], n1[3], method, pe_kind, mip, fmt, fast, valid, code_bits, npoly;
-    float step;
-    // nic_sample_lod: every mip of the chain (its grids, nodes and step); zero for the single-mip paths
-    int chain_mips;
-    const void* chain_g[2 * NIC_MAX_MIPS];
-    int chain_nodes[NIC_MAX_MIPS][6];
-    float chain_step[NIC_MAX_MIPS];
+  struct PreparedKey {       // what the tables in tc_weights / tc_shadow were last built from (compared with memcmp)
+    int kind;                // PreparedKind: the kernel they were built for (PREP_NONE: nothing valid)
+    int fmt, code_bits, npoly, method, pe_kind, mip, num_mips;
+    const void *w1, *b1, *w2, *b2, *w3, *b3;
+    struct Mip {             // each mip the call reads: one for a single-mip call, the whole chain for nic_sample_lod
+      const void *g0, *g1;
+      int n0[3], n1[3];
+      float step;
+    } mips[NIC_MAX_MIPS];
   } prepared;
   void* adam_desc;           // device copy of NicAdamTensor descriptors
   size_t adam_desc_bytes;
@@ -67,6 +67,12 @@ struct Handle {
   cudaEvent_t timed_ev[2 * 256];
 };
 #define NIC_MAX_TIMED 256
+
+// The kernels whose tables a PreparedKey describes: each builds its own weight image (and shadows or G1 rows), so tables
+// are shared only between calls of the same kind.
+enum PreparedKind { PREP_NONE = 0, PREP_GENERAL, PREP_FAST2D, PREP_CODES, PREP_CHAIN };
+// Marks the prepared tables stale: their scratch was reallocated, or overwritten by the training step.
+static inline void invalidate_prepared(Handle* h) { h->prepared.kind = PREP_NONE; }
 
 // Brackets the dominant kernel of a call with events when NIC_OPT_TIME_KERNELS is on (no-op otherwise).
 // Programmatic dependent launch (sm_90+): a kernel launched with launch_pdl() may start while its predecessor in the

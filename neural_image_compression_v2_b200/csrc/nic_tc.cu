@@ -920,13 +920,6 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
 // offset (bytes -> exact f16 integers through 0x6400 | b = 1024 + b), and 1 / (2^bits - 1) rides in W1 (pack_weights_kernel
 // gscale).  f16 only (the byte trick needs 11 mantissa bits); otherwise the structure of decode_tc_gws_kernel with NG = 3.
 constexpr int CQ_NG = 3;
-template <int METHOD>
-__host__ __device__ constexpr int cq_fixed_smem() {
-  using S = RowShape<METHOD>;
-  return b_image_bytes(64, S::KX) + b_image_bytes(64, TC_K2) + b_image_bytes(16, TC_K2) + TC_LUT_MAX * 16 + 2 * 2048 +
-         CQ_NG * (S::KX / 8) * 2048 + 256;
-}
-
 template <int METHOD, typename OutT, int NPOLY>
 __global__ void __launch_bounds__(CQ_NG * GW_GROUP, 1)
     decode_codes_smem_kernel(DevGeom g, const uint8_t* __restrict__ codes0, const uint8_t* __restrict__ codes1, int code_off,
@@ -1169,21 +1162,71 @@ __global__ void __launch_bounds__(CQ_NG * GW_GROUP, 1)
 }
 
 // ------------------------------------------------------------------------------------------------ launcher
-// NIC_OPT_REUSE_PREPARED: do the private tables already describe these inputs?
-static Handle::PreparedKey make_key(const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int fmt, int fast,
-                                    int code_bits, int npoly) {
+// NIC_OPT_REUSE_PREPARED: what the tables of a call are built from.  gm, g0 and g1 hold num_mips entries.
+static Handle::PreparedKey make_key(int kind, int fmt, int code_bits, int npoly, const MlpDev& m, const DevGeom* gm,
+                                    const void* const* g0, const void* const* g1, int num_mips) {
   Handle::PreparedKey k;
-  memset(&k, 0, sizeof(k));
-  k.g0 = g0; k.g1 = g1; k.w1 = m.w1; k.b1 = m.b1; k.w2 = m.w2; k.b2 = m.b2; k.w3 = m.w3; k.b3 = m.b3;
-  for (int a = 0; a < 3; ++a) { k.n0[a] = g.n0[a]; k.n1[a] = g.n1[a]; }
-  k.method = g.method; k.pe_kind = g.pe_kind; k.mip = g.mip; k.fmt = fmt; k.fast = fast; k.valid = 1;
-  k.code_bits = code_bits;
-  k.npoly = npoly;
-  k.step = g.step;
+  memset(&k, 0, sizeof(k));                            // (padding included: keys are compared with memcmp)
+  k.kind = kind; k.fmt = fmt; k.code_bits = code_bits; k.npoly = npoly;
+  k.method = gm[0].method; k.pe_kind = gm[0].pe_kind; k.mip = gm[0].mip; k.num_mips = num_mips;
+  k.w1 = m.w1; k.b1 = m.b1; k.w2 = m.w2; k.b2 = m.b2; k.w3 = m.w3; k.b3 = m.b3;
+  for (int i = 0; i < num_mips; ++i) {
+    Handle::PreparedKey::Mip& p = k.mips[i];
+    p.g0 = g0[i];
+    p.g1 = g1[i];
+    memcpy(p.n0, gm[i].n0, sizeof(p.n0));
+    memcpy(p.n1, gm[i].n1, sizeof(p.n1));
+    p.step = gm[i].step;
+  }
   return k;
 }
-static bool prepared_matches(Handle* h, const Handle::PreparedKey& k) {
-  return h->reuse_prepared && h->prepared.valid && memcmp(&h->prepared, &k, sizeof(k)) == 0;
+// Runs build() (NIC_OK or an error) unless reuse is on and the tables already describe `key`; the key is kept only when
+// the build succeeds.
+template <class Build>
+static int prepare_tables(Handle* h, const Handle::PreparedKey& key, Build&& build) {
+  if (h->reuse_prepared && memcmp(&h->prepared, &key, sizeof(key)) == 0) return NIC_OK;
+  invalidate_prepared(h);
+  const int rc = build();
+  if (rc == NIC_OK) memcpy(&h->prepared, &key, sizeof(key));
+  return rc;
+}
+
+// How many of every 8 activation pairs take the polynomial (FMA-pipe) GELU instead of MUFU.TANH: tuned per format so that
+// the XU and FMA pipes finish together (profiles/r02*); NIC_OPT_GELU_POLY overrides it for A/B runs.
+static int resolve_npoly(const Handle* h, int fmt) {
+  return h->gelu_poly >= 0 ? h->gelu_poly : (fmt == 0 ? WS_NPOLY_F16 : WS_NPOLY_BF16);
+}
+
+// Positional-encoding LUT length, or NIC_ERR_UNSUPPORTED: the triangular encoding has period 16/step texels.
+static int pe_lut_len(const DevGeom& g) {
+  const float period = 16.0f / g.step;
+  int n = 1;
+  while (n < period && n < TC_LUT_MAX) n <<= 1;
+  return g.pe_kind == NIC_PE_TRIANGULAR && (float)n < period ? NIC_ERR_UNSUPPORTED : n;
+}
+
+// Dynamic shared memory of decode_tc_gws_kernel with NG groups and a LUTCAP-entry LUT: weight images, LUT, ones block,
+// operand buffers, barriers, and behind them the chain table of a per-query-LOD launch.  The code-resident kernel has the
+// same layout with CQ_NG groups, followed by its two grids.
+template <int METHOD>
+constexpr int gws_smem(int ng, int lutcap, bool chain = false) {
+  using S = RowShape<METHOD>;
+  return b_image_bytes(64, S::KX) + b_image_bytes(64, TC_K2) + b_image_bytes(16, TC_K2) + lutcap * 16 + 2 * 2048 +
+         ng * (S::KX / 8) * 2048 + 256 + (chain ? (int)((sizeof(DevChain) + 15) & ~15) : 0);
+}
+
+// One launch of a persistent tensor-core kernel: at most one CTA per SM for `units` work units (tiles or tile groups).
+template <typename... KArgs, typename... Args>
+static int launch_persistent(Handle* h, void (*kern)(KArgs...), long long units, int threads, int smem, cudaStream_t st,
+                             const Args&... args) {
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e != cudaSuccess) return (int)e;
+  {
+    KernelTimer timer(h, st);
+    kern<<<(int)(units < h->sms ? units : h->sms), threads, smem, st>>>(args...);
+  }
+  h->launches++;
+  return (int)cudaGetLastError();
 }
 
 static bool fast2d_eligible(const DevGeom& g, const long long* origins) {
@@ -1193,34 +1236,33 @@ static bool fast2d_eligible(const DevGeom& g, const long long* origins) {
 }
 
 // Random-access queries (1-texel blocks) on a model given as uint8 codes whose two grids fit shared memory next to three
-// operand buffers: the code-resident kernel.  Returns -1000 when the call does not qualify (the caller falls through).
+// operand buffers: the code-resident kernel.
+static long long codes_bytes(const int* nodes, int dim) { return (plane_size_host(nodes, dim) * 12 + 15) & ~15ll; }
+template <int METHOD>
+static long long codes_smem(const DevGeom& g) {
+  return gws_smem<METHOD>(CQ_NG, TC_LUT_MAX) + codes_bytes(g.n0, g.dim) + codes_bytes(g.n1, g.dim);
+}
+template <int METHOD>
+static bool codes_smem_eligible(const DevGeom& g, int bits, const long long* origins) {
+  return bits >= 1 && bits <= 8 && origins && g.per_block == 1 && codes_smem<METHOD>(g) <= 227 * 1024;
+}
+
 template <int METHOD, typename OutT>
 static int launch_codes_smem(Handle* h, const DevGeom& g, const MlpDev& m, const void* c0, const void* c1, int bits,
                              const long long* origins, OutT* out, cudaStream_t st) {
   using S = RowShape<METHOD>;
-  const long long nodes0 = plane_size_host(g.n0, g.dim), nodes1 = plane_size_host(g.n1, g.dim);
-  const long long bytes0 = (nodes0 * 12 + 15) & ~15ll, bytes1 = (nodes1 * 12 + 15) & ~15ll;
-  const long long smem = cq_fixed_smem<METHOD>() + bytes0 + bytes1;
-  if (!origins || g.per_block != 1 || bits < 1 || bits > 8 || smem > 227 * 1024 || h->disable_fast2d) return -1000;
-  int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
+  int rc = tc_scratch(h, 0);
   if (rc) return rc;
-  const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : WS_NPOLY_F16;
-  const Handle::PreparedKey key = make_key(g, m, c0, c1, 0, 2, bits, npoly);
-  if (!prepared_matches(h, key)) {
-    h->prepared.valid = 0;
+  const int npoly = resolve_npoly(h, 0);
+  rc = prepare_tables(h, make_key(PREP_CODES, 0, bits, npoly, m, &g, &c0, &c1, 1), [&] {
     pack_weights_kernel<0><<<16, 256, 0, st>>>(m, g.lod, S::KX, (uint16_t*)h->tc_weights, npoly, 12 * (S::NC0 + 1),
                                                1.0f / (float)((1 << bits) - 1));
     h->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-    memcpy(&h->prepared, &key, sizeof(key));
-  }
-  int lut_n = 1;
-  {
-    float period = 16.0f / g.step;
-    while (lut_n < period && lut_n < TC_LUT_MAX) lut_n <<= 1;
-    if (g.pe_kind == NIC_PE_TRIANGULAR && (float)lut_n < period) return NIC_ERR_UNSUPPORTED;
-  }
+    return (int)cudaGetLastError();
+  });
+  if (rc) return rc;
+  const int lut_n = pe_lut_len(g);
+  if (lut_n < 0) return lut_n;
   if (g.N >= (1ll << 31) - TC_ROWS) return NIC_ERR_UNSUPPORTED;
   void (*kern)(DevGeom, const uint8_t*, const uint8_t*, int, int, const long long*, const uint4*, int, int, OutT*) = nullptr;
   switch (npoly) {
@@ -1228,50 +1270,34 @@ static int launch_codes_smem(Handle* h, const DevGeom& g, const MlpDev& m, const
     case 3: kern = decode_codes_smem_kernel<METHOD, OutT, 3>; break;
     default: return NIC_ERR_UNSUPPORTED;
   }
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  const long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS, groups = (ntiles + CQ_NG - 1) / CQ_NG;
-  const int grid = (int)(groups < h->sms ? groups : h->sms);
-  {
-    KernelTimer timer(h, st);
-    kern<<<grid, CQ_NG * GW_GROUP, (size_t)smem, st>>>(g, (const uint8_t*)c0, (const uint8_t*)c1, (1 << (bits - 1)) - 1,
-                                                        (int)bytes0, origins, (const uint4*)h->tc_weights, m.cout, lut_n, out);
-  }
-  h->launches++;
-  return (int)cudaGetLastError();
+  const long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS;
+  return launch_persistent(h, kern, (ntiles + CQ_NG - 1) / CQ_NG, CQ_NG * GW_GROUP, (int)codes_smem<METHOD>(g), st, g,
+                           (const uint8_t*)c0, (const uint8_t*)c1, (1 << (bits - 1)) - 1, (int)codes_bytes(g.n0, g.dim),
+                           origins, (const uint4*)h->tc_weights, m.cout, lut_n, out);
 }
 
 template <int FMT, typename OutT>
 static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
                          OutT* out, cudaStream_t st) {
-  int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
-  if (rc) return rc;
   const long long nodes0 = plane_size_host(g.n0, 2), nodes1 = plane_size_host(g.n1, 2);
-  const size_t b0 = ((size_t)nodes0 * g.C * 2 + 255) & ~(size_t)255, b1 = (size_t)nodes1 * 128;
-  rc = ensure_scratch(&h->tc_shadow, &h->tc_shadow_bytes, b0 + b1);
+  const size_t b0 = ((size_t)nodes0 * g.C * 2 + 255) & ~(size_t)255, b1 = (size_t)nodes1 * 128;     // the G0 shadow, then R
+  int rc = tc_scratch(h, b0 + b1);
   if (rc) return rc;
   uint16_t* s0 = (uint16_t*)h->tc_shadow;
   uint16_t* R = (uint16_t*)((uint8_t*)h->tc_shadow + b0);
-  cudaError_t e = cudaSuccess;
-  // how many of every 8 activation pairs take the polynomial (FMA-pipe) GELU instead of MUFU.TANH: tuned per format so
-  // that the XU and FMA pipes finish together (profiles/r02*); NIC_OPT_GELU_POLY overrides it for A/B runs
-  const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : (FMT == 0 ? WS_NPOLY_F16 : WS_NPOLY_BF16);
-  const Handle::PreparedKey key = make_key(g, m, g0, g1, FMT, 1, code_bits, npoly);
-  if (!prepared_matches(h, key)) {
-    h->prepared.valid = 0;
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, code_bits, g.n0, s0, st);
-    if (e != cudaSuccess) return (int)e;
+  const int npoly = resolve_npoly(h, FMT);
+  rc = prepare_tables(h, make_key(PREP_FAST2D, FMT, code_bits, npoly, m, &g, &g0, &g1, 1), [&] {
+    const int e = launch_relayout<FMT>(h, g, g0, code_bits, g.n0, s0, st);
+    if (e) return e;
     const long long tiles_r = (long long)((g.n1[0] + G1R_TX - 1) / G1R_TX) * ((g.n1[1] + G1R_TY - 1) / G1R_TY);
     const long long cap_r = 2ll * h->sms;
     g1_rows_kernel<FMT><<<(int)(tiles_r < cap_r ? tiles_r : cap_r), 256, 0, st>>>(m, (const float*)g1, g.n1[0], g.n1[1], R,
                                                                                  code_bits);
-    h->launches++;
     pack_fast_kernel<FMT><<<32, 256, 0, st>>>(m, g.lod, g.step, (uint16_t*)h->tc_weights, npoly);
-    h->launches++;
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-    memcpy(&h->prepared, &key, sizeof(key));
-  }
+    h->launches += 2;
+    return (int)cudaGetLastError();
+  });
+  if (rc) return rc;
   unsigned tiles_y = (unsigned)(g.B[1] / F_TY);
   long long ntiles = (long long)(g.B[0] / F_TX) * tiles_y;
   if (ntiles >= (1ll << 31) || g.N >= (1ll << 31)) return NIC_ERR_UNSUPPORTED;     // 32-bit texel index in the kernel
@@ -1295,136 +1321,57 @@ static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const voi
 #endif
     default: return NIC_ERR_UNSUPPORTED;
   }
-  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SMEM);
-  if (e != cudaSuccess) return (int)e;
-  int grid = (int)(ntiles < h->sms ? ntiles : h->sms);
-  {
-    KernelTimer timer(h, st);
-    kern<<<grid, WS_THREADS, WS_SMEM, st>>>(g, (const uint2*)s0, (const uint4*)R, (const uint4*)h->tc_weights, m.cout,
-                                             tiles_y, mul, sh, out, h->debug_flags);
-  }
-  h->launches++;
-  return (int)cudaGetLastError();
+  return launch_persistent(h, kern, ntiles, WS_THREADS, WS_SMEM, st, g, (const uint2*)s0, (const uint4*)R,
+                           (const uint4*)h->tc_weights, m.cout, tiles_y, mul, sh, out, h->debug_flags);
 }
 
 // TAPS > 0: filtered sampling (smp set, g.N = queries * TAPS rows) always runs on the general kernel: the fast 2-D kernel
 // and the code-resident kernel have no per-row texel and no tap epilogue.
-template <int METHOD, int FMT, typename OutT, int TAPS = 0>
+template <int METHOD, int FMT, int TAPS, typename OutT>
 static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
-                       const long long* origins, OutT* out, cudaStream_t st, const DevSampler* smp = nullptr) {
+                       const long long* origins, OutT* out, cudaStream_t st, const DevSampler& smp = DevSampler{}) {
   using S = RowShape<METHOD>;
   if constexpr (METHOD == NIC_METHOD_2D && TAPS == 0) {
     if (fast2d_eligible(g, origins) && !h->disable_fast2d) return launch_fast2d<FMT, OutT>(h, g, m, g0, g1, code_bits, out, st);
   }
   if constexpr (METHOD == NIC_METHOD_3D && FMT == 0 && TAPS == 0) {       // small models given as codes, random-access queries
-    if (code_bits > 0) {
-      const int crc = launch_codes_smem<METHOD, OutT>(h, g, m, g0, g1, code_bits, origins, out, st);
-      if (crc != -1000) return crc;
-    }
+    if (codes_smem_eligible<METHOD>(g, code_bits, origins) && !h->disable_fast2d)
+      return launch_codes_smem<METHOD, OutT>(h, g, m, g0, g1, code_bits, origins, out, st);
   }
-  constexpr int IMG = b_image_bytes(64, S::KX) + b_image_bytes(64, TC_K2) + b_image_bytes(16, TC_K2);
-  int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
+  const int npoly = resolve_npoly(h, FMT);
+  if (npoly != 0 && npoly != 3) return NIC_ERR_UNSUPPORTED;      // (the NIC_GELU_SWEEP values exist for the fast 2-D kernel only)
+  const ShadowLayout sl = shadow_layout(&g, &g0, &g1, 1);
+  int rc = tc_scratch(h, sl.total);
   if (rc) return rc;
-  // 16-bit channel-last shadows of the two active grids
-  const long long nodes0 = plane_size_host(g.n0, g.dim), nodes1 = plane_size_host(g.n1, g.dim);
-  const size_t b0 = ((size_t)nodes0 * g.C * 2 + 255) & ~(size_t)255, b1 = ((size_t)nodes1 * g.C * 2 + 255) & ~(size_t)255;
-  rc = ensure_scratch(&h->tc_shadow, &h->tc_shadow_bytes, b0 + b1);
-  if (rc) return rc;
-  uint16_t* s0 = (uint16_t*)h->tc_shadow;
-  uint16_t* s1 = (uint16_t*)((uint8_t*)h->tc_shadow + b0);
-  cudaError_t e = cudaSuccess;
-  const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : (FMT == 0 ? WS_NPOLY_F16 : WS_NPOLY_BF16);
-  const Handle::PreparedKey key = make_key(g, m, g0, g1, FMT, 0, code_bits, npoly);
-  if (!prepared_matches(h, key)) {
-    h->prepared.valid = 0;
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, code_bits, g.n0, s0, st);
-    if (e != cudaSuccess) return (int)e;
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g1, code_bits, g.n1, s1, st);
-    if (e != cudaSuccess) return (int)e;
+  rc = prepare_tables(h, make_key(PREP_GENERAL, FMT, code_bits, npoly, m, &g, &g0, &g1, 1), [&] {
+    const int e = build_shadows<FMT>(h, sl, &g, &g0, &g1, code_bits, st);
+    if (e) return e;
     pack_weights_kernel<FMT><<<16, 256, 0, st>>>(m, g.lod, S::KX, (uint16_t*)h->tc_weights, npoly);
     h->launches++;
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-    memcpy(&h->prepared, &key, sizeof(key));
-  }
-  // positional-encoding LUT length: the triangular encoding has period 16/step texels
-  int lut_n = 1;
-  {
-    float period = 16.0f / g.step;
-    while (lut_n < period && lut_n < TC_LUT_MAX) lut_n <<= 1;
-    if (g.pe_kind == NIC_PE_TRIANGULAR && (float)lut_n < period) return NIC_ERR_UNSUPPORTED;
-  }
+    return (int)cudaGetLastError();
+  });
+  if (rc) return rc;
+  const int lut_n = pe_lut_len(g);
+  if (lut_n < 0) return lut_n;
   if (g.N >= (1ll << 31) - TC_ROWS) return NIC_ERR_UNSUPPORTED;     // 32-bit sample index in the kernel
-  long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS;
-  ShadowGeom sg = {(const uint2*)s0, (const uint2*)s1};
+  const ShadowGeom sg = {(const uint2*)h->tc_shadow, (const uint2*)((uint8_t*)h->tc_shadow + sl.off[0][1])};
   // warp-specialised persistent kernel: one CTA per SM, NG groups of 4 warps
-  constexpr int NG0 = gws_groups(S::KX, 0);
-  constexpr int GSMEM0 = IMG + TC_LUT_MAX * 16 + 2 * 2048 + NG0 * (S::KX / 8) * 2048 + 256;
-  constexpr int GSMEM6 = IMG + 64 * 16 + 2 * 2048 + 6 * (S::KX / 8) * 2048 + 256;      // method 3: six groups, 64-entry LUT
+  constexpr int NG0 = gws_groups(S::KX, 0), GSMEM0 = gws_smem<METHOD>(NG0, TC_LUT_MAX);
+  constexpr int GSMEM6 = gws_smem<METHOD>(6, 64);                  // method 3: six groups, 64-entry LUT
   static_assert(GSMEM0 <= 227 * 1024 && (S::KX <= 80 || GSMEM6 <= 227 * 1024), "shared memory budget");
   // (not for random-access queries: they live on L1 hits, and the sixth group's 32 KB come out of the L1 — measured
   //  4.8 -> 4.2 Gquery/s on a 256^3 volume)
   const bool six = TAPS == 0 && S::KX > 80 && lut_n <= 64 && g.per_block > 1 && !(h->debug_flags & 128);
-  const int NG = six ? 6 : NG0, GSMEM = six ? GSMEM6 : GSMEM0;
-  void (*kern)(DevGeom, ShadowGeom, const long long*, const uint4*, int, int, OutT*, DevSampler) = nullptr;
+  const int NG = six ? 6 : NG0;
+  void (*kern)(DevGeom, ShadowGeom, const long long*, const uint4*, int, int, OutT*, DevSampler) =
+      npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 0, TC_LUT_MAX, TAPS>
+                 : decode_tc_gws_kernel<METHOD, FMT, OutT, 3, 0, TC_LUT_MAX, TAPS>;
   if constexpr (S::KX > 80 && TAPS == 0) {
     if (six) kern = npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 6, 64> : decode_tc_gws_kernel<METHOD, FMT, OutT, 3, 6, 64>;
   }
-  if (!kern)
-    kern = npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 0, TC_LUT_MAX, TAPS>
-                      : decode_tc_gws_kernel<METHOD, FMT, OutT, 3, 0, TC_LUT_MAX, TAPS>;
-  if (npoly != 0 && npoly != 3) return NIC_ERR_UNSUPPORTED;      // (the NIC_GELU_SWEEP values exist for the fast 2-D kernel only)
-  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, GSMEM);
-  if (e != cudaSuccess) return (int)e;
-  long long groups = (ntiles + NG - 1) / NG;
-  int grid = (int)(groups < h->sms ? groups : h->sms);
-  const DevSampler no_sampler = {};
-  {
-    KernelTimer timer(h, st);
-    kern<<<grid, NG * GW_GROUP, GSMEM, st>>>(g, sg, origins, (const uint4*)h->tc_weights, m.cout, lut_n, out,
-                                             smp ? *smp : no_sampler);
-  }
-  h->launches++;
-  return (int)cudaGetLastError();
-}
-
-template <int METHOD, int TAPS = 0>
-static int launch_tc_m(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
-                       const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st,
-                       const DevSampler* smp = nullptr) {
-  if (precision == NIC_PREC_F16) {
-    if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 0, uint8_t, TAPS>(h, g, m, g0, g1, code_bits, origins, (uint8_t*)out, st, smp);
-    return launch_tc_t<METHOD, 0, float, TAPS>(h, g, m, g0, g1, code_bits, origins, (float*)out, st, smp);
-  }
-  if (out_dtype == NIC_DT_U8) return launch_tc_t<METHOD, 1, uint8_t, TAPS>(h, g, m, g0, g1, code_bits, origins, (uint8_t*)out, st, smp);
-  return launch_tc_t<METHOD, 1, float, TAPS>(h, g, m, g0, g1, code_bits, origins, (float*)out, st, smp);
-}
-
-int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
-                     const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st) {
-  if (g.N == 0) return NIC_OK;
-  if (g.C != 12 || g.PE != 6 || m.hidden != 64 || m.cout > 16) return NIC_ERR_UNSUPPORTED;
-  switch (g.method) {
-    case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D>(h, g, m, g0, g1, code_bits, origins, out, out_dtype, precision, st);
-    case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D>(h, g, m, g0, g1, code_bits, origins, out, out_dtype, precision, st);
-    case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2>(h, g, m, g0, g1, code_bits, origins, out, out_dtype, precision, st);
-  }
-  return NIC_ERR_UNSUPPORTED;
-}
-
-int launch_sample_tc(Handle* h, const DevGeom& gq, const DevSampler& smp, const MlpDev& m, const void* g0, const void* g1,
-                     int code_bits, void* out, int out_dtype, int precision, cudaStream_t st) {
-  if (gq.nblocks == 0) return NIC_OK;
-  if (gq.C != 12 || gq.PE != 6 || m.hidden != 64 || m.cout > 16) return NIC_ERR_UNSUPPORTED;
-  DevGeom g = gq;                                   // one row per tap: queries x 2^dim rows
-  g.N = (long long)gq.nblocks << gq.dim;
-  if (g.N >= (1ll << 31) - TC_ROWS) return NIC_ERR_UNSUPPORTED;     // 32-bit row index in the kernel
-  switch (g.method) {
-    case NIC_METHOD_2D: return launch_tc_m<NIC_METHOD_2D, 4>(h, g, m, g0, g1, code_bits, nullptr, out, out_dtype, precision, st, &smp);
-    case NIC_METHOD_3D: return launch_tc_m<NIC_METHOD_3D, 8>(h, g, m, g0, g1, code_bits, nullptr, out, out_dtype, precision, st, &smp);
-    case NIC_METHOD_3D_V2: return launch_tc_m<NIC_METHOD_3D_V2, 8>(h, g, m, g0, g1, code_bits, nullptr, out, out_dtype, precision, st, &smp);
-  }
-  return NIC_ERR_UNSUPPORTED;
+  const long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS;
+  return launch_persistent(h, kern, (ntiles + NG - 1) / NG, NG * GW_GROUP, six ? GSMEM6 : GSMEM0, st, g, sg, origins,
+                           (const uint4*)h->tc_weights, m.cout, lut_n, out, smp);
 }
 
 // Per-query LOD: the shadow grids of every pyramid level the chain reaches (built once, keyed by the whole chain), the
@@ -1434,118 +1381,84 @@ static int launch_lod_t(Handle* h, const DevGeom* gm, DevChain c, const DevSampl
                         const void* const* g0, const void* const* g1, int code_bits, OutT* out, cudaStream_t st) {
   using S = RowShape<METHOD>;
   constexpr int TAPS = 2 << S::DIM;
-  int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
+  const ShadowLayout sl = shadow_layout(gm, g0, g1, c.num_mips);
+  if (sl.total / 8 >= (1ull << 32)) return NIC_ERR_UNSUPPORTED;            // 32-bit shadow offsets in the chain table
+  int rc = tc_scratch(h, sl.total);
   if (rc) return rc;
-  size_t off[NIC_MAX_MIPS][2];
-  int first[NIC_MAX_MIPS];                           // the first mip of the chain with the same grids (one shadow each)
-  size_t total = 0;
   for (int i = 0; i < c.num_mips; ++i) {
-    first[i] = i;
-    for (int j = 0; j < i && first[i] == i; ++j)
-      if (g0[j] == g0[i] && g1[j] == g1[i] && !memcmp(gm[j].n0, gm[i].n0, sizeof(gm[i].n0)) &&
-          !memcmp(gm[j].n1, gm[i].n1, sizeof(gm[i].n1)))
-        first[i] = j;
-    if (first[i] != i) {
-      off[i][0] = off[first[i]][0];
-      off[i][1] = off[first[i]][1];
-      continue;
-    }
-    off[i][0] = total;
-    total += ((size_t)plane_size_host(gm[i].n0, gm[i].dim) * gm[i].C * 2 + 255) & ~(size_t)255;
-    off[i][1] = total;
-    total += ((size_t)plane_size_host(gm[i].n1, gm[i].dim) * gm[i].C * 2 + 255) & ~(size_t)255;
+    c.mip[i].s0 = (unsigned)(sl.off[i][0] / 8);
+    c.mip[i].s1 = (unsigned)(sl.off[i][1] / 8);
   }
-  if (total / 8 >= (1ull << 32)) return NIC_ERR_UNSUPPORTED;            // 32-bit shadow offsets in the chain table
-  rc = ensure_scratch(&h->tc_shadow, &h->tc_shadow_bytes, total);
-  if (rc) return rc;
-  uint8_t* shadow = (uint8_t*)h->tc_shadow;
-  for (int i = 0; i < c.num_mips; ++i) {
-    c.mip[i].s0 = (unsigned)(off[i][0] / 8);
-    c.mip[i].s1 = (unsigned)(off[i][1] / 8);
-  }
-  cudaError_t e = cudaSuccess;
-  const int npoly = h->gelu_poly >= 0 ? h->gelu_poly : (FMT == 0 ? WS_NPOLY_F16 : WS_NPOLY_BF16);
+  const int npoly = resolve_npoly(h, FMT);
   if (npoly != 0 && npoly != 3) return NIC_ERR_UNSUPPORTED;
-  Handle::PreparedKey key = make_key(gm[0], m, g0[0], g1[0], FMT, 3, code_bits, npoly);
-  key.chain_mips = c.num_mips;
-  for (int i = 0; i < c.num_mips; ++i) {
-    key.chain_g[2 * i] = g0[i];
-    key.chain_g[2 * i + 1] = g1[i];
-    for (int a = 0; a < 3; ++a) { key.chain_nodes[i][a] = gm[i].n0[a]; key.chain_nodes[i][3 + a] = gm[i].n1[a]; }
-    key.chain_step[i] = gm[i].step;
-  }
-  if (!prepared_matches(h, key)) {
-    h->prepared.valid = 0;
-    for (int i = 0; i < c.num_mips; ++i) {
-      if (first[i] != i) continue;
-      e = (cudaError_t)launch_relayout<FMT>(h, gm[i], g0[i], code_bits, gm[i].n0, (uint16_t*)(shadow + off[i][0]), st);
-      if (e != cudaSuccess) return (int)e;
-      e = (cudaError_t)launch_relayout<FMT>(h, gm[i], g1[i], code_bits, gm[i].n1, (uint16_t*)(shadow + off[i][1]), st);
-      if (e != cudaSuccess) return (int)e;
-    }
+  rc = prepare_tables(h, make_key(PREP_CHAIN, FMT, code_bits, npoly, m, gm, g0, g1, c.num_mips), [&] {
+    const int e = build_shadows<FMT>(h, sl, gm, g0, g1, code_bits, st);
+    if (e) return e;
     pack_weights_kernel<FMT><<<16, 256, 0, st>>>(m, 0.0f, S::KX, (uint16_t*)h->tc_weights, npoly);
     pack_lod_columns_kernel<FMT><<<1, 64, 0, st>>>(m, (uint16_t*)h->tc_weights);
     h->launches += 2;
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-    memcpy(&h->prepared, &key, sizeof(key));
-  }
+    return (int)cudaGetLastError();
+  });
+  if (rc) return rc;
   if (!h->lod_chain && cudaMalloc(&h->lod_chain, sizeof(DevChain)) != cudaSuccess) {
     h->lod_chain = nullptr;
     return NIC_ERR_SCRATCH;
   }
-  e = cudaMemcpyAsync(h->lod_chain, &c, sizeof(DevChain), cudaMemcpyHostToDevice, st);
+  cudaError_t e = cudaMemcpyAsync(h->lod_chain, &c, sizeof(DevChain), cudaMemcpyHostToDevice, st);
   if (e != cudaSuccess) return (int)e;
   DevGeom g = gm[0];                                  // method, PE, coordinates; the rest is per row from the chain
   g.N = (long long)g.nblocks * TAPS;
   g.interp = 1;                                       // (g1_factors computes the weights; rows of step-2 mips drop them)
-  const long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS;
-  ShadowGeom sg = {(const uint2*)shadow, (const uint2*)shadow};
-  constexpr int IMG = b_image_bytes(64, S::KX) + b_image_bytes(64, TC_K2) + b_image_bytes(16, TC_K2);
-  constexpr int NG = gws_groups(S::KX, 0);
-  constexpr int GSMEM = IMG + TC_LUT_MAX * 16 + 2 * 2048 + NG * (S::KX / 8) * 2048 + 256 + ((sizeof(DevChain) + 15) & ~15);
+  const ShadowGeom sg = {(const uint2*)h->tc_shadow, (const uint2*)h->tc_shadow};
+  constexpr int NG = gws_groups(S::KX, 0), GSMEM = gws_smem<METHOD>(NG, TC_LUT_MAX, true);
   static_assert(GSMEM <= 227 * 1024, "shared memory budget");
   void (*kern)(DevGeom, ShadowGeom, const long long*, const uint4*, int, int, OutT*, DevSampler) =
       npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 0, TC_LUT_MAX, TAPS>
                  : decode_tc_gws_kernel<METHOD, FMT, OutT, 3, 0, TC_LUT_MAX, TAPS>;
-  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, GSMEM);
-  if (e != cudaSuccess) return (int)e;
-  const long long groups = (ntiles + NG - 1) / NG;
-  const int grid = (int)(groups < h->sms ? groups : h->sms);
-  {
-    KernelTimer timer(h, st);
-    kern<<<grid, NG * GW_GROUP, GSMEM, st>>>(g, sg, (const long long*)h->lod_chain, (const uint4*)h->tc_weights, m.cout, 64,
-                                             out, smp);
-  }
-  h->launches++;
-  return (int)cudaGetLastError();
+  const long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS;
+  return launch_persistent(h, kern, (ntiles + NG - 1) / NG, NG * GW_GROUP, GSMEM, st, g, sg, (const long long*)h->lod_chain,
+                           (const uint4*)h->tc_weights, m.cout, 64, out, smp);
 }
 
-template <int METHOD>
-static int launch_lod_m(Handle* h, const DevGeom* gm, const DevChain& c, const DevSampler& smp, const MlpDev& m,
-                        const void* const* g0, const void* const* g1, int code_bits, void* out, int out_dtype,
-                        int precision, cudaStream_t st) {
-  if (precision == NIC_PREC_F16) {
-    if (out_dtype == NIC_DT_U8) return launch_lod_t<METHOD, 0, uint8_t>(h, gm, c, smp, m, g0, g1, code_bits, (uint8_t*)out, st);
-    return launch_lod_t<METHOD, 0, float>(h, gm, c, smp, m, g0, g1, code_bits, (float*)out, st);
-  }
-  if (out_dtype == NIC_DT_U8) return launch_lod_t<METHOD, 1, uint8_t>(h, gm, c, smp, m, g0, g1, code_bits, (uint8_t*)out, st);
-  return launch_lod_t<METHOD, 1, float>(h, gm, c, smp, m, g0, g1, code_bits, (float*)out, st);
+// f(IntC<METHOD>, IntC<FMT>, out as OutT*) for the call's method, precision and output dtype (uint8 or float).
+template <class F>
+static int dispatch_tc(int method, int precision, int out_dtype, void* out, F&& f) {
+  return dispatch_method_fmt(method, precision, [&](auto M, auto FMT) {
+    return out_dtype == NIC_DT_U8 ? f(M, FMT, (uint8_t*)out) : f(M, FMT, (float*)out);
+  });
+}
+
+int launch_decode_tc(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
+                     const long long* origins, void* out, int out_dtype, int precision, cudaStream_t st) {
+  if (g.N == 0) return NIC_OK;
+  if (!tc_shape_ok(g, m)) return NIC_ERR_UNSUPPORTED;
+  return dispatch_tc(g.method, precision, out_dtype, out, [&](auto M, auto FMT, auto* o) {
+    return launch_tc_t<M.value, FMT.value, 0>(h, g, m, g0, g1, code_bits, origins, o, st);
+  });
+}
+
+int launch_sample_tc(Handle* h, const DevGeom& gq, const DevSampler& smp, const MlpDev& m, const void* g0, const void* g1,
+                     int code_bits, void* out, int out_dtype, int precision, cudaStream_t st) {
+  if (gq.nblocks == 0) return NIC_OK;
+  if (!tc_shape_ok(gq, m)) return NIC_ERR_UNSUPPORTED;
+  DevGeom g = gq;                                   // one row per tap: queries x 2^dim rows
+  g.N = (long long)gq.nblocks << gq.dim;
+  if (g.N >= (1ll << 31) - TC_ROWS) return NIC_ERR_UNSUPPORTED;     // 32-bit row index in the kernel
+  return dispatch_tc(g.method, precision, out_dtype, out, [&](auto M, auto FMT, auto* o) {
+    return launch_tc_t<M.value, FMT.value, 1 << RowShape<M.value>::DIM>(h, g, m, g0, g1, code_bits, nullptr, o, st, smp);
+  });
 }
 
 int launch_sample_lod_tc(Handle* h, const DevGeom* gm, const DevChain& c, const DevSampler& smp, const MlpDev& m,
                          const void* const* g0, const void* const* g1, int code_bits, void* out, int out_dtype,
                          int precision, cudaStream_t st) {
   if (gm[0].nblocks == 0) return NIC_OK;
-  if (gm[0].C != 12 || gm[0].PE != 6 || m.hidden != 64 || m.cout > 16) return NIC_ERR_UNSUPPORTED;
+  if (!tc_shape_ok(gm[0], m)) return NIC_ERR_UNSUPPORTED;
   for (int i = 0; i < c.num_mips; ++i)               // one 64-entry LUT at step 1/4 serves the triangular PE of every mip
     if (gm[0].pe_kind == NIC_PE_TRIANGULAR && gm[i].step < 0.25f) return NIC_ERR_UNSUPPORTED;
-  switch (gm[0].method) {
-    case NIC_METHOD_2D: return launch_lod_m<NIC_METHOD_2D>(h, gm, c, smp, m, g0, g1, code_bits, out, out_dtype, precision, st);
-    case NIC_METHOD_3D: return launch_lod_m<NIC_METHOD_3D>(h, gm, c, smp, m, g0, g1, code_bits, out, out_dtype, precision, st);
-    case NIC_METHOD_3D_V2: return launch_lod_m<NIC_METHOD_3D_V2>(h, gm, c, smp, m, g0, g1, code_bits, out, out_dtype, precision, st);
-  }
-  return NIC_ERR_UNSUPPORTED;
+  return dispatch_tc(gm[0].method, precision, out_dtype, out, [&](auto M, auto FMT, auto* o) {
+    return launch_lod_t<M.value, FMT.value>(h, gm, c, smp, m, g0, g1, code_bits, o, st);
+  });
 }
 
 }  // namespace nic

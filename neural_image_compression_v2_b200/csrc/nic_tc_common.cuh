@@ -2,6 +2,7 @@
 // relayout shared by the tensor-core kernels (nic_tc.cu: decode, nic_train_tc.cu: training step).
 #pragma once
 #include <cstring>
+#include <type_traits>
 
 #include "nic_internal.cuh"
 
@@ -377,5 +378,74 @@ static inline int launch_relayout(Handle* h, const DevGeom& g, const void* src, 
   return (int)cudaGetLastError();
 }
 
+// ------------------------------------------------------------------------------------------------ launcher helpers
+// The shapes the tensor-core kernels are built for.
+static inline bool tc_shape_ok(const DevGeom& g, const MlpDev& m) {
+  return g.C == 12 && g.PE == 6 && m.hidden == 64 && m.cout <= 16;
+}
+
+// The scratch of the tensor-core tables: the weight images (64 KB of tc_weights) and shadow_bytes of tc_shadow.  A
+// reallocated buffer holds no tables.
+static inline int tc_scratch(Handle* h, size_t shadow_bytes) {
+  const size_t wb = h->tc_weights_bytes, sb = h->tc_shadow_bytes;
+  int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
+  if (rc == NIC_OK) rc = ensure_scratch(&h->tc_shadow, &h->tc_shadow_bytes, shadow_bytes);
+  if (h->tc_weights_bytes != wb || h->tc_shadow_bytes != sb) invalidate_prepared(h);
+  return rc;
+}
+
+// The 16-bit shadows of the grids of mips [0, n) in tc_shadow: G0 then G1 of each mip, each rounded up to 256 bytes.  A mip
+// whose grids (pointers and node counts) equal an earlier mip's shares that mip's shadows.
+struct ShadowLayout {
+  int n;
+  size_t off[NIC_MAX_MIPS][2];       // byte offsets of mip i's G0 and G1 shadows
+  bool own[NIC_MAX_MIPS];            // mip i's shadows are built from its own grids
+  size_t total;
+};
+static inline ShadowLayout shadow_layout(const DevGeom* gm, const void* const* g0, const void* const* g1, int n) {
+  ShadowLayout s;
+  s.n = n;
+  s.total = 0;
+  for (int i = 0; i < n; ++i) {
+    int first = i;
+    for (int j = 0; j < i && first == i; ++j)
+      if (g0[j] == g0[i] && g1[j] == g1[i] && !memcmp(gm[j].n0, gm[i].n0, sizeof(gm[i].n0)) &&
+          !memcmp(gm[j].n1, gm[i].n1, sizeof(gm[i].n1)))
+        first = j;
+    s.own[i] = first == i;
+    for (int k = 0; k < 2; ++k) {
+      s.off[i][k] = s.own[i] ? s.total : s.off[first][k];
+      if (s.own[i]) s.total += ((size_t)plane_size_host(k ? gm[i].n1 : gm[i].n0, gm[i].dim) * gm[i].C * 2 + 255) & ~(size_t)255;
+    }
+  }
+  return s;
+}
+template <int FMT>
+static inline int build_shadows(Handle* h, const ShadowLayout& s, const DevGeom* gm, const void* const* g0,
+                                const void* const* g1, int code_bits, cudaStream_t st) {
+  uint8_t* base = (uint8_t*)h->tc_shadow;
+  for (int i = 0; i < s.n; ++i) {
+    if (!s.own[i]) continue;
+    int rc = launch_relayout<FMT>(h, gm[i], g0[i], code_bits, gm[i].n0, (uint16_t*)(base + s.off[i][0]), st);
+    if (rc == NIC_OK) rc = launch_relayout<FMT>(h, gm[i], g1[i], code_bits, gm[i].n1, (uint16_t*)(base + s.off[i][1]), st);
+    if (rc != NIC_OK) return rc;
+  }
+  return NIC_OK;
+}
+
+// The one place where a call's method and precision become template parameters: f(IntC<METHOD>, IntC<FMT>) with FMT 0
+// for NIC_PREC_F16 and 1 (bf16) otherwise.
+template <int V>
+using IntC = std::integral_constant<int, V>;
+template <class F>
+static inline int dispatch_method_fmt(int method, int precision, F&& f) {
+  auto by_fmt = [&](auto M) { return precision == NIC_PREC_F16 ? f(M, IntC<0>{}) : f(M, IntC<1>{}); };
+  switch (method) {
+    case NIC_METHOD_2D: return by_fmt(IntC<NIC_METHOD_2D>{});
+    case NIC_METHOD_3D: return by_fmt(IntC<NIC_METHOD_3D>{});
+    case NIC_METHOD_3D_V2: return by_fmt(IntC<NIC_METHOD_3D_V2>{});
+  }
+  return NIC_ERR_UNSUPPORTED;
+}
 
 }  // namespace nic

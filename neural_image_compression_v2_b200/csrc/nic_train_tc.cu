@@ -1383,14 +1383,13 @@ static int launch_train_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const
                              int noise_bits, unsigned long long seed, unsigned long long step, float grad_scale, float* dg0,
                              float* dg1, float* loss_sum, float* out_save, cudaStream_t st) {
   const long long nodes0 = plane_size_host(g.n0, g.dim), nodes1 = plane_size_host(g.n1, g.dim);
-  const size_t b0 = ((size_t)nodes0 * g.C * 2 + 255) & ~(size_t)255, b1 = ((size_t)nodes1 * g.C * 2 + 255) & ~(size_t)255;
-  int rc = ensure_scratch(&h->tc_weights, &h->tc_weights_bytes, 64 * 1024);
+  const void* grids[2] = {g0, g1};
+  const ShadowLayout sl = shadow_layout(&g, &grids[0], &grids[1], 1);
+  int rc = tc_scratch(h, sl.total);
   if (rc) return rc;
-  rc = ensure_scratch(&h->tc_shadow, &h->tc_shadow_bytes, b0 + b1);
-  if (rc) return rc;
-  h->prepared.valid = 0;                       // the decode tables share this scratch
+  invalidate_prepared(h);                      // the decode tables share this scratch
   uint16_t* s0 = (uint16_t*)h->tc_shadow;
-  uint16_t* s1 = (uint16_t*)((uint8_t*)h->tc_shadow + b0);
+  uint16_t* s1 = (uint16_t*)((uint8_t*)h->tc_shadow + sl.off[0][1]);
   // channel-last fp32 gradient scratch (zero between steps: grad_relayout_add_kernel re-zeroes what it consumes)
   const size_t gb0 = (size_t)nodes0 * g.C * 4, gb1 = (size_t)nodes1 * g.C * 4;
   float *gs0 = nullptr, *gs1 = nullptr;
@@ -1430,10 +1429,8 @@ static int launch_train_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const
   sa.t1 = small ? nodes1 * g.C : 0;
   if (sa.t0 >= (1ll << 32) || sa.t1 >= (1ll << 32)) return NIC_ERR_UNSUPPORTED;        // 32-bit index math in the side kernels
   if (!small) {
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g0, 0, g.n0, s0, st);
-    if (e != cudaSuccess) return (int)e;
-    e = (cudaError_t)launch_relayout<FMT>(h, g, g1, 0, g.n1, s1, st);
-    if (e != cudaSuccess) return (int)e;
+    rc = build_shadows<FMT>(h, sl, &g, &grids[0], &grids[1], 0, st);
+    if (rc) return rc;
   }
   {
     const long long items = sa.t0 + sa.t1 + 64 * sa.K1 + 64 * 80 + 16 * 80;
@@ -1539,17 +1536,12 @@ int launch_train_tc(Handle* h, const DevGeom& g, const MlpDev& m, const MlpGradD
                     unsigned long long seed, unsigned long long step, float grad_scale, float* dg0, float* dg1,
                     float* loss_sum, float* out_save, int precision, cudaStream_t st) {
   if (g.N == 0) return NIC_OK;
-  const bool m2d = g.method == NIC_METHOD_2D, m3 = g.method == NIC_METHOD_3D, m3v2 = g.method == NIC_METHOD_3D_V2;
-  const int cin = m2d ? TrainShape<NIC_METHOD_2D>::CIN : (m3 ? TrainShape<NIC_METHOD_3D>::CIN : TrainShape<NIC_METHOD_3D_V2>::CIN);
-  if ((!m2d && !m3 && !m3v2) || g.C != 12 || g.PE != 6 || m.hidden != 64 || m.cout > 16 || m.cin != cin || !origins)
-    return NIC_ERR_UNSUPPORTED;
-#define NIC_TT_CALL(F, M)                                                                                               \
-  launch_train_tc_t<F, M>(h, g, m, gm, g0, g1, origins, targets, noise, noise_bits, seed, step, grad_scale, dg0, dg1, \
-                          loss_sum, out_save, st)
-  if (precision == NIC_PREC_F16)
-    return m2d ? NIC_TT_CALL(0, NIC_METHOD_2D) : (m3 ? NIC_TT_CALL(0, NIC_METHOD_3D) : NIC_TT_CALL(0, NIC_METHOD_3D_V2));
-  return m2d ? NIC_TT_CALL(1, NIC_METHOD_2D) : (m3 ? NIC_TT_CALL(1, NIC_METHOD_3D) : NIC_TT_CALL(1, NIC_METHOD_3D_V2));
-#undef NIC_TT_CALL
+  if (!tc_shape_ok(g, m) || !origins) return NIC_ERR_UNSUPPORTED;
+  return dispatch_method_fmt(g.method, precision, [&](auto M, auto FMT) -> int {
+    if (m.cin != TrainShape<M.value>::CIN) return NIC_ERR_UNSUPPORTED;
+    return launch_train_tc_t<FMT.value, M.value>(h, g, m, gm, g0, g1, origins, targets, noise, noise_bits, seed, step,
+                                                 grad_scale, dg0, dg1, loss_sum, out_save, st);
+  });
 }
 
 }  // namespace nic
