@@ -101,7 +101,7 @@ int64_t nic_launch_count(const NicHandle* h);
  * geometry qualifies for the aligned full-resolution 2-D fast path (both must give the same image). */
 /* NIC_OPT_REUSE_PREPARED = 1: the caller asserts that grids and decoder weights have not changed since the previous
  * tensor-core call on this handle (nic_decode, nic_decode_codes, nic_sample, nic_sample_codes, nic_sample_lod,
- * nic_sample_lod_codes); if that call prepared its private tables (shadow grids, per-node G1 rows, packed weights) for the
+ * nic_sample_lod_codes, nic_decode_mips, nic_decode_mips_codes); if that call prepared its private tables (shadow grids, per-node G1 rows, packed weights) for the
  * same kernel, pointers, node counts, steps, mip level, code width and precision, they are reused instead of being
  * rebuilt (decoding one frame as several row bands).  A training step on the handle discards them.  Off by default: every
  * call rebuilds from the caller's tensors. */
@@ -289,6 +289,28 @@ int nic_sample_lod(NicHandle* h, const NicMipChain* c, const float* coords, cons
 int nic_sample_lod_codes(NicHandle* h, const NicMipChain* c, int bits, const float* coords, const float* lod,
                          const float* ddx, const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision,
                          void* stream);
+
+/* ---- the whole mip chain in one call --------------------------------------------------------------------- */
+/* Decodes every mip 0 .. L = num_mips - 1 of a model (what a renderer uploads as a mipmapped texture; the reference's
+ * process_images decodes each mip in turn, image_compression.py:400).  c->geom[i] describes mip i exactly as nic_decode takes
+ * a whole-mip block: num_blocks = 1, block = c->extent[i], origin0 = 0, mip_level = i; c->g0[i] / c->g1[i] are its grids
+ * (fp32) or codes (uint8); address and align_corners are not used.  Every mip is validated as nic_decode validates a
+ * host-known block (NIC_ERR_BOUNDS); num_mips outside [1, NIC_MAX_MIPS], an extent < 1, geom[i].block != extent[i],
+ * num_blocks != 1, a non-zero origin, mip_level != i, NULL grids or mips that differ in method, channels, PE channels or PE
+ * kind give NIC_ERR_ARG.
+ * out is the concatenated chain in mip order: mip i starts at row sum_{j<i} texels_j and is laid out exactly as nic_decode
+ * writes that block, [Sx, Sy(, Sz), cout] with x slowest, in out_dtype (NIC_DT_F32, or NIC_DT_U8 = floor(v*255+.5)).
+ *   NIC_PREC_F32: every mip equals nic_decode of that mip at NIC_PREC_F32 bit for bit (the reference-exact kernel once per mip).
+ *   F16 / BF16: mip 0 is decoded exactly as nic_decode decodes it (bit for bit).  Mips 1 .. L are ONE tensor-core pass in
+ *   which the mip is a decoder input, as in nic_sample_lod: texel idx of mip i equals nic_sample_lod at its centre
+ *   ((idx + .5) / S per axis, align_corners 0) with lambda = i bit for bit, and may differ from a scalar nic_decode of that
+ *   mip by 16-bit rounding.  The pass's rows, sum_{i>=1} texels_i, must stay below 2^31 - 128, and with the triangular PE
+ *   every mip >= 1 needs step >= 1/4 (NIC_ERR_UNSUPPORTED otherwise). */
+int nic_decode_mips(NicHandle* h, const NicMipChain* c, const NicMlp* m, void* out, int out_dtype, int precision,
+                    void* stream);
+/* The same from the saved model's uint8 codes (as nic_decode_codes).  Tensor-core precisions only. */
+int nic_decode_mips_codes(NicHandle* h, const NicMipChain* c, int bits, const NicMlp* m, void* out, int out_dtype,
+                          int precision, void* stream);
 
 /* ---- applying a baked 3-D colour LUT to images ------------------------------------------------------------ */
 /* A colour LUT is decoded once (nic_decode / nic_decode_codes of the whole 3-D mip, fp32 out), packed into a table of 4-channel

@@ -109,6 +109,8 @@ SYMBOLS = {
                               _I, _P]),
     "nic_sample_lod": (_I, [_P, C.POINTER(NicMipChain), _P, _P, _P, _P, C.POINTER(NicMlp), _P, _I, _I, _P]),
     "nic_sample_lod_codes": (_I, [_P, C.POINTER(NicMipChain), _I, _P, _P, _P, _P, C.POINTER(NicMlp), _P, _I, _I, _P]),
+    "nic_decode_mips": (_I, [_P, C.POINTER(NicMipChain), C.POINTER(NicMlp), _P, _I, _I, _P]),
+    "nic_decode_mips_codes": (_I, [_P, C.POINTER(NicMipChain), _I, C.POINTER(NicMlp), _P, _I, _I, _P]),
     "nic_lut_pack": (_I, [_P, _P, C.POINTER(C.c_int32), _I, _P, _I, _P]),
     "nic_lut_apply": (_I, [_P, C.POINTER(NicLut), _P, _I, _L, _P, _I, _I, _P]),
     "nic_train_step": (_I, [_P, C.POINTER(NicGeom), _P, _P, _P, C.POINTER(NicMlp), _P, _P, _I, C.c_uint64, C.c_uint64,

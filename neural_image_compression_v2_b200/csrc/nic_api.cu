@@ -487,22 +487,38 @@ int nic_sample_codes(NicHandle* h, const NicGeom* g, const uint8_t* codes0, cons
   return sample_impl(h, g, codes0, codes1, true, bits, coords, s, m, out, out_dtype, precision, stream);
 }
 
-// Geometry of a per-query-LOD call: every mip validated as flatten_sampler validates one, the chain's shared description,
-// and exactly one LOD source.
-static int flatten_chain(NicHandle* h, const NicMipChain* c, const float* coords, const float* lod, const float* ddx,
-                         const float* ddy, DevGeom* d, DevChain* dc, DevSampler* ds, const char* who) {
+// Mip i of a nic_decode_mips chain: one block that covers the whole mip (num_blocks 1, block = extent, origin 0), validated as
+// nic_decode validates a host-known block.
+static int flatten_whole_mip(NicHandle* h, const NicGeom* g, const int32_t* extent, int i, DevGeom* d, const char* who) {
+  const int dim = g->method == NIC_METHOD_2D ? 2 : 3;
+  if (g->num_blocks != 1) return fail(h, NIC_ERR_ARG, "%s: geom[%d].num_blocks is %d (one whole-mip block)", who, i, g->num_blocks);
+  for (int a = 0; a < dim; ++a) {
+    if (extent[a] < 1) return fail(h, NIC_ERR_ARG, "%s: extent %d of mip %d on axis %d", who, extent[a], i, a);
+    if (g->block[a] != extent[a] || g->origin0[a] != 0)
+      return fail(h, NIC_ERR_ARG, "%s: geom[%d] must be the whole mip (block = extent, origin 0) on axis %d", who, i, a);
+  }
+  return flatten_geom(h, g, false, d);
+}
+
+// Every mip of a chain, validated as flatten_sampler validates one (whole false: a sampling call's Q queries) or as
+// flatten_whole_mip does (whole true: nic_decode_mips), and the chain's shared description: method, channels and PE.
+static int flatten_mips(NicHandle* h, const NicMipChain* c, const float* coords, bool whole, DevGeom* d, DevChain* dc,
+                        DevSampler* ds, const char* who) {
   if (!c) return fail(h, NIC_ERR_ARG, "%s: chain is NULL", who);
   if (c->num_mips < 1 || c->num_mips > NIC_MAX_MIPS) return fail(h, NIC_ERR_ARG, "%s: num_mips %d (1..%d)", who, c->num_mips, NIC_MAX_MIPS);
-  if (!((lod && !ddx && !ddy) || (!lod && ddx && ddy)))
-    return fail(h, NIC_ERR_ARG, "%s: give exactly one of lod or the pair ddx / ddy", who);
   memset(dc, 0, sizeof(*dc));
   for (int i = 0; i < c->num_mips; ++i) {
-    NicSampler s;
-    memset(&s, 0, sizeof(s));
-    s.address = c->address;
-    s.align_corners = c->align_corners;
-    for (int a = 0; a < 3; ++a) s.extent[a] = c->extent[i][a];
-    int rc = flatten_sampler(h, &c->geom[i], &s, coords, &d[i], ds, who);
+    int rc;
+    if (whole) {
+      rc = flatten_whole_mip(h, &c->geom[i], c->extent[i], i, &d[i], who);
+    } else {
+      NicSampler s;
+      memset(&s, 0, sizeof(s));
+      s.address = c->address;
+      s.align_corners = c->align_corners;
+      for (int a = 0; a < 3; ++a) s.extent[a] = c->extent[i][a];
+      rc = flatten_sampler(h, &c->geom[i], &s, coords, &d[i], ds, who);
+    }
     if (rc) return rc;
     if (c->geom[i].mip_level != i) return fail(h, NIC_ERR_ARG, "%s: geom[%d].mip_level is %d", who, i, c->geom[i].mip_level);
     if (!c->g0[i] || !c->g1[i]) return fail(h, NIC_ERR_ARG, "%s: grids of mip %d are NULL", who, i);
@@ -510,18 +526,29 @@ static int flatten_chain(NicHandle* h, const NicMipChain* c, const float* coords
         d[i].nblocks != d[0].nblocks || memcmp(d[i].pe_div, d[0].pe_div, sizeof(d[0].pe_div)) != 0)
       return fail(h, NIC_ERR_ARG, "%s: mip %d differs from mip 0 in method, channels, PE or query count", who, i);
     DevMip& mp = dc->mip[i];
-    for (int a = 0; a < 3; ++a) { mp.n0[a] = d[i].n0[a]; mp.n1[a] = d[i].n1[a]; mp.S[a] = ds->S[a]; }
+    for (int a = 0; a < 3; ++a) { mp.n0[a] = d[i].n0[a]; mp.n1[a] = d[i].n1[a]; mp.S[a] = a < d[i].dim ? c->extent[i][a] : 1; }
     mp.step = d[i].step;
     mp.interp = d[i].interp;
     const int k = c->geom[i].step_log2 + 2;
     mp.lut_shift = k < 0 ? 0 : (k > 6 ? 6 : k);
   }
+  dc->num_mips = c->num_mips;
+  dc->dim = d[0].dim;
+  return NIC_OK;
+}
+
+// Geometry of a per-query-LOD call: every mip validated as flatten_sampler validates one, the chain's shared description,
+// and exactly one LOD source.
+static int flatten_chain(NicHandle* h, const NicMipChain* c, const float* coords, const float* lod, const float* ddx,
+                         const float* ddy, DevGeom* d, DevChain* dc, DevSampler* ds, const char* who) {
+  if (!((lod && !ddx && !ddy) || (!lod && ddx && ddy)))
+    return fail(h, NIC_ERR_ARG, "%s: give exactly one of lod or the pair ddx / ddy", who);
+  int rc = flatten_mips(h, c, coords, false, d, dc, ds, who);
+  if (rc) return rc;
   if (((long long)d[0].nblocks << (d[0].dim + 1)) >= (1ll << 31) - 128)
     return fail(h, NIC_ERR_UNSUPPORTED, "%s: %d queries x %d taps reach 2^31 - 128 rows; split the batch", who, d[0].nblocks,
                 2 << d[0].dim);
   ds->S[0] = ds->S[1] = ds->S[2] = 1;                // per mip: DevMip::S
-  dc->num_mips = c->num_mips;
-  dc->dim = d[0].dim;
   dc->address = ds->address;
   dc->align_corners = ds->align_corners;
   dc->lod = lod;
@@ -563,6 +590,42 @@ int nic_sample_lod_codes(NicHandle* h, const NicMipChain* c, int bits, const flo
                          const float* ddx, const float* ddy, const NicMlp* m, void* out, int out_dtype, int precision,
                          void* stream) {
   return sample_lod_impl(h, c, true, bits, coords, lod, ddx, ddy, m, out, out_dtype, precision, stream);
+}
+
+static int decode_mips_impl(NicHandle* h, const NicMipChain* c, bool codes, int bits, const NicMlp* m, void* out, int out_dtype,
+                            int precision, void* stream) {
+  NIC_ENTER(h);
+  const char* who = codes ? "nic_decode_mips_codes" : "nic_decode_mips";
+  DevGeom d[NIC_MAX_MIPS];
+  DevChain dc;
+  int rc = flatten_mips(h, c, nullptr, true, d, &dc, nullptr, who);
+  if (rc) return rc;
+  MlpDev md;
+  rc = flatten_mlp(h, m, &md, d[0].cin);
+  if (rc) return rc;
+  rc = check_call(h, codes, bits, !out, "out is NULL", out_dtype, precision, who);
+  if (rc) return rc;
+  if (precision == NIC_PREC_F32) {                   // the reference-exact kernel once per mip, into its slice of out
+    uint8_t* o = (uint8_t*)out;
+    for (int i = 0; i < c->num_mips; ++i) {
+      rc = launch_mlp_forward_f32(h, &d[i], md, (const float*)c->g0[i], (const float*)c->g1[i], nullptr, nullptr, 0, d[i].N, o,
+                                  out_dtype, nullptr, nullptr, st);
+      if (rc) return cuda_fail(h, rc, "nic_decode_mips(f32)");
+      o += (size_t)d[i].N * md.cout * (out_dtype == NIC_DT_U8 ? 1 : sizeof(float));
+    }
+    return NIC_OK;
+  }
+  return cuda_fail(h, launch_decode_mips_tc(h, d, dc, md, c->g0, c->g1, bits, out, out_dtype, precision, st),
+                   codes ? who : "nic_decode_mips(tensor core)");
+}
+
+int nic_decode_mips(NicHandle* h, const NicMipChain* c, const NicMlp* m, void* out, int out_dtype, int precision, void* stream) {
+  return decode_mips_impl(h, c, false, 0, m, out, out_dtype, precision, stream);
+}
+
+int nic_decode_mips_codes(NicHandle* h, const NicMipChain* c, int bits, const NicMlp* m, void* out, int out_dtype,
+                          int precision, void* stream) {
+  return decode_mips_impl(h, c, true, bits, m, out, out_dtype, precision, stream);
 }
 
 // Texels of a LUT extent: NIC_ERR_ARG for an extent < 1, NIC_ERR_UNSUPPORTED from 2^31 texels on (int texel indices).

@@ -238,6 +238,13 @@ struct DevChain {
   float E0[3];            // extent of mip 0 (derivatives are in normalised units)
   DevMip mip[NIC_MAX_MIPS];
 };
+// nic_decode_mips (tensor core): the chain table of the dense pass over mips 1 .. L and the pass's first row of each mip
+// (row0[0] = row0[1] = 0: mip 0 has no rows in the pass; 0xffffffff past the last mip).  Row n belongs to the mip with the
+// largest row0 <= n.
+struct DevMipRows {
+  DevChain c;
+  unsigned row0[NIC_MAX_MIPS];
+};
 
 // lambda of query q clamped to [0, L] (nic.h nic_sample_lod; every step one fp32 operation).  fmaxf maps NaN and the -inf
 // of zero derivatives to 0.

@@ -47,7 +47,8 @@ struct Handle {
   size_t data_scratch_bytes;
   void* sample_scratch;      // nic_sample.cu: tap texels, tap weights and tap outputs of the fp32 sampling arm
   size_t sample_scratch_bytes;
-  void* lod_chain;           // nic_sample_lod (tensor core): device copy of the call's DevChain
+  void* lod_chain;           // nic_sample_lod / nic_decode_mips (tensor core): device copy of the call's chain table
+                             // (sizeof(DevMipRows) bytes)
   int gelu_poly;             // NIC_OPT_GELU_POLY: -1 = tuned default, 0..8 = activation pairs (of 8) on the polynomial GELU
   struct PreparedKey {       // what the tables in tc_weights / tc_shadow were last built from (compared with memcmp)
     int kind;                // PreparedKind: the kernel they were built for (PREP_NONE: nothing valid)
@@ -263,6 +264,9 @@ int launch_sample_lod_tc(Handle* h, const DevGeom* g, const DevChain& c, const D
                          int precision, cudaStream_t st);
 int launch_sample_lod_f32(Handle* h, const DevGeom* g, const DevChain& c, const DevSampler& smp, const MlpDev& m,
                           const float* const* g0, const float* const* g1, void* out, int out_dtype, cudaStream_t st);
+// nic_decode_mips / nic_decode_mips_codes (tensor core): g[i] describes mip i as one whole-mip block; c the chain.
+int launch_decode_mips_tc(Handle* h, const DevGeom* g, const DevChain& c, const MlpDev& m, const void* const* g0,
+                          const void* const* g1, int code_bits, void* out, int out_dtype, int precision, cudaStream_t st);
 // nic_lut_pack / nic_lut_apply (nic_lut.cu): arguments validated by nic_api.cu.
 int launch_lut_pack(Handle* h, const float* dense, long long texels, int cout, void* table, int table_dtype, cudaStream_t st);
 int launch_lut_apply(Handle* h, const NicLut& lut, const void* src, int src_dtype, long long pixels, void* dst, int dst_dtype,

@@ -599,7 +599,12 @@ __global__ void __launch_bounds__(WS_THREADS, 1) decode_tc2d_ws_kernel(DevGeom g
 // points at and the CTA copies to shared memory (lanes of a warp read different mips).  The mip is a decoder input
 // (column CIN - 1; the bias moves to column CIN), one PE LUT built at step 1/4 serves every mip, and the two halves of a
 // query blend after their butterflies.
+// TAPS = TAPS_MIPS (nic_decode_mips): the dense chain.  Row n is a texel of the mip whose first row (DevMipRows::row0, in
+// shared memory behind the chain table) is the largest one <= n, at index n - row0 inside that mip, x slowest.  Everything
+// that varies by mip comes from the chain table as in the per-query-LOD mode, and so do the mip column and the step-1/4 PE
+// LUT; the epilogue is TAPS = 0's: each row stores its own output row.  Tiles may straddle mips, so small mips share tiles.
 constexpr int GW_GROUP = 128;
+constexpr int TAPS_MIPS = -1;
 
 // NGT / LUTCAP: groups per CTA and capacity of the positional-encoding LUT.  The defaults (8 groups, or 5 for method 3's
 // 32 KB operand buffers, 256 LUT entries) always fit; with a 64-entry LUT (step >= 1/4: every full-resolution decode) a
@@ -617,9 +622,12 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
   constexpr int OFF_LUT = W1_BYTES + W2_BYTES + W3_BYTES, OFF_ONE = OFF_LUT + LUTCAP * 16, OFF_ACT = OFF_ONE + 2 * KG;
   constexpr int ACT_BYTES = (KX / 8) * KG, OFF_BAR = OFF_ACT + NG * ACT_BYTES;
   constexpr bool LODQ = TAPS == (2 << S::DIM);
+  constexpr bool DENSE = TAPS == TAPS_MIPS;
+  constexpr bool CHAIN = LODQ || DENSE;              // per-row mip from the chain table
   constexpr int TQ = LODQ ? TAPS / 2 : TAPS;         // taps of one mip
   extern __shared__ __align__(128) uint8_t smem_raw[];
-  const DevChain* sChain = reinterpret_cast<const DevChain*>(smem_raw + OFF_BAR + 256);     // LODQ only
+  const DevChain* sChain = reinterpret_cast<const DevChain*>(smem_raw + OFF_BAR + 256);     // CHAIN only
+  const unsigned* sRow0 = reinterpret_cast<const DevMipRows*>(sChain)->row0;                // DENSE only
   uint8_t* sW1 = smem_raw;
   uint8_t* sW2 = sW1 + W1_BYTES;
   uint8_t* sW3 = sW2 + W2_BYTES;
@@ -639,7 +647,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
     uint4* dst = reinterpret_cast<uint4*>(smem_raw);
     for (int i = tid; i < OFF_LUT / 16; i += THREADS) dst[i] = __ldg(wimg + i);
     for (int i = tid; i < lut_n; i += THREADS) {
-      float u1 = __fmul_rn(__fmul_rn((float)i, LODQ ? 0.25f : g.step), 0.5f);
+      float u1 = __fmul_rn(__fmul_rn((float)i, CHAIN ? 0.25f : g.step), 0.5f);
       uint4 e;
       auto v0 = P::pack(pe_triangular(u1, 0, 6), pe_triangular(u1, 1, 6));
       auto v1 = P::pack(pe_triangular(u1, 2, 6), pe_triangular(u1, 3, 6));
@@ -650,10 +658,10 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
       e.w = 0u;
       sLut[i] = e;
     }
-    if constexpr (LODQ) {
+    if constexpr (CHAIN) {
       const uint32_t* src = reinterpret_cast<const uint32_t*>(origins);
       uint32_t* cdst = reinterpret_cast<uint32_t*>(smem_raw + OFF_BAR + 256);
-      for (int i = tid; i < (int)(sizeof(DevChain) / 4); i += THREADS) cdst[i] = __ldg(src + i);
+      for (int i = tid; i < (int)((LODQ ? sizeof(DevChain) : sizeof(DevMipRows)) / 4); i += THREADS) cdst[i] = __ldg(src + i);
     }
     if (slot == 0) {
       auto one = P::pack(1.0f, 0.0f);
@@ -696,7 +704,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
     const bool live = n < (unsigned)g.N;
     float tap_w = 0.f;                               // TAPS > 0: this row's filter weight (0 on dead rows)
     float lod_t = 0.f;                               // LODQ: the query's weight of mip m + 1
-    int row_mip = 0;                                 // LODQ: this row's mip and its entry of the chain table
+    int row_mip = 0;                                 // CHAIN: this row's mip and its entry of the chain table
     const DevMip* mp = nullptr;
     // ------------------------------------------------------------------------------------ gather -> operand buffer
     {
@@ -721,17 +729,30 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
           const float w = sample_tap(smp, S::DIM, u, row % TAPS, t.p);
           tap_w = live ? w : 0.f;
         }
+      } else if constexpr (DENSE) {
+        const unsigned r = live ? n : (unsigned)g.N - 1;
+#pragma unroll
+        for (int i = 1; i < NIC_MAX_MIPS; ++i) row_mip += r >= sRow0[i];
+        mp = &sChain->mip[row_mip];
+        const unsigned idx = r - sRow0[row_mip];     // x slowest: ((ix * Sy) + iy) * Sz + iz
+        const unsigned yz = (unsigned)mp->S[1] * (unsigned)mp->S[2];
+        const unsigned ix = idx / yz, r2 = idx - ix * yz;
+        const unsigned iy = S::DIM == 3 ? r2 / (unsigned)mp->S[2] : r2;
+        t.b = 0;
+        t.p[0] = (int)ix;
+        t.p[1] = (int)iy;
+        t.p[2] = S::DIM == 3 ? (int)(r2 - iy * (unsigned)mp->S[2]) : 0;
       } else {
         t = texel_of_fast(g, live ? n : (unsigned)g.N - 1, origins);
       }
-      const int* n0 = LODQ ? mp->n0 : g.n0;
-      const int* n1 = LODQ ? mp->n1 : g.n1;
-      const uint2* s0 = LODQ ? sg.s0 + mp->s0 : sg.s0;
-      const uint2* s1 = LODQ ? sg.s1 + mp->s1 : sg.s1;
+      const int* n0 = CHAIN ? mp->n0 : g.n0;
+      const int* n1 = CHAIN ? mp->n1 : g.n1;
+      const uint2* s0 = CHAIN ? sg.s0 + mp->s0 : sg.s0;
+      const uint2* s1 = CHAIN ? sg.s1 + mp->s1 : sg.s1;
       AxisCoord ax[3];
 #pragma unroll
       for (int a = 0; a < 3; ++a) {
-        ax[a] = axis_coord(t.p[a], LODQ ? mp->step : g.step);
+        ax[a] = axis_coord(t.p[a], CHAIN ? mp->step : g.step);
         ax[a].i0 = clampi(ax[a].i0, 0, n0[a] - 2 < 0 ? 0 : n0[a] - 2);
         ax[a].i1 = clampi(ax[a].i1, 0, n1[a] - 2 < 0 ? 0 : n1[a] - 2);
       }
@@ -751,7 +772,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
         const uint2* node = s1 + 3 * node_lin(n1, S::DIM, ax[0].i1 + d[2], ax[1].i1 + d[1], ax[2].i1 + dz);
         float f[3];
         g1_factors(g, j, ax, f);
-        if constexpr (LODQ) {
+        if constexpr (CHAIN) {
           if (!mp->interp) f[0] = f[1] = f[2] = 1.0f;
         }
         float w = f[0] * f[1];
@@ -777,7 +798,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
 #pragma unroll
       for (int a = 0; a < S::DIM; ++a) {
         if (g.pe_kind == NIC_PE_TRIANGULAR) {
-          uint4 e = sLut[LODQ ? ((t.p[a] << mp->lut_shift) & 63) : (t.p[a] & lut_mask)];
+          uint4 e = sLut[CHAIN ? ((t.p[a] << mp->lut_shift) & 63) : (t.p[a] & lut_mask)];
           tail[3 * a] = e.x;
           tail[3 * a + 1] = e.y;
           tail[3 * a + 2] = e.z;
@@ -791,7 +812,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
         }
       }
       {
-        auto one = P::pack(LODQ ? (float)row_mip : 1.0f, LODQ ? 1.0f : 0.0f);     // LODQ: [... | pe | mip | 1]
+        auto one = P::pack(CHAIN ? (float)row_mip : 1.0f, CHAIN ? 1.0f : 0.0f);   // CHAIN: [... | pe | mip | 1]
         tail[(S::CIN - 1 - T0) / 2] = *reinterpret_cast<uint32_t*>(&one);
       }
 #pragma unroll
@@ -1206,13 +1227,13 @@ static int pe_lut_len(const DevGeom& g) {
 }
 
 // Dynamic shared memory of decode_tc_gws_kernel with NG groups and a LUTCAP-entry LUT: weight images, LUT, ones block,
-// operand buffers, barriers, and behind them the chain table of a per-query-LOD launch.  The code-resident kernel has the
-// same layout with CQ_NG groups, followed by its two grids.
+// operand buffers, barriers, and behind them the `table` bytes of the chain table of a per-query-LOD (DevChain) or dense-chain
+// (DevMipRows) launch.  The code-resident kernel has the same layout with CQ_NG groups, followed by its two grids.
 template <int METHOD>
-constexpr int gws_smem(int ng, int lutcap, bool chain = false) {
+constexpr int gws_smem(int ng, int lutcap, size_t table = 0) {
   using S = RowShape<METHOD>;
   return b_image_bytes(64, S::KX) + b_image_bytes(64, TC_K2) + b_image_bytes(16, TC_K2) + lutcap * 16 + 2 * 2048 +
-         ng * (S::KX / 8) * 2048 + 256 + (chain ? (int)((sizeof(DevChain) + 15) & ~15) : 0);
+         ng * (S::KX / 8) * 2048 + 256 + (int)((table + 15) & ~(size_t)15);
 }
 
 // One launch of a persistent tensor-core kernel: at most one CTA per SM for `units` work units (tiles or tile groups).
@@ -1276,11 +1297,17 @@ static int launch_codes_smem(Handle* h, const DevGeom& g, const MlpDev& m, const
                            origins, (const uint4*)h->tc_weights, m.cout, lut_n, out);
 }
 
+// Bytes of tc_shadow the fast path's tables take: the G0 shadow (b0, rounded to 256 bytes), then R (b1).
+static void fast2d_table_bytes(const DevGeom& g, size_t* b0, size_t* b1) {
+  *b0 = ((size_t)plane_size_host(g.n0, 2) * g.C * 2 + 255) & ~(size_t)255;
+  *b1 = (size_t)plane_size_host(g.n1, 2) * 128;
+}
+
 template <int FMT, typename OutT>
 static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
                          OutT* out, cudaStream_t st) {
-  const long long nodes0 = plane_size_host(g.n0, 2), nodes1 = plane_size_host(g.n1, 2);
-  const size_t b0 = ((size_t)nodes0 * g.C * 2 + 255) & ~(size_t)255, b1 = (size_t)nodes1 * 128;     // the G0 shadow, then R
+  size_t b0, b1;
+  fast2d_table_bytes(g, &b0, &b1);
   int rc = tc_scratch(h, b0 + b1);
   if (rc) return rc;
   uint16_t* s0 = (uint16_t*)h->tc_shadow;
@@ -1374,6 +1401,30 @@ static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const void*
                            (const uint4*)h->tc_weights, m.cout, lut_n, out, smp);
 }
 
+// The chain table of a per-query-LOD or dense-chain launch (`bytes` of it) in the handle's device copy, on the call's stream.
+static int upload_chain_table(Handle* h, const void* table, size_t bytes, cudaStream_t st) {
+  if (!h->lod_chain && cudaMalloc(&h->lod_chain, sizeof(DevMipRows)) != cudaSuccess) {
+    h->lod_chain = nullptr;
+    return NIC_ERR_SCRATCH;
+  }
+  return (int)cudaMemcpyAsync(h->lod_chain, table, bytes, cudaMemcpyHostToDevice, st);
+}
+
+// The tables of a chain pass over mips gm[0, n) (per-query LOD or dense chain), keyed by the whole chain: the shadow grids of
+// every pyramid level those mips reach (layout `sl`, which tc_scratch already holds) and the W1 image with the mip column.
+template <int METHOD, int FMT>
+static int prepare_chain(Handle* h, const ShadowLayout& sl, const DevGeom* gm, const void* const* g0, const void* const* g1,
+                         int n, int code_bits, int npoly, const MlpDev& m, cudaStream_t st) {
+  return prepare_tables(h, make_key(PREP_CHAIN, FMT, code_bits, npoly, m, gm, g0, g1, n), [&] {
+    const int e = build_shadows<FMT>(h, sl, gm, g0, g1, code_bits, st);
+    if (e) return e;
+    pack_weights_kernel<FMT><<<16, 256, 0, st>>>(m, 0.0f, RowShape<METHOD>::KX, (uint16_t*)h->tc_weights, npoly);
+    pack_lod_columns_kernel<FMT><<<1, 64, 0, st>>>(m, (uint16_t*)h->tc_weights);
+    h->launches += 2;
+    return (int)cudaGetLastError();
+  });
+}
+
 // Per-query LOD: the shadow grids of every pyramid level the chain reaches (built once, keyed by the whole chain), the
 // W1 image with the mip column, the chain table in device memory, one pass of the general kernel with 2 * 2^D rows a query.
 template <int METHOD, int FMT, typename OutT>
@@ -1391,26 +1442,15 @@ static int launch_lod_t(Handle* h, const DevGeom* gm, DevChain c, const DevSampl
   }
   const int npoly = resolve_npoly(h, FMT);
   if (npoly != 0 && npoly != 3) return NIC_ERR_UNSUPPORTED;
-  rc = prepare_tables(h, make_key(PREP_CHAIN, FMT, code_bits, npoly, m, gm, g0, g1, c.num_mips), [&] {
-    const int e = build_shadows<FMT>(h, sl, gm, g0, g1, code_bits, st);
-    if (e) return e;
-    pack_weights_kernel<FMT><<<16, 256, 0, st>>>(m, 0.0f, S::KX, (uint16_t*)h->tc_weights, npoly);
-    pack_lod_columns_kernel<FMT><<<1, 64, 0, st>>>(m, (uint16_t*)h->tc_weights);
-    h->launches += 2;
-    return (int)cudaGetLastError();
-  });
+  rc = prepare_chain<METHOD, FMT>(h, sl, gm, g0, g1, c.num_mips, code_bits, npoly, m, st);
   if (rc) return rc;
-  if (!h->lod_chain && cudaMalloc(&h->lod_chain, sizeof(DevChain)) != cudaSuccess) {
-    h->lod_chain = nullptr;
-    return NIC_ERR_SCRATCH;
-  }
-  cudaError_t e = cudaMemcpyAsync(h->lod_chain, &c, sizeof(DevChain), cudaMemcpyHostToDevice, st);
-  if (e != cudaSuccess) return (int)e;
+  rc = upload_chain_table(h, &c, sizeof(DevChain), st);
+  if (rc) return rc;
   DevGeom g = gm[0];                                  // method, PE, coordinates; the rest is per row from the chain
   g.N = (long long)g.nblocks * TAPS;
   g.interp = 1;                                       // (g1_factors computes the weights; rows of step-2 mips drop them)
   const ShadowGeom sg = {(const uint2*)h->tc_shadow, (const uint2*)h->tc_shadow};
-  constexpr int NG = gws_groups(S::KX, 0), GSMEM = gws_smem<METHOD>(NG, TC_LUT_MAX, true);
+  constexpr int NG = gws_groups(S::KX, 0), GSMEM = gws_smem<METHOD>(NG, TC_LUT_MAX, sizeof(DevChain));
   static_assert(GSMEM <= 227 * 1024, "shared memory budget");
   void (*kern)(DevGeom, ShadowGeom, const long long*, const uint4*, int, int, OutT*, DevSampler) =
       npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 0, TC_LUT_MAX, TAPS>
@@ -1418,6 +1458,58 @@ static int launch_lod_t(Handle* h, const DevGeom* gm, DevChain c, const DevSampl
   const long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS;
   return launch_persistent(h, kern, (ntiles + NG - 1) / NG, NG * GW_GROUP, GSMEM, st, g, sg, (const long long*)h->lod_chain,
                            (const uint4*)h->tc_weights, m.cout, 64, out, smp);
+}
+
+// Whole mip chain: mip 0 through the single-mip path (launch_tc_t: it equals nic_decode), then mips 1 .. L in ONE pass of
+// the general kernel in its dense-chain mode, on the tables of launch_lod_t built for those mips.  tc_scratch is sized for
+// the larger of the two passes before either builds: growing it between them would cudaFree, which synchronises the device.
+template <int METHOD, int FMT, typename OutT>
+static int launch_mips_t(Handle* h, const DevGeom* gm, const DevChain& c, const MlpDev& m, const void* const* g0,
+                         const void* const* g1, int code_bits, OutT* out, cudaStream_t st) {
+  using S = RowShape<METHOD>;
+  const int L = c.num_mips - 1;
+  const ShadowLayout sl = shadow_layout(gm + 1, g0 + 1, g1 + 1, L);
+  if (sl.total / 8 >= (1ull << 32)) return NIC_ERR_UNSUPPORTED;            // 32-bit shadow offsets in the chain table
+  const int npoly = resolve_npoly(h, FMT);
+  if (L > 0 && npoly != 0 && npoly != 3) return NIC_ERR_UNSUPPORTED;
+  size_t need0;                                       // what launch_tc_t takes for mip 0 (it never takes the code-resident path)
+  if (METHOD == NIC_METHOD_2D && fast2d_eligible(gm[0], nullptr) && !h->disable_fast2d) {
+    size_t b0, b1;
+    fast2d_table_bytes(gm[0], &b0, &b1);
+    need0 = b0 + b1;
+  } else {
+    need0 = shadow_layout(gm, g0, g1, 1).total;
+  }
+  int rc = tc_scratch(h, need0 > sl.total ? need0 : sl.total);
+  if (rc) return rc;
+  rc = launch_tc_t<METHOD, FMT, 0>(h, gm[0], m, g0[0], g1[0], code_bits, nullptr, out, st);
+  if (rc || L == 0) return rc;
+  rc = prepare_chain<METHOD, FMT>(h, sl, gm + 1, g0 + 1, g1 + 1, L, code_bits, npoly, m, st);
+  if (rc) return rc;
+  DevMipRows t;
+  t.c = c;
+  long long rows = 0;                                 // < 2^31 - TC_ROWS (launch_decode_mips_tc)
+  for (int i = 0; i < NIC_MAX_MIPS; ++i) {
+    t.row0[i] = i <= L ? (unsigned)rows : 0xffffffffu;
+    if (i < 1 || i > L) continue;
+    rows += gm[i].N;
+    t.c.mip[i].s0 = (unsigned)(sl.off[i - 1][0] / 8);
+    t.c.mip[i].s1 = (unsigned)(sl.off[i - 1][1] / 8);
+  }
+  rc = upload_chain_table(h, &t, sizeof(t), st);
+  if (rc) return rc;
+  DevGeom g = gm[1];                                  // method and PE; the rest is per row from the chain
+  g.N = rows;
+  g.interp = 1;                                       // (g1_factors computes the weights; rows of step-2 mips drop them)
+  const ShadowGeom sg = {(const uint2*)h->tc_shadow, (const uint2*)h->tc_shadow};
+  constexpr int NG = gws_groups(S::KX, 0), GSMEM = gws_smem<METHOD>(NG, TC_LUT_MAX, sizeof(DevMipRows));
+  static_assert(GSMEM <= 227 * 1024, "shared memory budget");
+  void (*kern)(DevGeom, ShadowGeom, const long long*, const uint4*, int, int, OutT*, DevSampler) =
+      npoly == 0 ? decode_tc_gws_kernel<METHOD, FMT, OutT, 0, 0, TC_LUT_MAX, TAPS_MIPS>
+                 : decode_tc_gws_kernel<METHOD, FMT, OutT, 3, 0, TC_LUT_MAX, TAPS_MIPS>;
+  const long long ntiles = (g.N + TC_ROWS - 1) / TC_ROWS;
+  return launch_persistent(h, kern, (ntiles + NG - 1) / NG, NG * GW_GROUP, GSMEM, st, g, sg, (const long long*)h->lod_chain,
+                           (const uint4*)h->tc_weights, m.cout, 64, out + (size_t)gm[0].N * m.cout, DevSampler{});
 }
 
 // f(IntC<METHOD>, IntC<FMT>, out as OutT*) for the call's method, precision and output dtype (uint8 or float).
@@ -1458,6 +1550,20 @@ int launch_sample_lod_tc(Handle* h, const DevGeom* gm, const DevChain& c, const 
     if (gm[0].pe_kind == NIC_PE_TRIANGULAR && gm[i].step < 0.25f) return NIC_ERR_UNSUPPORTED;
   return dispatch_tc(gm[0].method, precision, out_dtype, out, [&](auto M, auto FMT, auto* o) {
     return launch_lod_t<M.value, FMT.value>(h, gm, c, smp, m, g0, g1, code_bits, o, st);
+  });
+}
+
+int launch_decode_mips_tc(Handle* h, const DevGeom* gm, const DevChain& c, const MlpDev& m, const void* const* g0,
+                          const void* const* g1, int code_bits, void* out, int out_dtype, int precision, cudaStream_t st) {
+  if (!tc_shape_ok(gm[0], m)) return NIC_ERR_UNSUPPORTED;
+  long long rows = 0;                                 // of the chain pass: mips 1 .. L
+  for (int i = 1; i < c.num_mips; ++i) {              // one 64-entry LUT at step 1/4 serves the triangular PE of every mip
+    if (gm[0].pe_kind == NIC_PE_TRIANGULAR && gm[i].step < 0.25f) return NIC_ERR_UNSUPPORTED;
+    rows += gm[i].N;
+  }
+  if (rows >= (1ll << 31) - TC_ROWS) return NIC_ERR_UNSUPPORTED;     // 32-bit row index in the kernel
+  return dispatch_tc(gm[0].method, precision, out_dtype, out, [&](auto M, auto FMT, auto* o) {
+    return launch_mips_t<M.value, FMT.value>(h, gm, c, m, g0, g1, code_bits, o, st);
   });
 }
 

@@ -364,11 +364,13 @@ def _lod_inputs(lod, grad, coords, dim):
 
 
 def _mip_chain(fp_like, q, address, align_corners, method, table):
-    """NicMipChain of mips 0 .. min(MAX_MIP_LEVEL, max(table)), each at its default extent IMAGE_SIZE >> mip."""
+    """NicMipChain of mips 0 .. min(MAX_MIP_LEVEL, max(table)), each at its default extent IMAGE_SIZE >> mip: q one-texel
+    queries per mip (nic_sample_lod), or with q None one block that covers the whole mip (nic_decode_mips)."""
     dim = 2 if method == L.METHOD_2D else 3
     last = min(var2.MAX_MIP_LEVEL, max(table))
     if last + 1 > L.MAX_MIPS:
-        raise ValueError(f"a per-query lod reaches at most {L.MAX_MIPS} mips; the table has {last + 1}")
+        what = "a per-query lod reaches" if q is not None else "a mip chain holds"
+        raise ValueError(f"{what} at most {L.MAX_MIPS} mips; the table has {last + 1}")
     c = L.NicMipChain()
     c.num_mips, c.address, c.align_corners = last + 1, _ADDRESS[address], int(bool(align_corners))
     grids = []
@@ -376,10 +378,12 @@ def _mip_chain(fp_like, q, address, align_corners, method, table):
         fl = table[mip]
         g0, g1 = fp_like[fl * 2], fp_like[fl * 2 + 1]
         grids += [g0, g1]
-        c.geom[mip] = L.make_geom(method, g0, g1, 1, q, _step_log2(mip, fl), mip, var2.PE_CHANNELS, _pe_kind(method))
+        extent = [var2.IMAGE_SIZE // pow(2, mip) if a < dim else 1 for a in range(3)]
+        block, blocks = (1, q) if q is not None else (extent[:dim], 1)
+        c.geom[mip] = L.make_geom(method, g0, g1, block, blocks, _step_log2(mip, fl), mip, var2.PE_CHANNELS, _pe_kind(method))
         c.g0[mip], c.g1[mip] = L.ptr(g0), L.ptr(g1)
         for a in range(3):
-            c.extent[mip][a] = var2.IMAGE_SIZE // pow(2, mip) if a < dim else 1
+            c.extent[mip][a] = extent[a]
     return c, grids
 
 
@@ -456,6 +460,57 @@ def sample_codes(codes, decoder, coords, num_bits, lod=None, size=None, address=
     of models.load4fp is fused into the grid read.  Tensor-core precisions only."""
     return _sample(codes, num_bits, decoder, coords, lod, size, address, align_corners, precision, out_dtype, method,
                    level_table, grad)
+
+
+# ------------------------------------------------------------------------------------------------ whole mip chain
+def _decode_mips(fp_like, bits, decoder, precision, out_dtype, out, method, level_table):
+    """Common body of decode_mips (bits None: float32 grids) and decode_mips_codes (uint8 codes of width bits)."""
+    method = _method() if method is None else method
+    dim = 2 if method == L.METHOD_2D else 3
+    table = feature_pyramid_mip_levels() if level_table is None else level_table
+    if out_dtype not in (torch.float32, torch.uint8):
+        raise TypeError("out_dtype must be torch.float32 or torch.uint8")
+    chain, grids = _mip_chain(fp_like, None, "clamp", False, method, table)
+    params = [p.detach().contiguous() for p in decoder.parameters_list()]
+    m = L.make_mlp(params)
+    shapes = [tuple(chain.extent[i][:dim]) for i in range(chain.num_mips)]
+    total = sum(math.prod(s) for s in shapes)
+    device = grids[0].device
+    if out is None:
+        out = torch.empty((total, m.cout), dtype=out_dtype, device=device)
+    elif (not torch.is_tensor(out) or tuple(out.shape) != (total, m.cout) or out.dtype != out_dtype or not out.is_contiguous()
+          or out.device != device):
+        raise ValueError(f"out must be a contiguous {out_dtype} tensor of shape {(total, m.cout)} on {device}")
+    _check_grids(grids, bits)
+    lib = L.load_library()
+    _launch(L.handle(device), lib.nic_decode_mips, lib.nic_decode_mips_codes, bits, (precision or var2.DECODE_PRECISION).lower(),
+            (C.byref(chain),), (C.byref(m), L.ptr(out), L.DT_U8 if out_dtype == torch.uint8 else L.DT_F32),
+            L.stream_ptr(device))
+    views, row = [], 0
+    for s in shapes:
+        views.append(out[row:row + math.prod(s)].view(s + (m.cout,)))
+        row += math.prod(s)
+    return views
+
+
+def decode_mips(fp, decoder, precision=None, out_dtype=torch.float32, out=None, method=None, level_table=None):
+    """Every mip of the model in one call (nic.h nic_decode_mips has the exact rule): mips 0 .. min(MAX_MIP_LEVEL,
+    max(level_table)) at extents IMAGE_SIZE >> mip, the mips and extents `sample(lod=tensor)` filters across — what
+    process_images decodes mip by mip (image_compression.py:400) and a renderer uploads as a mipmapped texture.
+
+    Returns a list of per-mip tensors `[S, S(, S), Cout]` that are consecutive views of one contiguous `[total_texels, Cout]`
+    buffer; `out`, if given, is that buffer.  precision: "f32" | "f16" | "bf16" | "auto" (default var2.DECODE_PRECISION), as
+    for `decode`.  At f32 every mip equals `decode` of that mip bit for bit; on the tensor-core precisions mip 0 equals
+    `decode` bit for bit and mips 1 .. L run as one pass with the mip as a decoder input, so a texel equals
+    `sample(lod=tensor)` at its centre and may differ from `decode` of its mip by 16-bit rounding (+-1 LSB of 8 bits)."""
+    return _decode_mips(fp, None, decoder, precision, out_dtype, out, method, level_table)
+
+
+def decode_mips_codes(codes, decoder, num_bits, precision="f16", out_dtype=torch.uint8, out=None, method=None,
+                      level_table=None):
+    """`decode_mips` straight from the saved model (`codes`: the uint8 list of fp_savable, one code per byte); the
+    de-quantisation of models.load4fp is fused into the grid read.  Tensor-core precisions only."""
+    return _decode_mips(codes, num_bits, decoder, precision, out_dtype, out, method, level_table)
 
 
 # ------------------------------------------------------------------------------------------------ baked colour LUTs
