@@ -3,10 +3,14 @@
 // Reference behaviour: finally_decode_input_* + ColorDecoder.forward inside decode_image
 // (Projects/image_compression.py:54-68, 170-211, 313-327).
 //
-// Two kernels, both ONE persistent CTA per SM made of independent groups of 4 warps (a group = one tile of 128 texels =
-// the MMA M = the TMEM lanes; a group owns 64 accumulator columns of TMEM and its operand buffers in shared memory):
+// Two kernel bodies, both ONE persistent CTA per SM made of independent groups of 4 warps (a group = one tile of 128
+// texels = the MMA M = the TMEM lanes; a group owns 64 accumulator columns of TMEM and its operand buffers in shared memory):
 //   decode_tc2d_ws_kernel   aligned full-resolution 2-D frames; layer 1 re-associated so no input row is ever built;
-//   decode_tc_gws_kernel    everything else (any mip / origin / block shape, both 3-D methods, random-access queries).
+//   decode_tc_gws_body      everything else (any mip / origin / block shape, both 3-D methods, random-access queries),
+//                           behind two entry points that differ in where the grids come from:
+//     decode_tc_gws_kernel      16-bit shadows of the grids in global memory (ShadowGeom);
+//     decode_codes_smem_kernel  random-access queries on a small model whose uint8 codes stay resident in shared memory
+//                               (ResidentCodes).
 // Per tile: layer 1 (KX/16 or 5 tcgen05.mma, M=128 N=64 K=16, SS form) -> epilogue: tcgen05.ld, packed GELU, st.shared in
 // the UMMA K-major layout -> layer 2 (4 MMAs + 1 bias MMA against a constant ones block) -> epilogue -> layer 3 (N=16)
 // -> sigmoid, quantise, store.  The 1/2 of GELU is folded into the next layer's weights.
@@ -22,8 +26,8 @@ namespace nic {
 // W1': [64 x KX]  col k < cin-1: W1[n][k];  col cin-1: b1[n] + lod*W1[n][cin-1];  rest 0.
 // W2': [64 x 80]  col k < 64: W2[n][k]/2 (W2[n][k] for hidden columns on the polynomial GELU);   col 64: b2[n];  rest 0.
 // W3': [16 x 80]  row n < cout: col k < 64: W3[n][k]/2 (same rule); col 64: b3[n];  rest 0.
-// (code-resident path, decode_codes_smem_kernel: the A operand holds the integer grid codes minus their offset, so the
-//  grid columns k < grid_cols of W1 carry the 1 / (2^bits - 1) of models.load4fp: gscale.)
+// (code-resident path, the general body reading ResidentCodes: the A operand holds the integer grid codes minus their
+//  offset, so the grid columns k < grid_cols of W1 carry the 1 / (2^bits - 1) of models.load4fp: gscale.)
 template <int FMT>
 __global__ void pack_weights_kernel(MlpDev m, float lod, int KX, uint16_t* __restrict__ img, int npoly, int grid_cols = 0,
                                     float gscale = 1.0f) {
@@ -81,11 +85,6 @@ struct RowShape {
   static constexpr int C = 12, PE = 6;
   static constexpr int CIN = C * (NC0 + 1) + PE * DIM + 1;    // 73 / 127 / 79
   static constexpr int KX = (CIN + 15) / 16 * 16;            // 80 / 128 / 80
-};
-
-struct ShadowGeom {
-  const uint2* s0;   // shadow of G0, 3 x uint2 per node
-  const uint2* s1;   // shadow of G1
 };
 
 __device__ __forceinline__ int node_lin(const int* n, int dim, int x, int y, int z) {
@@ -579,14 +578,78 @@ __global__ void __launch_bounds__(WS_THREADS, 1) decode_tc2d_ws_kernel(DevGeom g
   if (warp == 0) tmem_dealloc(tmem, WS_TMEM_COLS);
 }
 
+// ================================================================================================ grid sources
+// Where the general body reads a corner's 12 features.  stage() runs in the CTA prologue and may fill the shared memory
+// behind the barriers (the place of the CHAIN modes' chain table: a source that stages never runs in a CHAIN mode),
+// start() once after the CTA barrier.  Then node(grid, i) locates node i of G0 (grid 0) or G1 (grid 1), piece(node, q)
+// loads what holds the node's features [4q, 4q + 4), and pair(piece, h) is features 4q + 2h, 4q + 2h + 1 as a packed
+// 16-bit pair.
+
+// The 16-bit channel-last shadows of both grids in global memory, read with __ldg: every decode_tc_gws_kernel launch.
+struct ShadowGeom {
+  const uint2* s0;   // shadow of G0, 3 x uint2 per node
+  const uint2* s1;   // shadow of G1
+  __device__ __forceinline__ void stage(uint8_t*, const DevGeom&, int, int, int) {}
+  __device__ __forceinline__ void start() {}
+  // CHAIN modes: the shadows of the row's mip, at its offsets in the chain table
+  __device__ __forceinline__ ShadowGeom at_mip(const DevMip& m) const { return {s0 + m.s0, s1 + m.s1}; }
+  __device__ __forceinline__ const uint2* node(int grid, int i) const { return (grid ? s1 : s0) + 3 * i; }
+  __device__ __forceinline__ uint2 piece(const uint2* node, int q) const { return __ldg(node + q); }
+  __device__ __forceinline__ uint32_t pair(uint2 v, int h) const { return h ? v.y : v.x; }
+};
+
+// Random-access decode of a SMALL model straight from its saved uint8 codes (BASELINE config 4: a 65^3 colour LUT, 1e9
+// query points): both grids live in SHARED MEMORY as channel-last codes for the life of the CTA (18^3 + 10^3 nodes x 12
+// bytes = 82 KB), so a query's 16 corner reads are shared-memory loads instead of 48 uncoalesced 8-byte global loads —
+// with the grids in global memory a tile of 128 queries costs ~6,000 L1 wavefronts (one 32-byte sector per thread and
+// load), which is what bounds ShadowGeom at 6 Gquery/s.  The A operand holds the INTEGER codes minus their
+// offset (bytes -> exact f16 integers through 0x6400 | b = 1024 + b), and 1 / (2^bits - 1) rides in W1 (pack_weights_kernel
+// gscale).  f16 only: the byte trick needs 11 mantissa bits.
+struct ResidentCodes {
+  const uint8_t* codes0;   // the caller's codes, channel-major [C][z][y][x] (x fastest)
+  const uint8_t* codes1;
+  int code_off;            // the offset of the codes: the A operand holds code - code_off
+  int bytes0;              // shared-memory bytes of G0 (a multiple of 16); G1 follows
+  const uint8_t* base;     // set by stage(): both grids in shared memory, channel-last [x][y][z][12]
+  __half2 neg;             // set by start(): -(1024 + code_off)
+
+  __device__ __forceinline__ void stage(uint8_t* smem, const DevGeom& g, int dim, int tid, int threads) {
+    // read the codes linearly (coalesced), store them channel-last
+    for (int which = 0; which < 2; ++which) {
+      const uint8_t* src = which == 0 ? codes0 : codes1;
+      uint8_t* dstg = which == 0 ? smem : smem + bytes0;
+      const int* nn = which == 0 ? g.n0 : g.n1;
+      const int nx = nn[0], ny = nn[1], nz = dim == 3 ? nn[2] : 1;
+      const int plane = nx * ny * nz;
+      for (int i = tid; i < 12 * plane; i += threads) {
+        const int c = i / plane, r = i - c * plane;               // r = (z * ny + y) * nx + x
+        const int x = r % nx, yz = r / nx, y = yz % ny, z = yz / ny;
+        dstg[((x * ny + y) * nz + z) * 12 + c] = __ldg(src + i);
+      }
+    }
+    base = smem;
+  }
+  __device__ __forceinline__ void start() { neg = __float2half2_rn(-(1024.0f + (float)code_off)); }
+  __device__ __forceinline__ const uint32_t* node(int grid, int i) const {
+    return reinterpret_cast<const uint32_t*>((grid ? base + bytes0 : base) + 12 * i);
+  }
+  // code word q of the node; its pair h: code bytes 2h, 2h + 1 -> a packed pair of exact f16 integers (code - offset)
+  __device__ __forceinline__ uint32_t piece(const uint32_t* node, int q) const { return node[q]; }
+  __device__ __forceinline__ uint32_t pair(uint32_t w, int h) const {
+    const uint32_t v = __byte_perm(w, 0x64646464u, h ? 0x5342 : 0x5140);
+    const __half2 p = __hadd2(*reinterpret_cast<const __half2*>(&v), neg);
+    return *reinterpret_cast<const uint32_t*>(&p);
+  }
+};
+
 // ================================================================================================ general kernel, v2
 // The general decode (any mip / origin / block shape, 2-D and both 3-D methods, random-access queries) in the same
 // warp-specialised form as decode_tc2d_ws_kernel: ONE persistent CTA per SM made of NG independent groups of 4 warps
 // (NG = 8 for a decoder input of <= 80 columns, 5 for method 3's 128), group s owning TMEM columns [64 s, +64) and one
 // [128 x KX] operand buffer in shared memory.  A group's thread = one texel of its tile:
-//   gather : the texel's decoder-input row goes STRAIGHT from the 16-bit channel-last shadow grids to the operand
-//            buffer — a G0 corner is three 8-byte loads and three 8-byte shared stores, G1 is interpolated in packed
-//            16-bit math (6 registers), the triangular PE comes from a shared LUT — so no thread ever holds the row;
+//   gather : the texel's decoder-input row goes STRAIGHT from the grid source to the operand buffer — a G0 corner is
+//            three 8-byte pieces and three 8-byte shared stores, G1 is interpolated in packed 16-bit math (6 registers),
+//            the triangular PE comes from a shared LUT — so no thread ever holds the row;
 //   layers : SS-form tcgen05.mma issued by the group's elected lane after a 128-thread named barrier (layer 1: KX/16
 //            MMAs; layers 2, 3: 4 MMAs + 1 bias MMA against a shared constant ones block), the epilogue overwrites the
 //            operand buffer with the next layer's activations;  the groups never meet at a CTA-wide barrier.
@@ -610,10 +673,9 @@ constexpr int TAPS_MIPS = -1;
 // 32 KB operand buffers, 256 LUT entries) always fit; with a 64-entry LUT (step >= 1/4: every full-resolution decode) a
 // SIXTH 32 KB group fits the 227 KB of shared memory for method 3 (225.8 KB), 20 % more tiles in flight.
 constexpr int gws_groups(int kx, int ngt) { return ngt ? ngt : (kx > 80 ? 5 : 8); }
-template <int METHOD, int FMT, typename OutT, int NPOLY, int NGT = 0, int LUTCAP = TC_LUT_MAX, int TAPS = 0>
-__global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GROUP, 1)
-    decode_tc_gws_kernel(DevGeom g, ShadowGeom sg, const long long* __restrict__ origins, const uint4* __restrict__ wimg,
-                         int cout, int lut_n, OutT* __restrict__ out, DevSampler smp) {
+template <int METHOD, int FMT, int NPOLY, int NGT, int LUTCAP, int TAPS, typename OutT, class Grids>
+__device__ __forceinline__ void decode_tc_gws_body(const DevGeom& g, Grids grids, const long long* origins, const uint4* wimg,
+                                                   int cout, int lut_n, OutT* out, const DevSampler& smp) {
   using S = RowShape<METHOD>;
   using P = Pair<FMT>;
   constexpr int KX = S::KX, NG = gws_groups(KX, NGT), THREADS = NG * GW_GROUP;
@@ -668,6 +730,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
       *reinterpret_cast<uint4*>(sOne + roff) = make_uint4(*reinterpret_cast<uint32_t*>(&one), 0, 0, 0);
       *reinterpret_cast<uint4*>(sOne + KG + roff) = make_uint4(0, 0, 0, 0);
     }
+    grids.stage(smem_raw + OFF_BAR + 256, g, S::DIM, tid, THREADS);
   }
   fence_async_smem();
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -695,6 +758,7 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
   const uint32_t loW1 = smem_desc_lo(aW1, LBO_64), loW2 = smem_desc_lo(aW2, LBO_64), loW3 = smem_desc_lo(aW3, LBO_16);
   // this thread's 8-byte piece holding features [f, f + 4) of its row (f a multiple of 4)
   auto piece = [&](int f) -> uint2* { return reinterpret_cast<uint2*>(sAct + (f >> 3) * KG + roff + (f & 7) * 2); };
+  grids.start();
 
   const unsigned ntiles = (unsigned)((g.N + TC_ROWS - 1) / TC_ROWS);
   const int lut_mask = lut_n - 1;
@@ -747,8 +811,8 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
       }
       const int* n0 = CHAIN ? mp->n0 : g.n0;
       const int* n1 = CHAIN ? mp->n1 : g.n1;
-      const uint2* s0 = CHAIN ? sg.s0 + mp->s0 : sg.s0;
-      const uint2* s1 = CHAIN ? sg.s1 + mp->s1 : sg.s1;
+      Grids src = grids;
+      if constexpr (CHAIN) src = grids.at_mip(*mp);
       AxisCoord ax[3];
 #pragma unroll
       for (int a = 0; a < 3; ++a) {
@@ -757,19 +821,22 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
         ax[a].i1 = clampi(ax[a].i1, 0, n1[a] - 2 < 0 ? 0 : n1[a] - 2);
       }
 #pragma unroll
-      for (int j = 0; j < S::NC0; ++j) {             // G0 corners: raw copies
+      for (int j = 0; j < S::NC0; ++j) {             // G0 corners: the source's pairs, unweighted
         const int8_t* d = S::DIM == 2 ? kCorner2D[j] : (METHOD == NIC_METHOD_3D ? kCorner3D[j] : kCorner3Dv2[j]);
         const int dz = S::DIM == 3 ? d[0] : 0;
-        const uint2* node = s0 + 3 * node_lin(n0, S::DIM, ax[0].i0 + d[2], ax[1].i0 + d[1], ax[2].i0 + dz);
+        const auto node = src.node(0, node_lin(n0, S::DIM, ax[0].i0 + d[2], ax[1].i0 + d[1], ax[2].i0 + dz));
 #pragma unroll
-        for (int q = 0; q < 3; ++q) *piece(12 * j + 4 * q) = __ldg(node + q);
+        for (int q = 0; q < 3; ++q) {
+          const auto v = src.piece(node, q);
+          *piece(12 * j + 4 * q) = make_uint2(src.pair(v, 0), src.pair(v, 1));
+        }
       }
       typename P::T2 acc[6];                          // G1: weighted sum of corners
 #pragma unroll
       for (int j = 0; j < S::NC1; ++j) {
         const int8_t* d = S::DIM == 2 ? kCorner2D[j] : kCorner3D[j];
         const int dz = S::DIM == 3 ? d[0] : 0;
-        const uint2* node = s1 + 3 * node_lin(n1, S::DIM, ax[0].i1 + d[2], ax[1].i1 + d[1], ax[2].i1 + dz);
+        const auto node = src.node(1, node_lin(n1, S::DIM, ax[0].i1 + d[2], ax[1].i1 + d[1], ax[2].i1 + dz));
         float f[3];
         g1_factors(g, j, ax, f);
         if constexpr (CHAIN) {
@@ -780,10 +847,13 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
         typename P::T2 w2 = P::cst(w);
 #pragma unroll
         for (int q = 0; q < 3; ++q) {
-          uint2 v = __ldg(node + q);
-          typename P::T2 va = *reinterpret_cast<typename P::T2*>(&v.x), vb = *reinterpret_cast<typename P::T2*>(&v.y);
-          acc[2 * q] = j == 0 ? __hmul2(va, w2) : __hfma2(va, w2, acc[2 * q]);
-          acc[2 * q + 1] = j == 0 ? __hmul2(vb, w2) : __hfma2(vb, w2, acc[2 * q + 1]);
+          const auto v = src.piece(node, q);
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            uint32_t pr = src.pair(v, h);
+            typename P::T2 vh = *reinterpret_cast<typename P::T2*>(&pr);
+            acc[2 * q + h] = j == 0 ? __hmul2(vh, w2) : __hfma2(vh, w2, acc[2 * q + h]);
+          }
         }
       }
 #pragma unroll
@@ -932,254 +1002,24 @@ __global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GRO
   if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
-// ================================================================================================ code-resident queries
-// Random-access decode of a SMALL model straight from its saved uint8 codes (BASELINE config 4: a 65^3 colour LUT, 1e9
-// query points): both grids live in SHARED MEMORY as channel-last codes for the life of the CTA (18^3 + 10^3 nodes x 12
-// bytes = 82 KB), so a query's 16 corner reads are shared-memory loads instead of 48 uncoalesced 8-byte global loads —
-// with the grids in global memory a tile of 128 queries costs ~6,000 L1 wavefronts (one 32-byte sector per thread and
-// load), which is what bounds decode_tc_gws_kernel at 6 Gquery/s.  The A operand holds the INTEGER codes minus their
-// offset (bytes -> exact f16 integers through 0x6400 | b = 1024 + b), and 1 / (2^bits - 1) rides in W1 (pack_weights_kernel
-// gscale).  f16 only (the byte trick needs 11 mantissa bits); otherwise the structure of decode_tc_gws_kernel with NG = 3.
+// The general kernel: the grids come from their 16-bit shadows in global memory.
+template <int METHOD, int FMT, typename OutT, int NPOLY, int NGT = 0, int LUTCAP = TC_LUT_MAX, int TAPS = 0>
+__global__ void __launch_bounds__(gws_groups(RowShape<METHOD>::KX, NGT) * GW_GROUP, 1)
+    decode_tc_gws_kernel(DevGeom g, ShadowGeom sg, const long long* __restrict__ origins, const uint4* __restrict__ wimg,
+                         int cout, int lut_n, OutT* __restrict__ out, DevSampler smp) {
+  decode_tc_gws_body<METHOD, FMT, NPOLY, NGT, LUTCAP, TAPS>(g, sg, origins, wimg, cout, lut_n, out, smp);
+}
+
+// Code-resident queries: the general body on random-access queries with both grids resident in shared memory as codes
+// (ResidentCodes), f16, three groups (the grids take the shared memory of the others).
 constexpr int CQ_NG = 3;
 template <int METHOD, typename OutT, int NPOLY>
 __global__ void __launch_bounds__(CQ_NG * GW_GROUP, 1)
     decode_codes_smem_kernel(DevGeom g, const uint8_t* __restrict__ codes0, const uint8_t* __restrict__ codes1, int code_off,
                              int bytes0, const long long* __restrict__ origins, const uint4* __restrict__ wimg, int cout,
                              int lut_n, OutT* __restrict__ out) {
-  using S = RowShape<METHOD>;
-  constexpr int FMT = 0;
-  using P = Pair<FMT>;
-  constexpr int KX = S::KX, NG = CQ_NG, THREADS = NG * GW_GROUP;
-  constexpr int W1_BYTES = b_image_bytes(64, KX), W2_BYTES = b_image_bytes(64, TC_K2), W3_BYTES = b_image_bytes(16, TC_K2);
-  constexpr int KG = 16 * 128;
-  constexpr int OFF_LUT = W1_BYTES + W2_BYTES + W3_BYTES, OFF_ONE = OFF_LUT + TC_LUT_MAX * 16, OFF_ACT = OFF_ONE + 2 * KG;
-  constexpr int ACT_BYTES = (KX / 8) * KG, OFF_BAR = OFF_ACT + NG * ACT_BYTES, OFF_GRID = OFF_BAR + 256;
-  extern __shared__ __align__(128) uint8_t smem_raw[];
-  uint8_t* sW1 = smem_raw;
-  uint8_t* sW2 = sW1 + W1_BYTES;
-  uint8_t* sW3 = sW2 + W2_BYTES;
-  uint4* sLut = reinterpret_cast<uint4*>(smem_raw + OFF_LUT);
-  uint8_t* sOne = smem_raw + OFF_ONE;
-  uint64_t* bar_full = reinterpret_cast<uint64_t*>(smem_raw + OFF_BAR);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_full + NG);
-  uint8_t* sG0 = smem_raw + OFF_GRID;                  // codes, channel-last: [x][y][z][12]
-  uint8_t* sG1 = sG0 + bytes0;                         // (bytes0 is a multiple of 16)
-
-  const int tid = threadIdx.x, warp = uniform_warp_index(), lane = tid & 31;
-  const int slot = warp >> 2;
-  const int row = 32 * (warp & 3) + lane;
-  const int roff = (row >> 3) * 128 + (row & 7) * 16;
-  if (warp == 0) tmem_alloc(tmem_slot, 512);
-  if (tid == 0)
-    for (int s = 0; s < NG; ++s) mbar_init(bar_full + s, 1);
-  {
-    uint4* dst = reinterpret_cast<uint4*>(smem_raw);
-    for (int i = tid; i < OFF_LUT / 16; i += THREADS) dst[i] = __ldg(wimg + i);
-    for (int i = tid; i < lut_n; i += THREADS) {
-      float u1 = __fmul_rn(__fmul_rn((float)i, g.step), 0.5f);
-      uint4 e;
-      auto v0 = P::pack(pe_triangular(u1, 0, 6), pe_triangular(u1, 1, 6));
-      auto v1 = P::pack(pe_triangular(u1, 2, 6), pe_triangular(u1, 3, 6));
-      auto v2 = P::pack(pe_triangular(u1, 4, 6), pe_triangular(u1, 5, 6));
-      e.x = *reinterpret_cast<uint32_t*>(&v0);
-      e.y = *reinterpret_cast<uint32_t*>(&v1);
-      e.z = *reinterpret_cast<uint32_t*>(&v2);
-      e.w = 0u;
-      sLut[i] = e;
-    }
-    if (slot == 0) {
-      auto one = P::pack(1.0f, 0.0f);
-      *reinterpret_cast<uint4*>(sOne + roff) = make_uint4(*reinterpret_cast<uint32_t*>(&one), 0, 0, 0);
-      *reinterpret_cast<uint4*>(sOne + KG + roff) = make_uint4(0, 0, 0, 0);
-    }
-    // the caller's codes are channel-major [C][z][y][x] (x fastest): read them linearly (coalesced), store channel-last
-    for (int which = 0; which < 2; ++which) {
-      const uint8_t* src = which == 0 ? codes0 : codes1;
-      uint8_t* dstg = which == 0 ? sG0 : sG1;
-      const int* nn = which == 0 ? g.n0 : g.n1;
-      const int nx = nn[0], ny = nn[1], nz = S::DIM == 3 ? nn[2] : 1;
-      const int plane = nx * ny * nz;
-      for (int i = tid; i < 12 * plane; i += THREADS) {
-        const int c = i / plane, r = i - c * plane;               // r = (z * ny + y) * nx + x
-        const int x = r % nx, yz = r / nx, y = yz % ny, z = yz / ny;
-        dstg[((x * ny + y) * nz + z) * 12 + c] = __ldg(src + i);
-      }
-    }
-  }
-  fence_async_smem();
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const uint32_t tDs = tmem + slot * 64;
-  const uint32_t tD = tDs + ((uint32_t)((warp & 3) * 32) << 16);
-  uint8_t* sAct = smem_raw + OFF_ACT + slot * ACT_BYTES;
-  const bool issuer_warp = (warp & 3) == (slot & 3);
-  constexpr uint32_t IDESC_64 = make_idesc(FMT, 128, 64, 0, 1), IDESC_16 = make_idesc(FMT, 128, 16);
-  constexpr uint32_t LBO_64 = (64 / 8) * 128, LBO_16 = (16 / 8) * 128, SBO = 128;
-  const uint32_t aW1 = smem_u32(sW1), aW2 = smem_u32(sW2), aW3 = smem_u32(sW3), aOne = smem_u32(sOne), aAct = smem_u32(sAct);
-  auto group_sync = [&]() { asm volatile("bar.sync %0, %1;" ::"r"(1 + slot), "n"(GW_GROUP) : "memory"); };
-  auto group_wait = [&](uint32_t phase) {
-    if (issuer_warp) mbar_wait(bar_full + slot, phase);
-    group_sync();
-  };
-  constexpr uint32_t HI_SBO = smem_desc_hi(SBO);
-  const uint32_t loAct = smem_desc_lo(aAct, KG), loOne = smem_desc_lo(aOne, KG);
-  const uint32_t loW1 = smem_desc_lo(aW1, LBO_64), loW2 = smem_desc_lo(aW2, LBO_64), loW3 = smem_desc_lo(aW3, LBO_16);
-  auto piece = [&](int f) -> uint2* { return reinterpret_cast<uint2*>(sAct + (f >> 3) * KG + roff + (f & 7) * 2); };
-  // four code bytes -> two packed pairs of exact f16 integers (code - offset)
-  const __half2 neg = __float2half2_rn(-(1024.0f + (float)code_off));
-  auto pair_lo = [&](uint32_t w) {
-    const uint32_t v = __byte_perm(w, 0x64646464u, 0x5140);
-    return __hadd2(*reinterpret_cast<const __half2*>(&v), neg);
-  };
-  auto pair_hi = [&](uint32_t w) {
-    const uint32_t v = __byte_perm(w, 0x64646464u, 0x5342);
-    return __hadd2(*reinterpret_cast<const __half2*>(&v), neg);
-  };
-  auto bits2 = [](__half2 v) { return *reinterpret_cast<uint32_t*>(&v); };
-
-  const unsigned ntiles = (unsigned)((g.N + TC_ROWS - 1) / TC_ROWS);
-  const int lut_mask = lut_n - 1;
-  uint32_t ph = 0;
-  for (unsigned tile = blockIdx.x + gridDim.x * slot; tile < ntiles; tile += gridDim.x * NG) {
-    const unsigned n = tile * TC_ROWS + row;
-    const bool live = n < (unsigned)g.N;
-    {
-      Texel t = texel_of_fast(g, live ? n : (unsigned)g.N - 1, origins);
-      AxisCoord ax[3];
-#pragma unroll
-      for (int a = 0; a < 3; ++a) {
-        ax[a] = axis_coord(t.p[a], g.step);
-        ax[a].i0 = clampi(ax[a].i0, 0, g.n0[a] - 2 < 0 ? 0 : g.n0[a] - 2);
-        ax[a].i1 = clampi(ax[a].i1, 0, g.n1[a] - 2 < 0 ? 0 : g.n1[a] - 2);
-      }
-#pragma unroll
-      for (int j = 0; j < S::NC0; ++j) {             // G0 corners: 12 code bytes -> 12 features
-        const int8_t* d = S::DIM == 2 ? kCorner2D[j] : (METHOD == NIC_METHOD_3D ? kCorner3D[j] : kCorner3Dv2[j]);
-        const int dz = S::DIM == 3 ? d[0] : 0;
-        const uint32_t* node = reinterpret_cast<const uint32_t*>(sG0 + 12 * node_lin(g.n0, S::DIM, ax[0].i0 + d[2], ax[1].i0 + d[1], ax[2].i0 + dz));
-#pragma unroll
-        for (int q = 0; q < 3; ++q) {
-          const uint32_t w = node[q];
-          *piece(12 * j + 4 * q) = make_uint2(bits2(pair_lo(w)), bits2(pair_hi(w)));
-        }
-      }
-      __half2 acc[6];                                 // G1: weighted sum of corners
-#pragma unroll
-      for (int j = 0; j < S::NC1; ++j) {
-        const int8_t* d = S::DIM == 2 ? kCorner2D[j] : kCorner3D[j];
-        const int dz = S::DIM == 3 ? d[0] : 0;
-        const uint32_t* node = reinterpret_cast<const uint32_t*>(sG1 + 12 * node_lin(g.n1, S::DIM, ax[0].i1 + d[2], ax[1].i1 + d[1], ax[2].i1 + dz));
-        float f[3];
-        g1_factors(g, j, ax, f);
-        float wgt = f[0] * f[1];
-        if (S::DIM == 3) wgt *= f[2];
-        const __half2 w2 = __float2half2_rn(wgt);
-#pragma unroll
-        for (int q = 0; q < 3; ++q) {
-          const uint32_t w = node[q];
-          acc[2 * q] = j == 0 ? __hmul2(pair_lo(w), w2) : __hfma2(pair_lo(w), w2, acc[2 * q]);
-          acc[2 * q + 1] = j == 0 ? __hmul2(pair_hi(w), w2) : __hfma2(pair_hi(w), w2, acc[2 * q + 1]);
-        }
-      }
-#pragma unroll
-      for (int q = 0; q < 3; ++q) *piece(12 * S::NC0 + 4 * q) = make_uint2(bits2(acc[2 * q]), bits2(acc[2 * q + 1]));
-      constexpr int T0 = 12 * (S::NC0 + 1), NTAIL = (KX - T0) / 2;
-      uint32_t tail[NTAIL];
-#pragma unroll
-      for (int i = 0; i < NTAIL; ++i) tail[i] = 0u;
-#pragma unroll
-      for (int a = 0; a < S::DIM; ++a) {
-        if (g.pe_kind == NIC_PE_TRIANGULAR) {
-          uint4 e = sLut[t.p[a] & lut_mask];
-          tail[3 * a] = e.x;
-          tail[3 * a + 1] = e.y;
-          tail[3 * a + 2] = e.z;
-        } else {
-#pragma unroll
-          for (int q = 0; q < 3; ++q) {
-            float arg = __fmul_rn(ax[a].u1, g.pe_div[q]);
-            auto v = P::pack(sinf(arg), cosf(arg));
-            tail[3 * a + q] = *reinterpret_cast<uint32_t*>(&v);
-          }
-        }
-      }
-      {
-        auto one = P::pack(1.0f, 0.0f);
-        tail[(S::CIN - 1 - T0) / 2] = *reinterpret_cast<uint32_t*>(&one);
-      }
-#pragma unroll
-      for (int i = 0; i < NTAIL / 2; ++i) *piece(T0 + 4 * i) = make_uint2(tail[2 * i], tail[2 * i + 1]);
-    }
-    fence_async_smem();
-    tc_fence_before();
-    group_sync();
-    if (issuer_warp) {
-      if (elect_one()) {
-        tc_fence_after();
-#pragma unroll
-        for (int kc = 0; kc < KX / 16; ++kc)
-          mma_ss_lohi(tDs, loAct + kc * (2 * KG >> 4), HI_SBO, loW1 + kc * (2 * LBO_64 >> 4), HI_SBO, IDESC_64, kc > 0);
-        tc_commit(bar_full + slot);
-      }
-      __syncwarp();
-    }
-#pragma unroll 1
-    for (int layer = 0; layer < 2; ++layer) {
-      group_wait(ph);
-      ph ^= 1;
-      tc_fence_after();
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        uint32_t acc[8], hp[8];
-        tmem_ld8_pack16(tD + 16 * q, acc);
-        tc_wait_ld();
-#pragma unroll
-        for (int k = 0; k < 8; ++k) hp[k] = gelu_poly_pair_sel(k, NPOLY) ? gelu_poly_packed<FMT>(acc[k]) : gelu2x_packed<FMT>(acc[k]);
-        *reinterpret_cast<uint4*>(sAct + (2 * q) * KG + roff) = make_uint4(hp[0], hp[1], hp[2], hp[3]);
-        *reinterpret_cast<uint4*>(sAct + (2 * q + 1) * KG + roff) = make_uint4(hp[4], hp[5], hp[6], hp[7]);
-      }
-      fence_async_smem();
-      tc_fence_before();
-      group_sync();
-      if (issuer_warp) {
-        if (elect_one()) {
-          tc_fence_after();
-          const uint32_t loW = layer == 0 ? loW2 : loW3, stepW = layer == 0 ? (2 * LBO_64 >> 4) : (2 * LBO_16 >> 4);
-          const uint32_t idesc = layer == 0 ? IDESC_64 : IDESC_16;
-#pragma unroll
-          for (int kc = 0; kc < 4; ++kc)
-            mma_ss_lohi(tDs, loAct + kc * (2 * KG >> 4), HI_SBO, loW + kc * stepW, HI_SBO, idesc, kc > 0);
-          mma_ss_lohi(tDs, loOne, HI_SBO, loW + 4 * stepW, HI_SBO, idesc, 1);
-          tc_commit(bar_full + slot);
-        }
-        __syncwarp();
-      }
-    }
-    group_wait(ph);
-    ph ^= 1;
-    tc_fence_after();
-    uint32_t acc[16];
-    if (cout > 4) tmem_ld16(tD, acc);
-    else tmem_ld4(tD, acc);
-    tc_wait_ld();
-    tc_fence_before();
-    if (live) {
-#pragma unroll
-      for (int c = 0; c < 4; ++c)
-        if (c < cout) store_sigmoid(out + (size_t)n * cout + c, __uint_as_float(acc[c]));
-      if (cout > 4) {
-#pragma unroll
-        for (int c = 4; c < 16; ++c)
-          if (c < cout) store_sigmoid(out + (size_t)n * cout + c, __uint_as_float(acc[c]));
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem, 512);
+  decode_tc_gws_body<METHOD, 0, NPOLY, CQ_NG, TC_LUT_MAX, 0>(g, ResidentCodes{codes0, codes1, code_off, bytes0}, origins,
+                                                            wimg, cout, lut_n, out, DevSampler{});
 }
 
 // ------------------------------------------------------------------------------------------------ launcher
@@ -1226,9 +1066,9 @@ static int pe_lut_len(const DevGeom& g) {
   return g.pe_kind == NIC_PE_TRIANGULAR && (float)n < period ? NIC_ERR_UNSUPPORTED : n;
 }
 
-// Dynamic shared memory of decode_tc_gws_kernel with NG groups and a LUTCAP-entry LUT: weight images, LUT, ones block,
+// Dynamic shared memory of decode_tc_gws_body with NG groups and a LUTCAP-entry LUT: weight images, LUT, ones block,
 // operand buffers, barriers, and behind them the `table` bytes of the chain table of a per-query-LOD (DevChain) or dense-chain
-// (DevMipRows) launch.  The code-resident kernel has the same layout with CQ_NG groups, followed by its two grids.
+// (DevMipRows) launch.  With ResidentCodes (CQ_NG groups) the two grids take that place instead.
 template <int METHOD>
 constexpr int gws_smem(int ng, int lutcap, size_t table = 0) {
   using S = RowShape<METHOD>;
@@ -1353,7 +1193,7 @@ static int launch_fast2d(Handle* h, const DevGeom& g, const MlpDev& m, const voi
 }
 
 // TAPS > 0: filtered sampling (smp set, g.N = queries * TAPS rows) always runs on the general kernel: the fast 2-D kernel
-// and the code-resident kernel have no per-row texel and no tap epilogue.
+// has no per-row texel and no tap epilogue, and the code-resident kernel is built for TAPS = 0 only.
 template <int METHOD, int FMT, int TAPS, typename OutT>
 static int launch_tc_t(Handle* h, const DevGeom& g, const MlpDev& m, const void* g0, const void* g1, int code_bits,
                        const long long* origins, OutT* out, cudaStream_t st, const DevSampler& smp = DevSampler{}) {
